@@ -2,7 +2,7 @@
 """Benchmark of the matching-pursuit hot path (BASELINE.json metric: MP atoms selected/s and signal
 samples encoded/s at 1/2/4/8 B200).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4|c2|c5] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4|c2|c5] [--impl b200|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (K1 initial correlation + K2 select/update loop to the stop
 rule) over one batch of synthetic signals.  Default workload: BASELINE config 4's per-GPU shard
@@ -319,7 +319,50 @@ def cpu_baseline_sample(w, D, budget_s=14.0):
 # GPU arm
 # ------------------------------------------------------------------------------------------------
 
-def quick_workload(hsc, torch, dev, local_rank, name):
+DUMP_LIMIT_BYTES = 60 * 10 ** 6          # under 64 MB with the .npy headers, whichever megabyte is meant
+DUMP_RESIDUAL_BYTES = 16 * 2 ** 20
+
+
+def dump_outputs(out_dir, compact, resid, states):
+    """Writes what one step of the timed path returned, as float32 / float64 .npy files under out_dir, so that two builds
+    can be compared output for output on the same seeded inputs:
+      code_signal, code_pos, code_filter, code_coef  the sparse codes: one entry per selected atom, signal by signal in
+                                                     selection order (the engine's device compaction of the event buffers)
+      energy_residual                                the final residual energy the engine reports for every signal
+      residual_signals, residual                     the residual signals [n, T, F] of a fixed seeded sample of n signals
+                                                     (all of them would not fit the 64 MB the dump may take)
+    When the codes of all signals could not fit either (at the event-buffer capacity of every signal), a fixed seeded sample
+    of signals, chosen from the number of signals and that capacity alone, keeps its codes: two builds dump the same signals.
+    With several GPUs this is rank 0's own shard, as rank 0 computed it before the gather of the codes."""
+    import torch
+    S, T, F = resid.shape
+    off = compact['offsets'].cpu().numpy()
+    total = int(off[-1])
+    sig = np.repeat(np.arange(S), np.diff(off))
+    pos = compact['pos'][:total].cpu().numpy()
+    idx = compact['idx'][:total].cpu().numpy()
+    coef = compact['coef'][:total].cpu().numpy()
+    n_res = max(1, min(S, DUMP_RESIDUAL_BYTES // (T * F * resid.element_size())))
+    res_rows = np.sort(np.random.RandomState(0).choice(S, n_res, replace=False))
+    per_atom = 3 * 8 + coef.itemsize
+    budget = DUMP_LIMIT_BYTES - n_res * (8 + T * F * resid.element_size()) - 8 * S
+    cap = compact['pos'].numel() // S
+    if S * cap * per_atom > budget:
+        keep = np.sort(np.random.RandomState(1).permutation(S)[:budget // (cap * per_atom)])
+        mask = np.isin(sig, keep)
+        sig, pos, idx, coef = sig[mask], pos[mask], idx[mask], coef[mask]
+    arrays = {'code_signal': sig.astype(np.float64), 'code_pos': pos.astype(np.float64), 'code_filter': idx.astype(np.float64),
+              'code_coef': coef, 'energy_residual': np.array([st.energy_residual for st in states], dtype=np.float64),
+              'residual_signals': res_rows.astype(np.float64),
+              'residual': resid[torch.as_tensor(res_rows, device=resid.device)].cpu().numpy()}
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_LIMIT_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), name
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
+def quick_workload(hsc, torch, dev, local_rank, name, steps, warmup):
     """A few resident steps of another BASELINE configuration (one step after the other, CUDA events), for the `extra` section."""
     w = dict(WORKLOADS[name])
     if name == 'c2':
@@ -338,7 +381,7 @@ def quick_workload(hsc, torch, dev, local_rank, name):
     evc = torch.empty((S, cap), dtype=torch.float32, device=dev)
     stream = torch.cuda.current_stream(dev)
     k1, k2, atoms = [], [], 0
-    for it in range(4):
+    for it in range(warmup + steps):
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
         ev[0].record(stream)
         eng.begin_only(xd, opt, resid)
@@ -346,7 +389,7 @@ def quick_workload(hsc, torch, dev, local_rank, name):
         states = eng.run_only(evp, evi, evc, cap, sync_states=True)
         ev[2].record(stream)
         torch.cuda.synchronize(dev)
-        if it > 0:
+        if it >= warmup:
             k1.append(ev[0].elapsed_time(ev[1]))
             k2.append(ev[1].elapsed_time(ev[2]))
         atoms = int(sum(st.n_events for st in states))
@@ -354,20 +397,20 @@ def quick_workload(hsc, torch, dev, local_rank, name):
     out = {'workload': w['desc'] if name != 'c2' else 'config2 shape: 1 sequence x 1e6, 16 filters x 32, nbNonzeroCoefs=3000',
            'atoms_per_step': atoms, 'k1_ms': k1m, 'k2_ms': k2m, 'atoms_per_s': atoms / ((k1m + k2m) / 1e3),
            'us_per_selection_per_signal': 1e3 * k2m / (atoms / S), 'k2_algorithmic_gbs': atoms * per_atom_bytes(w) / (k2m / 1e3) / 1e9,
-           'mode': 'one step after the other, 3 timed steps'}
+           'mode': 'one step after the other, %d timed steps' % steps}
     if name == 'c5':
         rs = np.random.RandomState(7)
         D0 = D.astype(np.float64) + 0.3 * rs.randn(*D.shape) / math.sqrt(D.shape[1] * D.shape[2])
         D0 /= np.sqrt(np.sum(D0 * D0, axis=(1, 2), keepdims=True))
         del xd, resid, evp, evi, evc
         learner = hsc.ConvolutionalDictionaryLearner(K, L, algorithm='ksvd', device=local_rank)
-        learner.train(x_host, method='cmp', maxIterations=5, toleranceSnr=None, nbNonzeroCoefs=n_atoms, initD=D0, dtype=np.float32)
+        learner.train(x_host, method='cmp', maxIterations=warmup + steps, toleranceSnr=None, nbNonzeroCoefs=n_atoms, initD=D0, dtype=np.float32)
         torch.cuda.synchronize(dev)
-        h = learner.history[2:]
+        h = learner.history[warmup:]
         out['ksvd_loop'] = {'iterations': len(learner.history), 'encode_ms': 1e3 * float(np.mean([q['encode_s'] for q in h])),
                             'update_ms': 1e3 * float(np.mean([q['update_s'] for q in h])),
                             'per_iteration_ms': [[round(1e3 * q['encode_s'], 1), round(1e3 * q['update_s'], 1)] for q in learner.history],
-                            'note': 'ConvolutionalDictionaryLearner(algorithm=ksvd).train on the 190 segments (cmp, float32 inference, float64 update); mean of iterations 3-5'}
+                            'note': 'ConvolutionalDictionaryLearner(algorithm=ksvd).train on the 190 segments (cmp, float32 inference, float64 update); mean of iterations %d-%d' % (warmup + 1, warmup + steps)}
     eng.close()
     torch.cuda.empty_cache()
     return out
@@ -446,6 +489,7 @@ def run_b200_arm(args, w):
                 return states, n_buffered
 
     step_no = [0]
+    last_step = {}
 
     def step_resident(record):
         nonlocal atoms_step
@@ -463,6 +507,7 @@ def run_b200_arm(args, w):
             k1_ms.append(ev[0].elapsed_time(ev[1]))
             k2_ms.append(ev[1].elapsed_time(ev[2]))
         atoms_step = int(sum(st.n_events for st in states))
+        last_step.update(es=es, states=states)
         run_info['reranked_selections'] = int(sum(st.reranked for st in states))
         stop_hist.clear()
         for st in states:
@@ -568,11 +613,18 @@ def run_b200_arm(args, w):
     clocks = sampler.stop()
     launches = launches_now() - launches0
     total_ms = t_start.elapsed_time(t_end)
+    if args.dump_outputs and rank == 0:
+        if args.pipeline:
+            sl = slots[(args.steps - 1) % n_slots]
+            dump_outputs(args.dump_outputs, sl.compact(None, stream), sl.resid, sl.states)
+        else:
+            es = last_step['es']
+            dump_outputs(args.dump_outputs, eng.compact_events(es['evp'], es['evi'], es['evc']), resid, last_step['states'])
     # stand-alone durations of the two kernels (outside the timed region): inside the pipeline a launch shares the GPU with
     # the tail of the previous pursuit and with the next correlation, so its event-to-event time is not its own cost
     solo_k1, solo_k2 = [], []
     if args.pipeline:
-        for _ in range(2):
+        for _ in range(args.steps):
             es = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
             es[0].record(stream)
             slots[0].begin(xd, opt, stream)
@@ -609,7 +661,7 @@ def run_b200_arm(args, w):
                 d2h = int(sum(len(p) for p in r.gathered['pos']) * 12 + world * (S + 1) * 8 + S * 104)
         return atoms, d2h
 
-    e2e_steps = max(4, min(2 * args.steps, 12))      # enough batches to amortise the pipeline's fill and drain
+    e2e_steps = args.steps
     e2e_runs = {}
     for tag, want_res in (('codes', False), ('codes+residual', True)):
         run_e2e(min(args.warmup, 2), want_res)
@@ -650,7 +702,7 @@ def run_b200_arm(args, w):
         torch.cuda.empty_cache()
         for name in ('c5', 'c2'):
             try:
-                others[name] = quick_workload(hsc, torch, dev, local_rank, name)
+                others[name] = quick_workload(hsc, torch, dev, local_rank, name, args.steps, args.warmup)
             except Exception as e:          # noqa: BLE001  (the headline line must not depend on the extras)
                 others[name] = {'error': repr(e)[:300]}
 
@@ -704,9 +756,9 @@ def run_b200_arm(args, w):
                 rk['ms_per_launch'] = solo_ms
                 rk['achieved'] = work / (solo_ms / 1e3)
                 rk['frac'] = rk['achieved'] / rk['peak']
-                rk['measured'] = ('stand-alone launch, CUDA events on its stream, right after the timed region (mean of 2); inside the '
+                rk['measured'] = ('stand-alone launch, CUDA events on its stream, right after the timed region (mean of %d); inside the '
                                   'streaming pipeline the same launch takes pipelined_ms_per_launch because it shares the GPU with the '
-                                  'previous pursuit\'s tail and the next correlation')
+                                  'previous pursuit\'s tail and the next correlation' % args.steps)
             roof_k1['issued_tflops'] = 3.0 * kd_pad * roof_k1['achieved']
             roof_k1['issued_frac'] = roof_k1['issued_tflops'] / k1_peak
             roof_k1['hbm_gbs'] = correlation_bytes(w) / (k1_solo / 1e3) / 1e9
@@ -776,7 +828,14 @@ def main():
     ap.add_argument('--slots', type=int, default=2, help='pipeline: encode slots (workspaces) in flight')
     ap.add_argument('--pipeline', type=int, default=1, help='1: steps run as a streaming pipeline on several CUDA streams (default); 0: one step after the other')
     ap.add_argument('--ksvd-iters', type=int, default=0, help='also time N K-SVD iterations (encode + dictionary update) on the workload')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last one returned (sparse codes, residual energies, a seeded sample '
+                         'of residual signals) as .npy files under DIR, at most 64 MB; with several GPUs, the shard of rank 0')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes what the GPU path computed; it has no meaning with --impl reference')
     w = dict(WORKLOADS[args.workload])
     if args.signals:
         w['S'] = args.signals

@@ -26,6 +26,11 @@ def coo_sorted(m):
     return c.row[order].astype(np.int64), c.col[order].astype(np.int64), c.data[order].astype(np.float64)
 
 
+def stored_code(z, key):
+    """The csc code [T,K] stored under key_t / key_k / key_v / key_shape (tests/golden/make_golden_dropin.py)."""
+    return scipy.sparse.coo_matrix((z[key + '_v'], (z[key + '_t'], z[key + '_k'])), shape=tuple(z[key + '_shape'])).tocsc()
+
+
 def snr_db(x, residual):
     e = float(np.sum(np.square(np.asarray(residual, dtype=np.float64))))
     s = float(np.sum(np.square(np.asarray(x, dtype=np.float64))))
@@ -122,14 +127,16 @@ LONG_CASES = {
     'c5_s1': ('c5', 55, 1, 655),
     'c2_s0': ('c2', 77, 0, 1200),
 }
+# the stored config-2 toy input is split into this many consecutive parts so that every file stays under 1 MB
+C2TOY_PARTS = 3
 
 
 def long_case_inputs(name):
     """(x, D, nbNonzeroCoefs) of a long case: the seeded synthetic signals of bench.py (legacy RandomState streams), or
     the stored toy training signal for 'c2toy'."""
     if name == 'c2toy':
-        z = load_npz('c2_toy_1e6.npz')
-        return z['x'], z['D'], 1000
+        parts = [load_npz('c2_toy_1e6_part%d.npz' % i) for i in range(C2TOY_PARTS)]
+        return np.concatenate([z['x'] for z in parts]), parts[0]['D'], 1000
     import bench
     wl, seed, s, n = LONG_CASES[name]
     w = dict(bench.WORKLOADS[wl])

@@ -1,6 +1,6 @@
 """Pins `oracle/hsc_oracle.py` against the reference: golden vectors of the reference's own tests,
 traces recorded from the unmodified reference (tests/golden/*.npz, made by make_golden.py), and -
-when /root/reference is mounted - the live reference, bit for bit.  CPU only."""
+where a copy of the reference is supplied (HSC_REFERENCE_ROOT or baseline/_ref) - the live reference, bit for bit.  CPU only."""
 import os
 import sys
 
@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 import scipy.sparse
 
-from helpers import load_npz, case_kwargs, coo_sorted, GOLDEN
+from helpers import load_npz, case_kwargs, coo_sorted, stored_code, GOLDEN
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden'))
 import ref_loader  # noqa: E402
@@ -231,35 +231,30 @@ def test_ksvd_update_pca_matches_reference():
         assert alpha > 0
 
 
-# ---------------- live reference (dev container only) -------------------------------------------
+# ---------------- stored random cases, and the live reference where a copy is supplied ----------
 
-@pytest.mark.skipif(not HAVE_REF, reason='/root/reference not mounted (GPU box)')
 def test_oracle_equals_live_reference_bit_for_bit():
-    ref_loader.load_reference()
-    from hsc.modeling import ConvolutionalMatchingPursuit, LoCOMP
-    import logging
-    logging.getLogger('hsc').setLevel(logging.ERROR)
-    rs = np.random.RandomState(31337)
-    for trial in range(24):
-        T = int(rs.choice([57, 130, 300]))
-        L = int(rs.choice([3, 4, 7]))            # edge-dominated tiny cases can cycle forever in the reference
-        K = int(rs.choice([3, 8]))
-        F = int(rs.choice([1, 2, 5]))
-        dtype = rs.choice([np.float32, np.float64])
-        x = rs.randn(T, F).astype(dtype)
-        D = O.normalize(rs.randn(K, L, F)).astype(dtype)
-        if F == 1 and trial % 2 == 0:
-            x, D = x[:, 0], D[:, :, 0]
-        kw = [dict(nbNonzeroCoefs=12), dict(toleranceSnr=9.0, nbNonzeroCoefs=60), dict(toleranceSnr=6.0, nbBlocks=4, nbNonzeroCoefs=60),
-              dict(toleranceResidualScale=0.8, nbNonzeroCoefs=30), dict(toleranceSnr=7.0, nbBlocks="auto", nbNonzeroCoefs=40)][trial % 5]
-        if trial % 3 == 0:
-            kw['weights'] = np.where(np.arange(K) < max(K // 2, 1), 0.7, 1.0).astype(dtype)
-        for cls, fn in ((ConvolutionalMatchingPursuit, O.mp_encode), (LoCOMP, O.locomp_encode)):
-            c_ref, r_ref = cls().computeCoefficients(x, D, **kw)
-            c_or, r_or = fn(x, D, **kw)
-            assert (c_ref != c_or).nnz == 0, (trial, cls.__name__, kw)
-            assert np.array_equal(r_ref, r_or), (trial, cls.__name__, kw)
-            assert r_ref.dtype == r_or.dtype and r_ref.shape == r_or.shape
+    """24 small random MP / LoCOMP cases (tests/golden/oracle_trials.npz, make_golden_dropin.py): the oracle returns
+    exactly the stored codes and residuals; where a copy of the reference is supplied, so does the reference."""
+    z = load_npz('oracle_trials.npz')
+    live = None
+    if HAVE_REF:
+        ref_loader.load_reference()
+        from hsc.modeling import ConvolutionalMatchingPursuit, LoCOMP
+        import logging
+        logging.getLogger('hsc').setLevel(logging.ERROR)
+        live = {'cmp': ConvolutionalMatchingPursuit, 'locomp': LoCOMP}
+    assert int(z['count']) == 24
+    for trial in range(int(z['count'])):
+        name = 'trial%d' % trial
+        x, D, kw = z[name + '_x'], z[name + '_D'], case_kwargs(z, name)
+        for method, fn in (('cmp', O.mp_encode), ('locomp', O.locomp_encode)):
+            key = '%s_%s' % (name, method)
+            c_st, r_st = stored_code(z, key), z[key + '_res']
+            outs = [fn(x, D, **kw)] + ([live[method]().computeCoefficients(x, D, **kw)] if live else [])
+            for c, r in outs:
+                assert all(np.array_equal(a, b) for a, b in zip(coo_sorted(c), coo_sorted(c_st))), (key, kw)
+                assert r.dtype == r_st.dtype and r.shape == r_st.shape and np.array_equal(r, r_st), (key, kw)
 
 
 def test_kmeans_oracle_matches_reference_golden():
