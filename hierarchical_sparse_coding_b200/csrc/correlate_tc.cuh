@@ -10,7 +10,9 @@
 //     an 11 + 11 bit significand like 3xTF32.  2^e is a per-signal power of two that puts max|x| in [2^9, 2^10) (the
 //     dictionary gets one global power of two), the two lo products accumulate in their own TMEM columns and the
 //     epilogue forms (acc_hh + 2^-11 * acc_lo) * 2^-e: all scalings are exact.
-//   * 3xTF32 (kind::tf32): hi = tf32(x), lo = tf32(x - hi).  HSC_K1=tf32 selects it.
+//   * 3xTF32 (kind::tf32): hi = tf32(x*2^e), lo = tf32(x*2^e - hi) with the same powers of two (the tensor core flushes
+//     subnormal tf32 operands and products, so unscaled inputs below ~2^-115 lost their map), the epilogue forms
+//     (acc_hh + acc_lo) * 2^-e.  HSC_K1=tf32 selects it.
 // Below, "element" is an fp16 or fp32 operand element and R = 16 / sizeof(element) is the number of elements in a
 // 16-byte core-matrix row (8 or 4).
 //
@@ -56,10 +58,21 @@ struct Plan {            // host-side geometry of one dictionary
     int nslices;
     int slab_elems;      // R*(kTileM-1) + Kd
     int slab_stride_bytes;
-    float d_scale;       // power of two applied to the dictionary before the split (fp16: max|D| in [0.5, 1))
+    float d_scale;       // power of two applied to the dictionary before the split (max|D| in [0.5, 1))
     size_t smem_bytes;
     bool ok;
 };
+
+// Power-of-two exponent e of the operand split (3xFP16 and 3xTF32) that puts max|v| * 2^e in [2^top, 2^(top+1)): top = 9 for a signal,
+// top = -1 for the dictionary.  Clamped to [-126, 127] so that 2^e and 2^-e are finite and non-zero: an input too
+// small to reach the target range (max|x| < 2^-118, max|D| < 2^-128) is scaled by 2^127 instead, which still leaves
+// its largest element at 2^-22 or more and every float32 subnormal exactly representable in hi + lo.  In-range
+// inputs get the unclamped exponent, so their split and their map are unchanged.
+__host__ __device__ inline int split_exponent(float mx, int top) {
+    if (!(mx > 0.f) || !isfinite(mx)) return 0;
+    const int e = top - ilogbf(mx);
+    return e < -126 ? -126 : (e > 127 ? 127 : e);
+}
 
 inline Plan make_plan(int K, int L, int F, bool half, int ns_max = 128) {
     Plan p{};
@@ -109,16 +122,15 @@ constexpr float kLoScale = 2048.f;      // fp16 split: the lo part is stored tim
 // lo parts of a slice are stacked along N, [B_hi ; B_lo], so that ONE MMA of N = 2*NS computes A_hi*B_hi
 // and A_hi*B_lo while reading A_hi from shared memory once:
 //   out[((slice*(Kd/R) + kc)*2*NS + part*NS + n)*R + j] = part(B'[slice*NS + n][kc*R + j])
-// Returns raw bytes (fp32 or fp16 elements).  For fp16, p.d_scale is set to the power of two used.
+// Returns raw bytes (fp32 or fp16 elements).  p.d_scale is set to the power of two used.
 inline void build_b_operand(const float* D, int K, int L, int F, Plan& p, std::vector<unsigned char>& out) {
     const size_t n = (size_t)p.nslices * 2 * p.NS * p.Kd;
     out.assign(n * p.esz, 0);
     const int LF = L * F;
-    p.d_scale = 1.f;
-    if (p.half) {
+    {
         float mx = 0.f;
         for (size_t i = 0; i < (size_t)K * LF; ++i) mx = fmaxf(mx, fabsf(D[i]));
-        if (mx > 0.f && isfinite(mx)) p.d_scale = ldexpf(1.f, -1 - ilogbf(mx));      // max|D|*scale in [0.5, 1)
+        p.d_scale = ldexpf(1.f, split_exponent(mx, -1));      // max|D|*scale in [0.5, 1)
     }
     float* of = reinterpret_cast<float*>(out.data());
     __half* oh = reinterpret_cast<__half*>(out.data());
@@ -258,20 +270,25 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t* v) {
                  : "r"(taddr));
 }
 
-// Zero-padded 3xTF32 split of the signals: out[s][pad_front + i] = part(x[s][i]); everything else 0.
+// Zero-padded 3xTF32 split of the signals: out[s][pad_front + i] = part(x[s][i] * 2^e); everything else 0.  2^e and
+// out_scale[s] as in split_signal_half_kernel below.
 // pad_front = off*F makes the slab of tile m0 start at float 4*m0 of the padded signal (16-byte aligned),
 // and the tail padding covers the last tile plus the reduction overhang, so every slab is one in-bounds
 // contiguous chunk the TMA engine can fetch.
 __global__ void __launch_bounds__(256) split_signal_kernel(const float* __restrict__ x, float* __restrict__ hi,
                                                            float* __restrict__ lo, long long n_valid, long long stride,
-                                                           int pad_front) {
+                                                           int pad_front, const unsigned* __restrict__ absmax,
+                                                           float inv_d_scale, float* __restrict__ out_scale) {
     const long long s = blockIdx.y;
+    const int e = split_exponent(__uint_as_float(absmax[s]), 9);
+    const float sc = ldexpf(1.f, e);
+    if (blockIdx.x == 0 && threadIdx.x == 0) out_scale[s] = ldexpf(inv_d_scale, -e);
     const float* xs = x + s * n_valid;
     float* hs = hi + s * stride;
     float* ls = lo + s * stride;
     for (long long j = blockIdx.x * (long long)blockDim.x + threadIdx.x; j < stride; j += (long long)gridDim.x * blockDim.x) {
         const long long i = j - pad_front;
-        const float v = (i >= 0 && i < n_valid) ? __ldg(xs + i) : 0.f;
+        const float v = (i >= 0 && i < n_valid) ? __ldg(xs + i) * sc : 0.f;
         const float h = to_tf32(v);
         hs[j] = h;
         ls[j] = to_tf32(v - h);
@@ -296,8 +313,7 @@ __global__ void __launch_bounds__(256) split_signal_half_kernel(const float* __r
                                                                 int pad_front, const unsigned* __restrict__ absmax,
                                                                 float inv_d_scale, float* __restrict__ out_scale) {
     const long long s = blockIdx.y;
-    const float mx = __uint_as_float(absmax[s]);
-    const int e = (mx > 0.f && isfinite(mx)) ? 9 - ilogbf(mx) : 0;
+    const int e = split_exponent(__uint_as_float(absmax[s]), 9);
     const float sc = ldexpf(1.f, e);
     if (blockIdx.x == 0 && threadIdx.x == 0) out_scale[s] = ldexpf(inv_d_scale, -e);
     const float* xs = x + s * n_valid;
@@ -320,8 +336,7 @@ __global__ void __launch_bounds__(256) split_signal_half_vec8_kernel(const float
                                                                      int pad_front, const unsigned* __restrict__ absmax,
                                                                      float inv_d_scale, float* __restrict__ out_scale) {
     const long long s = blockIdx.y;
-    const float mx = __uint_as_float(absmax[s]);
-    const int e = (mx > 0.f && isfinite(mx)) ? 9 - ilogbf(mx) : 0;
+    const int e = split_exponent(__uint_as_float(absmax[s]), 9);
     const float sc = ldexpf(1.f, e);
     if (blockIdx.x == 0 && threadIdx.x == 0) out_scale[s] = ldexpf(inv_d_scale, -e);
     const float* xs = x + s * n_valid;
@@ -369,7 +384,7 @@ struct Args {
     const void* x_lo;     //                   and the 'lo' part
     long long xpad_stride;     // elements
     const void* b_op;     // [nslices][Kd/R][2*NS][R]: stacked hi / lo dictionary slices
-    const float* out_scale;    // fp16: [S] factor applied to the accumulators (2^-e / d_scale); tf32: nullptr
+    const float* out_scale;    // [S] factor applied to the accumulators (2^-e / d_scale)
     float* map;           // [S][T][K]
     int S, T, F, K, off;
     int s, Kd, Ntot, NS, nslices, slab_elems, slab_stride_bytes;
@@ -558,7 +573,7 @@ __global__ void __launch_bounds__(kThreads, 2) correlate_tc_kernel(Args a) {
             const int sig = (int)(tile / MT);
             const int m0 = (int)(tile % MT) * kTileM;
             float* ms = a.map + (long long)sig * map_elems;
-            const float osc = H ? __ldg(a.out_scale + sig) : 1.f;
+            const float osc = __ldg(a.out_scale + sig);
             constexpr float lsc = H ? (1.f / kLoScale) : 1.f;
 #ifdef HSC_PROFILE_PHASES
             long long c0_ = clock64();
@@ -588,7 +603,7 @@ __global__ void __launch_bounds__(kThreads, 2) correlate_tc_kernel(Args a) {
 #pragma unroll
                 for (int j = 0; j < 32; ++j) {
                     if constexpr (H) f[j] = fmaf(__uint_as_float(w[j]), lsc, __uint_as_float(v[j])) * osc;   // power-of-two scalings: exact
-                    else f[j] = __uint_as_float(v[j]) + __uint_as_float(w[j]);
+                    else f[j] = (__uint_as_float(v[j]) + __uint_as_float(w[j])) * osc;
                 }
                 const int col0 = slice * NS + c0;
                 if (row < Ts && col0 < a.Ntot) {

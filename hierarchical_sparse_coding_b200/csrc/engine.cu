@@ -146,12 +146,11 @@ int set_dictionary_t(hsc_engine* e, const void* D_host, const void* w_host) {
             // expanded / shifted / split dictionary operand, built on the device from the uploaded D (the padding of the
             // last slice stays zero); tc::build_b_operand is the host restatement of the same layout
             const size_t bytes = (size_t)p.nslices * 2 * p.NS * p.Kd * p.esz;
-            p.d_scale = 1.f;
-            if (p.half) {
+            {
                 float mx = 0.f;
                 const float* Dh = (const float*)D_host;
                 for (size_t i = 0; i < nD; ++i) mx = fmaxf(mx, fabsf(Dh[i]));
-                if (mx > 0.f && isfinite(mx)) p.d_scale = ldexpf(1.f, -1 - ilogbf(mx));      // max|D|*scale in [0.5, 1)
+                p.d_scale = ldexpf(1.f, tc::split_exponent(mx, -1));      // max|D|*scale in [0.5, 1)
             }
             if (!e->tc_bop) HSC_CUDA(e, cudaMalloc(&e->tc_bop, bytes));
             HSC_CUDA(e, cudaMemset(e->tc_bop, 0, bytes));
@@ -211,14 +210,14 @@ int correlate_tc(hsc_engine* e, const void* x, long long S, long long T, void* m
         if (bx > 1024) bx = 1024;
         dim3 grid(bx, (unsigned)S);
         const int pad_front = centre_offset((int)e->L) * (int)e->F;
+        HSC_CUDA(e, cudaMemsetAsync(absmax, 0, (size_t)S * 4, st));
+        // few blocks per signal: one atomicMax per warp on the signal's slot (a (1024, S) grid spent 0.6 ms in atomics)
+        const long long nval = (long long)T * e->F;
+        unsigned ax = (unsigned)((nval + 256 * 64 - 1) / (256 * 64));
+        if (ax < 1) ax = 1;
+        if (ax > 16) ax = 16;
+        tc::signal_absmax_kernel<<<dim3(ax, (unsigned)S), 256, 0, st>>>((const float*)x, nval, absmax);
         if (p.half) {
-            HSC_CUDA(e, cudaMemsetAsync(absmax, 0, (size_t)S * 4, st));
-            // few blocks per signal: one atomicMax per warp on the signal's slot (a (1024, S) grid spent 0.6 ms in atomics)
-            const long long nval = (long long)T * e->F;
-            unsigned ax = (unsigned)((nval + 256 * 64 - 1) / (256 * 64));
-            if (ax < 1) ax = 1;
-            if (ax > 16) ax = 16;
-            tc::signal_absmax_kernel<<<dim3(ax, (unsigned)S), 256, 0, st>>>((const float*)x, nval, absmax);
             static const bool scalar_split = getenv("HSC_K1_SPLIT_SCALAR") != nullptr;
             if (!scalar_split && pad_front % 4 == 0 && nval % 4 == 0 && xstride % 8 == 0 && ((uintptr_t)x & 15) == 0) {
                 unsigned gx = (unsigned)((xstride / 8 + 255) / 256);
@@ -229,15 +228,15 @@ int correlate_tc(hsc_engine* e, const void* x, long long S, long long T, void* m
                 tc::split_signal_half_kernel<<<grid, 256, 0, st>>>((const float*)x, (__half*)xhi, (__half*)xlo, nval, xstride,
                                                                    pad_front, absmax, 1.f / p.d_scale, out_scale);
             }
-            e->launches += 2;
         } else {
-            tc::split_signal_kernel<<<grid, 256, 0, st>>>((const float*)x, (float*)xhi, (float*)xlo, (long long)T * e->F, xstride, pad_front);
-            e->launches++;
+            tc::split_signal_kernel<<<grid, 256, 0, st>>>((const float*)x, (float*)xhi, (float*)xlo, nval, xstride, pad_front,
+                                                          absmax, 1.f / p.d_scale, out_scale);
         }
+        e->launches += 2;
         HSC_CUDA(e, cudaGetLastError());
     }
     a.x_hi = xhi; a.x_lo = xlo; a.xpad_stride = xstride; a.b_op = e->tc_bop; a.map = (float*)map;
-    a.out_scale = p.half ? out_scale : nullptr;
+    a.out_scale = out_scale;
     a.S = (int)S; a.T = (int)T; a.F = (int)e->F; a.K = (int)e->K; a.off = centre_offset((int)e->L);
     a.s = p.s; a.Kd = p.Kd; a.Ntot = p.Ntot; a.NS = p.NS; a.nslices = p.nslices; a.slab_elems = p.slab_elems;
     a.slab_stride_bytes = p.slab_stride_bytes;
