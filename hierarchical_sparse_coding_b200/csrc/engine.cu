@@ -553,15 +553,17 @@ int run_t(hsc_engine* e, int32_t* evp, int32_t* evi, void* evc, long long cap, c
     return HSC_OK;
 }
 
+// offsets == nullptr: one signal, atoms [0, n); otherwise S signals, atoms of signal s in [offsets[s], offsets[s+1]).
 template <typename real>
-int decode_t(hsc_engine* e, const int32_t* pos, const int32_t* idx, const void* coef, long long n, long long T, void* out,
-             cudaStream_t st) {
-    long long total = T * e->F;
-    int blocks = (int)((total + 255) / 256);
+int decode_t(hsc_engine* e, const int64_t* offsets, const int32_t* pos, const int32_t* idx, const void* coef, long long n,
+             long long S, long long T, void* out, cudaStream_t st) {
+    long long total = S * T * e->F;
+    long long blocks = (total + 255) / 256;
     if (blocks > 148 * 16) blocks = 148 * 16;
     if (blocks < 1) blocks = 1;
-    decode_gather_kernel<real><<<blocks, 256, 0, st>>>(pos, idx, (const real*)coef, n, (const real*)e->D_dev, (int)T,
-                                                        (int)e->K, (int)e->L, (int)e->F, centre_offset((int)e->L), (real*)out);
+    decode_gather_kernel<real><<<(unsigned)blocks, 256, 0, st>>>((const long long*)offsets, n, pos, idx, (const real*)coef,
+                                                                 (const real*)e->D_dev, S, (int)T, (int)e->K, (int)e->L, (int)e->F,
+                                                                 centre_offset((int)e->L), (real*)out);
     e->launches++;
     HSC_CUDA(e, cudaGetLastError());
     return HSC_OK;
@@ -849,8 +851,20 @@ int hsc_b200_decode(hsc_engine* e, const int32_t* pos_dev, const int32_t* idx_de
     if (n == 0) return HSC_OK;
     HSC_CUDA(e, cudaSetDevice(e->device));
     cudaStream_t st = (cudaStream_t)stream;
-    return e->dtype == HSC_F32 ? decode_t<float>(e, pos_dev, idx_dev, coef_dev, n, T, out_dev, st)
-                               : decode_t<double>(e, pos_dev, idx_dev, coef_dev, n, T, out_dev, st);
+    return e->dtype == HSC_F32 ? decode_t<float>(e, nullptr, pos_dev, idx_dev, coef_dev, n, 1, T, out_dev, st)
+                               : decode_t<double>(e, nullptr, pos_dev, idx_dev, coef_dev, n, 1, T, out_dev, st);
+}
+
+int hsc_b200_decode_batch(hsc_engine* e, const int64_t* offsets_dev, const int32_t* pos_dev, const int32_t* idx_dev,
+                          const void* coef_dev, int64_t S, int64_t T, void* out_dev, void* stream) {
+    if (!e) return HSC_E_INVALID;
+    if (!e->D_dev) return fail(e, HSC_E_STATE, "decode_batch: no dictionary set");
+    if (!out_dev || !offsets_dev || S <= 0 || T <= 0 || T >= (1ll << 31) || !pos_dev || !idx_dev || !coef_dev)
+        return fail(e, HSC_E_INVALID, "decode_batch: bad arguments");
+    HSC_CUDA(e, cudaSetDevice(e->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    return e->dtype == HSC_F32 ? decode_t<float>(e, offsets_dev, pos_dev, idx_dev, coef_dev, 0, S, T, out_dev, st)
+                               : decode_t<double>(e, offsets_dev, pos_dev, idx_dev, coef_dev, 0, S, T, out_dev, st);
 }
 
 int hsc_b200_copy_to_host(hsc_engine* e, const void* src_dev, void* dst_host, size_t bytes) {

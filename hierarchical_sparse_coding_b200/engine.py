@@ -821,19 +821,44 @@ class Engine(object):
     # ------------------------------------------------------------------ decoder
     @_with_stream
     def decode(self, pos, idx, coef, T, out=None, stream=None):
-        """reconstructSignal for one signal: returns the device tensor [T,F] (+= into `out` if given)."""
+        """reconstructSignal for one signal: returns the device tensor [T,F] (+= into `out` if given).  The S = 1 case of
+        decode_batch."""
         torch = _torch()
+        T = int(T)
         with torch.cuda.device(self.device):
-            pos = np.asarray(pos, dtype=np.int32)
-            order = np.argsort(pos, kind='stable')
+            if out is None:
+                out = torch.zeros((T, self.F), dtype=self.torch_dtype, device=self.device)
+            n = len(np.asarray(pos))
+            self.decode_batch(np.array([0, n], dtype=np.int64), pos, idx, coef, 1, T, out=out.view(1, T, self.F))
+        return out
+
+    @_with_stream
+    def decode_batch(self, offsets, pos, idx, coef, S, T, out=None, stream=None):
+        """reconstructSignal for S signals of length T in one launch: returns the device tensor [S,T,F] (+= into `out` if
+        given).  The atoms of signal s are entries [offsets[s], offsets[s+1]) of the flat host arrays pos / idx / coef
+        (offsets: S+1 integers from 0, the layout compact_events returns).  Each signal's atoms are put in the order decode()
+        uses (stable sort by position), so signal s gets bit for bit what decode() gives for its atoms alone."""
+        torch = _torch()
+        S, T = int(S), int(T)
+        offsets = np.asarray(offsets, dtype=np.int64)
+        pos = np.asarray(pos, dtype=np.int32)
+        assert offsets.shape == (S + 1,) and offsets[0] == 0 and np.all(np.diff(offsets) >= 0) and offsets[S] == len(pos)
+        assert len(idx) == len(pos) and len(coef) == len(pos)
+        with torch.cuda.device(self.device):
+            if out is None:
+                out = torch.zeros((S, T, self.F), dtype=self.torch_dtype, device=self.device)
+            assert out.shape == (S, T, self.F) and out.dtype == self.torch_dtype and out.is_contiguous()
+            if len(pos) == 0:
+                return out
+            # stable within each signal: the segments are already in signal order, lexsort keeps equal positions in list order
+            order = np.lexsort((pos, np.repeat(np.arange(S, dtype=np.int64), np.diff(offsets))))
+            o = torch.from_numpy(offsets).to(self.device)
             p = torch.from_numpy(np.ascontiguousarray(pos[order])).to(self.device)
             i = torch.from_numpy(np.ascontiguousarray(np.asarray(idx, dtype=np.int32)[order])).to(self.device)
             c = torch.from_numpy(np.ascontiguousarray(np.asarray(coef, dtype=self.dtype)[order])).to(self.device)
-            if out is None:
-                out = torch.zeros((T, self.F), dtype=self.torch_dtype, device=self.device)
-            N.check(self.lib, self.handle, self.lib.hsc_b200_decode(
-                self.handle, ctypes.c_void_p(p.data_ptr()), ctypes.c_void_p(i.data_ptr()), ctypes.c_void_p(c.data_ptr()),
-                int(p.numel()), int(T), ctypes.c_void_p(out.data_ptr()), self._stream_ptr(stream)))
+            N.check(self.lib, self.handle, self.lib.hsc_b200_decode_batch(
+                self.handle, ctypes.c_void_p(o.data_ptr()), ctypes.c_void_p(p.data_ptr()), ctypes.c_void_p(i.data_ptr()),
+                ctypes.c_void_p(c.data_ptr()), S, T, ctypes.c_void_p(out.data_ptr()), self._stream_ptr(stream)))
         return out
 
 

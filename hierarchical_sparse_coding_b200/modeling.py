@@ -14,10 +14,15 @@ device raises.
 
 New entry points (the reference encodes one signal per call, :1664): `computeCoefficientsBatch` /
 `encodeBatch` take [B,T,F] and shard nothing themselves - see `distributed.py` for the multi-GPU
-partition by independent signals.
+partition by independent signals.  The hierarchical coder has them too: one level loop
+(`HierarchicalConvolutionalMatchingPursuit._forward_batch`) runs B sequences of one length through every
+level at once and `computeCoefficients` is its B = 1 call, so a sequence's codes and residual in a batch
+are bit for bit those of its own call.  `reconstructBatch` decodes B codes in one launch
+(`Engine.decode_batch`, the kernel behind `Engine.decode` too).
 """
 import collections.abc
 import copy
+import ctypes
 import logging
 
 import numpy as np
@@ -112,6 +117,45 @@ def reconstructSignal(coefficients, D, device=None):
     keep = cx.data != 0.0
     sig = eng.decode(cx.row[keep], cx.col[keep], cx.data[keep], cx.shape[0]).cpu().numpy().astype(out_dtype)
     return sig[:, 0] if squeeze else sig
+
+
+def _events_to_csc(pos, idx, coef, T, K):
+    """One signal's events of one level -> the reference's csc [T,K] float64 (hsc/modeling.py:1180-1186): duplicates summed
+    in selection order, |x| < 1e-16 dropped, zeros eliminated."""
+    m = scipy.sparse.coo_matrix((coef.astype(np.float64), (pos.astype(np.int64), idx.astype(np.int64))), shape=(T, K)).tocsc()
+    m.sum_duplicates()
+    m.data[np.abs(m.data) < 1e-16] = 0.0
+    m.eliminate_zeros()
+    return m
+
+
+def _decode_codes(eng, codes, T, out):
+    """out [S,T,F] (device) += the reconstruction of S codes (csc / any sparse [T,K]) with eng's dictionary, one decoder
+    launch.  Each code's atoms are its coo's nonzero entries, the list reconstructSignal decodes."""
+    pos, idx, coef = [], [], []
+    offsets = np.zeros(len(codes) + 1, dtype=np.int64)
+    for s, c in enumerate(codes):
+        cx = scipy.sparse.coo_matrix(c)
+        assert cx.shape[0] == T, 'every code must have %d rows' % T
+        keep = cx.data != 0.0
+        pos.append(cx.row[keep])
+        idx.append(cx.col[keep])
+        coef.append(cx.data[keep])
+        offsets[s + 1] = offsets[s] + int(np.count_nonzero(keep))
+    cat = lambda a, dt: np.concatenate(a).astype(dt, copy=False) if a else np.zeros(0, dt)
+    return eng.decode_batch(offsets, cat(pos, np.int32), cat(idx, np.int32), cat(coef, eng.dtype), len(codes), T, out=out)
+
+
+def _reconstruct_batch(codes, D, device=None):
+    """reconstructSignal for B codes of one shape [T,K] with dictionary D, one decoder launch."""
+    D = np.asarray(D)
+    assert D.ndim == 2 or D.ndim == 3
+    eng = get_engine(device)
+    eng.set_dictionary(D, dtype=np.float64)
+    dt = np.result_type(*[c.dtype for c in codes])
+    out_dtype = dt if dt in (np.float32, np.float64) else np.float64
+    sig = _decode_codes(eng, codes, codes[0].shape[0], None).cpu().numpy().astype(out_dtype)
+    return sig[:, :, 0] if D.ndim == 2 else sig
 
 
 def normalize(X, axis=None):
@@ -488,36 +532,33 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
         raise Exception('Unsupported sparse coding method: %s' % (self.method))
 
     def _forward(self, sequence, coefficients, multilevelDict, toleranceSnr, nbBlocks, singletonWeight):
-        """The forward phase (:1432-1492 / :1494-1554) with the level hand-off ON THE DEVICE: level l's events stay in
-        device memory, hsc_b200_mp_events_to_dense turns them into the dense float64 code map that is level l+1's
-        K_l-channel input (:1489), and every level's dictionary lives in its own native engine, so nothing is uploaded
-        twice.  The host reads all levels' events once, at the end, and builds the csc matrices the reference returns."""
-        import torch
+        """The forward phase (:1432-1492 / :1494-1554) of one sequence: the B = 1 call of _forward_batch.  With given
+        `coefficients` (computeCoefficientsFromLevel) the loop starts at the next level, its input the dense map of the last
+        given level (:1498)."""
+        given = list(coefficients)
+        x0 = np.asarray(sequence) if len(given) == 0 else np.asarray(given[-1].todense())
+        x0 = x0[:, None] if x0.ndim == 1 else x0
+        return self._forward_batch(x0[None], given, multilevelDict, toleranceSnr, nbBlocks, singletonWeight)[0]
+
+    def _forward_batch(self, x, given, multilevelDict, toleranceSnr, nbBlocks, singletonWeight):
+        """The forward phase of B independent sequences x [B,T,F] (the input of level len(given)) with the level hand-off ON
+        THE DEVICE: level l's events stay in device memory, hsc_b200_mp_events_to_dense turns them into the dense float64
+        code map that is level l+1's K_l-channel input (:1489), and every level's dictionary lives in its own native engine,
+        so nothing is uploaded twice.  The signals run in chunks that fit the device (_chunk_size); per chunk the host reads
+        every level's events once, at the end, and builds the csc matrices the reference returns.  Returns one list per
+        sequence: the given codes followed by one csc [T,K_l] per encoded level."""
         if self.method == 'cmp':
             meth = 0
         elif self.method == 'locomp':
             meth = 1
         else:
             raise Exception('Unsupported sparse coding method: %s' % (self.method))
-        sequence = np.asarray(sequence)
-        T = sequence.shape[0] if len(coefficients) == 0 else coefficients[-1].shape[0]
-        given = list(coefficients)
-        cap_scale = 1
-        while True:
-            try:
-                return self._forward_once(sequence, list(given), multilevelDict, toleranceSnr, nbBlocks, singletonWeight, meth, T, cap_scale)
-            except _CapacityExhausted:
-                # a level wrote more events than its buffers hold (LoCOMP emits one event per refitted group atom): the
-                # later levels saw a truncated code, so the whole forward phase is repeated with larger buffers
-                cap_scale *= 8
-                if cap_scale > 4096:
-                    raise N.HscError(N.HSC_E_NOMEM, 'hierarchical encode: event buffers exhausted')
-
-    def _forward_once(self, sequence, coefficients, multilevelDict, toleranceSnr, nbBlocks, singletonWeight, meth, T, cap_scale):
-        import torch
-        xd = None
-        levels = []              # (engine, evp, evi, evc, K) per encoded level
-        for level in range(len(coefficients), multilevelDict.getNbLevels()):
+        B, T = x.shape[0], x.shape[1]
+        out = [list(given) for _ in range(B)]
+        if len(given) >= multilevelDict.getNbLevels() or B == 0:
+            return out
+        specs = []               # (D, weights, engine dtype, options, K, level) per encoded level
+        for level in range(len(given), multilevelDict.getNbLevels()):
             if toleranceSnr is not None and isinstance(toleranceSnr, collections.abc.Iterable):
                 targetSnr = toleranceSnr[level]
             else:
@@ -527,47 +568,90 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
             nbSingletons = D.shape[0] - multilevelDict.countsNoSingletons[level]
             weights = np.ones((D.shape[0],), dtype=D.dtype)                     # :1448-1450
             weights[:nbSingletons] = singletonWeight
-            if xd is None:
-                # first level to encode: the input sequence, or the dense map of the last given level (:1498)
-                x0 = sequence if len(coefficients) == 0 else np.asarray(coefficients[-1].todense())
-                x0 = x0[:, None] if x0.ndim == 1 else x0
-                dt = engine_dtype(x0, D)
-                eng = engine_for_dictionary(D, weights, dt, self.device)
-                xd = torch.from_numpy(np.ascontiguousarray(x0[None], dtype=dt)).to(eng.device)
-            else:
-                dt = engine_dtype(np.zeros(0, np.float64), D)                    # the dense code map is float64 (:1489)
-                eng = engine_for_dictionary(D, weights, dt, self.device)
-            assert xd.shape[2] == eng.F, 'level %d: the dictionary has %d channels, its input %d' % (level, eng.F, xd.shape[2])
+            # the first level encodes the input; later levels the dense code map, which is float64 (:1489)
+            dt = engine_dtype(x, D) if not specs else engine_dtype(np.zeros(0, np.float64), D)
+            eng = engine_for_dictionary(D, weights, dt, self.device)
             opt = eng.make_options(None, None, targetSnr, nbBlocks, 1e-16, use_weights=True, coef_mode=self.coef_mode, method=meth,
                                    energy_eps=_dict_eps(D))
-            cap = eng.default_capacity(opt, T) * cap_scale
-            evp, evi, evc, _, _ = eng.encode_device(xd, opt, cap, sync_states=False)
-            levels.append((eng, evp, evi, evc, D.shape[0]))
-            if level + 1 < multilevelDict.getNbLevels():
-                xd = eng.events_to_dense(evp, evi, evc, 1e-16)
-        # one synchronisation: states + events of every level
-        for (eng, evp, evi, evc, K) in levels:
-            states = (N.SignalState * 1)()
-            N.check(eng.lib, eng.handle, eng.lib.hsc_b200_mp_states(eng.handle, states, eng._stream_ptr()))
-            st = states[0]
-            if st.status == N.HSC_STOP_GROUP:
-                raise NotImplementedError('LoCOMP: a selection has more than 255 common-support atoms; the device refit '
-                                          'holds groups of at most 256')
-            if st.status in (N.HSC_PAUSE_CAPACITY, N.HSC_PAUSE_PASSES, N.HSC_RUNNING):
-                raise _CapacityExhausted()
-            n = int(st.n_buffered)
-            p = evp[0, :n].cpu().numpy().astype(np.int64)
-            i = evi[0, :n].cpu().numpy().astype(np.int64)
-            c = evc[0, :n].cpu().numpy().astype(np.float64)
-            m = scipy.sparse.coo_matrix((c, (p, i)), shape=(T, K)).tocsc()
-            m.sum_duplicates()
-            m.data[np.abs(m.data) < 1e-16] = 0.0
-            m.eliminate_zeros()
-            coefficients.append(m)
+            specs.append((D, weights, dt, opt, D.shape[0], level))
+        self._encode_chunks(x, 0, B, specs, 1, out)
+        for (D, weights, dt, _, _, _) in specs:
+            eng = engine_for_dictionary(D, weights, dt, self.device)
             ws = getattr(eng, '_ws_cache', None)
             if ws is not None and ws.numel() > (256 << 20):      # the per-level engines outlive the call: do not pin large maps
                 eng._ws_cache = eng._last_workspace = None
-        return coefficients
+        return out
+
+    def _chunk_size(self, T, specs, cap_scale):
+        """Signals per chunk: every level's workspace, its input and residual, the dense hand-off [S,T,K_l] float64 and the
+        event buffers (padded and compacted) of all levels fit 80 % of the free device memory; at most 65535 signals
+        (hsc_b200_mp_begin)."""
+        import torch
+        per = 0
+        eng = None
+        for (D, weights, dt, opt, K, _) in specs:
+            eng = engine_for_dictionary(D, weights, dt, self.device)
+            cap = eng.default_capacity(opt, T) * cap_scale
+            per += eng.workspace_bytes(1, T) + 2 * T * eng.F * eng.dtype.itemsize + T * K * 8 + 2 * cap * (8 + eng.dtype.itemsize)
+        free, _ = torch.cuda.mem_get_info(eng.device)
+        free += torch.cuda.memory_reserved(eng.device) - torch.cuda.memory_allocated(eng.device)
+        return int(max(1, min(65535, int(free * 0.8) // per)))
+
+    def _encode_chunks(self, x, lo, hi, specs, cap_scale, out):
+        if cap_scale > 4096:
+            raise N.HscError(N.HSC_E_NOMEM, 'hierarchical encode: event buffers exhausted')
+        T = x.shape[1]
+        n = self._chunk_size(T, specs, cap_scale)
+        for a in range(lo, hi, n):
+            b = min(hi, a + n)
+            try:
+                levels = self._forward_chunk(x[a:b], specs, cap_scale)
+            except _CapacityExhausted:
+                # a level wrote more events than its buffers hold (LoCOMP emits one event per refitted group atom): the
+                # later levels saw a truncated code, so the chunk's forward phase is repeated with larger buffers
+                self._encode_chunks(x, a, b, specs, cap_scale * 8, out)
+                continue
+            for (K, off, p, i, c) in levels:
+                for s in range(b - a):
+                    out[a + s].append(_events_to_csc(p[off[s]:off[s + 1]], i[off[s]:off[s + 1]], c[off[s]:off[s + 1]], T, K))
+
+    def _forward_chunk(self, x, specs, cap_scale):
+        """All levels of S <= 65535 signals x [S,T,F].  Right after a level's run, on the same stream, its events are compacted
+        into buffers this call owns and its states copied to pinned memory, so that a later level cannot overwrite them even
+        when two levels share one cached engine.  One synchronisation after the last level; then one read per level of the
+        offsets and the flat event arrays.  Returns (K, offsets, pos, idx, coef) host arrays per level."""
+        import torch
+        S, T = x.shape[0], x.shape[1]
+        xd = None
+        pending = []
+        for li, (D, weights, dt, opt, K, level) in enumerate(specs):
+            eng = engine_for_dictionary(D, weights, dt, self.device)
+            if xd is None:
+                xd = torch.from_numpy(np.ascontiguousarray(x, dtype=dt)).to(eng.device)
+            assert xd.shape[2] == eng.F, 'level %d: the dictionary has %d channels, its input %d' % (level, eng.F, xd.shape[2])
+            cap = eng.default_capacity(opt, T) * cap_scale
+            evp, evi, evc, _, _ = eng.encode_device(xd, opt, cap, sync_states=False)
+            flat = eng.compact_events(evp, evi, evc)
+            hstate = torch.empty((S * ctypes.sizeof(N.SignalState),), dtype=torch.uint8, pin_memory=True)
+            states = (N.SignalState * S).from_address(hstate.data_ptr())
+            N.check(eng.lib, eng.handle, eng.lib.hsc_b200_mp_states_async(eng.handle, states, eng._stream_ptr()))
+            pending.append((K, flat, hstate, states))
+            if li + 1 < len(specs):
+                xd = eng.events_to_dense(evp, evi, evc, 1e-16)
+        torch.cuda.current_stream(xd.device).synchronize()
+        levels = []
+        for (K, flat, hstate, states) in pending:
+            status = np.ctypeslib.as_array(states)['status']
+            if np.any(status == N.HSC_STOP_GROUP):
+                raise NotImplementedError('LoCOMP: a selection has more than 255 common-support atoms; the device refit '
+                                          'holds groups of at most 256')
+            if np.any((status == N.HSC_PAUSE_CAPACITY) | (status == N.HSC_PAUSE_PASSES) | (status == N.HSC_RUNNING)):
+                raise _CapacityExhausted()
+            off = flat['offsets'].cpu().numpy()
+            n = int(off[S])
+            levels.append((K, off, flat['pos'][:n].cpu().numpy(), flat['idx'][:n].cpu().numpy(),
+                           flat['coef'][:n].cpu().numpy()))
+        return levels
 
     def convertToDistributedCoefficients(self, coefficients):
         """:1556-1594.  The singleton (pass-through) columns [0, K_l) of the LAST level's code are the events of level l: they
@@ -595,28 +679,30 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
         return out
 
     def _calculateResidual(self, sequence, coefficients, multilevelDict):
-        """:1596-1611: sequence - sum over the levels of decode(code_l, input-level representations of level l).  The
-        reconstruction is accumulated in ONE float64 device buffer by the decoder kernel (each level's representations
-        live in their own engine), subtracted on the device and read back once."""
+        """:1596-1611 for one sequence: the B = 1 call of _calculateResidualBatch."""
+        T = coefficients[0].shape[0]
+        return self._calculateResidualBatch(np.asarray(sequence).reshape(1, T, -1), [coefficients], multilevelDict)[0]
+
+    def _calculateResidualBatch(self, sequences, codes, multilevelDict):
+        """:1596-1611 for B sequences [B,T,F] and their codes (one list of per-level csc per sequence): sequence - sum over
+        the levels of decode(code_l, input-level representations of level l).  Per level, the codes of all sequences go
+        into one decoder launch (each level's representations live in their own engine) that accumulates into ONE float64
+        device buffer [B,T,F]; the input is subtracted on the device and read back once.  Float64 [B,T] if the base
+        dictionary is 2-D, else [B,T,F]."""
         import torch
         baseDict = multilevelDict.getBaseDictionary()
-        T = coefficients[0].shape[0]
+        B = len(codes)
+        T = codes[0][0].shape[0]
         representations = multilevelDict.getMultiscaleDictionaries()
         recon = None
-        dev = None
         for level in range(multilevelDict.getNbLevels()):
-            cx = scipy.sparse.coo_matrix(coefficients[level])
-            keep = cx.data != 0.0
             eng = engine_for_dictionary(representations[level], None, np.float64, self.device)
             if recon is None:
-                dev = eng.device
-                recon = torch.zeros((T, eng.F), dtype=torch.float64, device=dev)
-            if np.any(keep):
-                eng.decode(cx.row[keep], cx.col[keep], cx.data[keep], T, out=recon)
-        x = np.asarray(sequence)
-        xd = torch.from_numpy(np.ascontiguousarray(x.reshape(T, -1), dtype=np.float64)).to(dev)
+                recon = torch.zeros((B, T, eng.F), dtype=torch.float64, device=eng.device)
+            _decode_codes(eng, [c[level] for c in codes], T, recon)
+        xd = torch.from_numpy(np.ascontiguousarray(np.asarray(sequences).reshape(B, T, -1), dtype=np.float64)).to(recon.device)
         residual = (xd - recon).cpu().numpy()
-        return residual[:, 0] if baseDict.ndim == 2 else residual
+        return residual[:, :, 0] if baseDict.ndim == 2 else residual
 
     def _postprocessCoefficients(self, coefficients, multilevelDict, returnDistributed=True):
         if returnDistributed:
@@ -637,6 +723,25 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
         coefficients = self._postprocessCoefficients(coefficients, multilevelDict, returnDistributed)
         residual = self._calculateResidual(np.asarray(sequence), coefficients, multilevelDict)
         return coefficients, residual
+
+    def computeCoefficientsBatch(self, sequences, multilevelDict, nbNonzeroCoefs=None, toleranceResidualScale=None,
+                                 toleranceSnr=None, nbBlocks=1, minCoefficients=None, singletonWeight=0.5, returnDistributed=True):
+        """computeCoefficients for B independent sequences [B,T] or [B,T,F] of one length: returns a list of B per-level lists
+        of float64 csc matrices and the float64 residual [B,T] or [B,T,F] (the shape rule of computeCoefficients).  Every
+        argument means what it means there (nbNonzeroCoefs, toleranceResidualScale and minCoefficients are ignored there
+        too).  Each sequence gets bit for bit the codes and residual of its own computeCoefficients call: the levels run on
+        all sequences of a chunk at once, the pursuit one CTA per sequence."""
+        assert _is_multilevel_dictionary(multilevelDict)
+        sequences = np.asarray(sequences)
+        assert sequences.ndim == 2 or sequences.ndim == 3
+        x = sequences[:, :, None] if sequences.ndim == 2 else sequences
+        codes = self._forward_batch(x, [], multilevelDict, toleranceSnr, nbBlocks, singletonWeight)
+        codes = [self._postprocessCoefficients(c, multilevelDict, returnDistributed) for c in codes]
+        if len(codes) == 0:
+            F = np.asarray(multilevelDict.getBaseDictionary()).shape[2:]
+            return codes, np.zeros((0, x.shape[1]) + F, dtype=np.float64)
+        residual = self._calculateResidualBatch(x, codes, multilevelDict)
+        return codes, residual
 
     def computeCoefficientsFromLevel(self, sequence, coefficients, multilevelDict, nbNonzeroCoefs=None,
                                      toleranceResidualScale=None, toleranceSnr=None, nbBlocks=1, minCoefficients=None,
@@ -667,6 +772,12 @@ class ConvolutionalSparseCoder(object):
         assert coefficients.ndim == 1 or coefficients.ndim == 2
         return reconstructSignal(coefficients, self.D, device=getattr(self.approximator, 'device', None))
 
+    def reconstructBatch(self, codes):
+        """reconstruct for B codes of one shape [T,K] in one decoder launch: [B,T] (2-D dictionary) or [B,T,F], each row
+        bit for bit reconstruct(codes[b]), in the dtype reconstruct gives (the codes' float dtype, else float64)."""
+        assert len(codes) > 0 and all(c.ndim == 2 and c.shape == codes[0].shape for c in codes)
+        return _reconstruct_batch(codes, self.D, getattr(self.approximator, 'device', None))
+
 
 class HierarchicalConvolutionalSparseCoder(object):
     """hsc/modeling.py:1671-1705."""
@@ -682,6 +793,10 @@ class HierarchicalConvolutionalSparseCoder(object):
         assert sequence.ndim == 1 or sequence.ndim == 2
         return self.approximator.computeCoefficients(sequence, self.multilevelDict, *args, **kwargs)
 
+    def encodeBatch(self, X, *args, **kwargs):
+        assert X.ndim == 2 or X.ndim == 3
+        return self.approximator.computeCoefficientsBatch(X, self.multilevelDict, *args, **kwargs)
+
     def encodeFromLevel(self, sequence, coefficients, *args, **kwargs):
         assert len(coefficients) > 0
         return self.approximator.computeCoefficientsFromLevel(sequence, coefficients, self.multilevelDict, *args, **kwargs)
@@ -695,4 +810,17 @@ class HierarchicalConvolutionalSparseCoder(object):
         for level in range(self.multilevelDict.getNbLevels()):
             signal += reconstructSignal(coefficients[level], representations[level],
                                         device=getattr(self.approximator, 'device', None))
+        return signal
+
+    def reconstructBatch(self, codes):
+        """reconstruct for B sequences' per-level codes (as encodeBatch returns them): one decoder launch per level, the
+        levels summed on the host in level order like reconstruct, so each row is bit for bit reconstruct(codes[b])."""
+        assert len(codes) > 0 and all(len(c) == self.multilevelDict.getNbLevels() for c in codes)
+        representations = self.multilevelDict.getMultiscaleDictionaries()
+        signal = None
+        for level in range(self.multilevelDict.getNbLevels()):
+            lvl = _reconstruct_batch([c[level] for c in codes], representations[level], getattr(self.approximator, 'device', None))
+            if signal is None:
+                signal = np.zeros(lvl.shape, dtype=codes[0][0].dtype)
+            signal += lvl
         return signal

@@ -201,6 +201,15 @@ const void* hsc_b200_mp_map_dev(const hsc_engine* e);
 int hsc_b200_decode(hsc_engine* e, const int32_t* pos_dev, const int32_t* idx_dev, const void* coef_dev, int64_t n,
                     int64_t T, void* out_dev, void* stream);
 
+/* The same decoder for S signals of length T in one launch: out_dev[S][T][F] += the reconstruction of every signal.  The
+ * atoms of signal s are entries [offsets_dev[s], offsets_dev[s+1]) of the flat device lists pos_dev / idx_dev / coef_dev,
+ * sorted by centre position within the signal; offsets_dev[S+1] (int64, non-decreasing, offsets_dev[0] = 0) is the layout
+ * hsc_b200_mp_compact_events writes.  Empty segments are legal.  Each sample sums its own signal's atoms in list order in
+ * float64, so signal s gets bit for bit what hsc_b200_decode gives for its atoms alone.  hsc_b200_decode is the S = 1
+ * case.  HSC_E_INVALID for a NULL pointer, S <= 0 or T outside [1, 2^31); HSC_E_STATE without a dictionary.  Asynchronous. */
+int hsc_b200_decode_batch(hsc_engine* e, const int64_t* offsets_dev, const int32_t* pos_dev, const int32_t* idx_dev,
+                          const void* coef_dev, int64_t S, int64_t T, void* out_dev, void* stream);
+
 /* Convenience, host buffers end to end (allocates and frees its own device memory, synchronous):
  * x_host[S][T][F] -> residual_host[S][T][F], events [S][capacity], counts_host[S], states_host[S]
  * (either may be NULL).  Returns HSC_E_NOMEM if a signal needs more than `capacity` events. */
