@@ -31,7 +31,7 @@ EXPORTED_SYMBOLS = [
     'hsc_b200_mp_map_dev', 'hsc_b200_decode', 'hsc_b200_mp_encode_host', 'hsc_b200_launch_count', 'hsc_b200_copy_to_host', 'hsc_b200_create_view',
     'hsc_b200_mp_states_async', 'hsc_b200_mp_begin_part', 'hsc_b200_ksvd_update', 'hsc_b200_ksvd_set_pca', 'hsc_b200_kmeans_assign',
     'hsc_b200_ksvd_begin', 'hsc_b200_ksvd_filter_gram', 'hsc_b200_ksvd_filter_finish', 'hsc_b200_ksvd_end',
-    'hsc_b200_mp_compact_events', 'hsc_b200_mp_events_to_dense', 'hsc_b200_decode_batch',
+    'hsc_b200_mp_compact_events', 'hsc_b200_mp_events_to_dense', 'hsc_b200_decode_batch', 'hsc_b200_canonicalize_codes',
 ]
 
 
@@ -125,6 +125,9 @@ def load_library():
     lib.hsc_b200_decode.argtypes = [vp, vp, vp, vp, i64, i64, vp, vp]
     lib.hsc_b200_decode_batch.restype = ctypes.c_int
     lib.hsc_b200_decode_batch.argtypes = [vp, vp, vp, vp, vp, i64, i64, vp, vp]
+    lib.hsc_b200_canonicalize_codes.restype = ctypes.c_int
+    lib.hsc_b200_canonicalize_codes.argtypes = [vp, vp, vp, vp, vp, i64, i64, i64, i64, ctypes.POINTER(i64), i64, ctypes.c_double,
+                                                vp, vp, vp, vp, vp]
     lib.hsc_b200_mp_encode_host.restype = ctypes.c_int
     lib.hsc_b200_mp_encode_host.argtypes = [vp, vp, i64, i64, ctypes.POINTER(MpOptions), vp, vp, vp, i64, vp, vp,
                                             ctypes.POINTER(SignalState)]

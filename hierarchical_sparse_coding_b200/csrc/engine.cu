@@ -95,6 +95,8 @@ struct hsc_engine {
     size_t ksvd_scratch_bytes = 0;
     double* locomp_scratch = nullptr;     // [S][256*257] doubles, allocated at the first LoCOMP run
     size_t locomp_scratch_signals = 0;
+    unsigned char* canon_scratch = nullptr;   // hsc_b200_canonicalize_codes: sort keys of long signals, per-level counts
+    size_t canon_scratch_bytes = 0;
     long long launches = 0;
     // encode in flight
     bool active = false;
@@ -569,6 +571,35 @@ int decode_t(hsc_engine* e, const int64_t* offsets, const int32_t* pos, const in
     return HSC_OK;
 }
 
+template <typename real>
+int canonicalize_t(hsc_engine* e, const int64_t* offsets, const int32_t* pos, const int32_t* idx, const void* coef, long long capacity,
+                   long long S, long long K, const events::LevelBounds& lb, double min_coef, int64_t* out_offsets, int32_t* out_pos,
+                   int32_t* out_idx, double* out_coef, cudaStream_t st) {
+    const long long L = lb.n + 1;
+    const size_t off_ev = align_up((size_t)capacity * sizeof(long long));
+    const size_t off_counts = off_ev + align_up((size_t)capacity * sizeof(int));
+    const size_t need = off_counts + (size_t)L * S * sizeof(long long);
+    if (e->canon_scratch_bytes < need) {          // grows only (cudaFree waits for the launches that may still use it)
+        if (e->canon_scratch) cudaFree(e->canon_scratch);
+        e->canon_scratch = nullptr; e->canon_scratch_bytes = 0;
+        HSC_CUDA(e, cudaMalloc(&e->canon_scratch, need));
+        e->canon_scratch_bytes = need;
+    }
+    long long* gkey = (long long*)e->canon_scratch;
+    int* gev = (int*)(e->canon_scratch + off_ev);
+    long long* counts = (long long*)(e->canon_scratch + off_counts);
+    events::canonical_codes_kernel<real, false><<<(unsigned)S, events::CANON_THREADS, 0, st>>>(
+        (const long long*)offsets, pos, idx, (const real*)coef, capacity, (int)S, K, lb, min_coef, gkey, gev, counts, nullptr, nullptr,
+        nullptr, nullptr);
+    events::level_offsets_kernel<<<(unsigned)L, 1024, 0, st>>>(counts, (int)S, (long long*)out_offsets);
+    events::canonical_codes_kernel<real, true><<<(unsigned)S, events::CANON_THREADS, 0, st>>>(
+        (const long long*)offsets, pos, idx, (const real*)coef, capacity, (int)S, K, lb, min_coef, gkey, gev, counts,
+        (const long long*)out_offsets, out_pos, out_idx, out_coef);
+    e->launches += 3;
+    HSC_CUDA(e, cudaGetLastError());
+    return HSC_OK;
+}
+
 // Scratch that does not depend on the dictionary (split-signal staging of K1, LoCOMP / K-SVD scratch): kept across
 // hsc_b200_set_dictionary calls - a learning loop sets a new dictionary every iteration - and released with the engine.
 void free_scratch(hsc_engine* e) {
@@ -580,6 +611,8 @@ void free_scratch(hsc_engine* e) {
     e->locomp_scratch = nullptr; e->locomp_scratch_signals = 0;
     if (e->tc_xsplit) cudaFree(e->tc_xsplit);
     e->tc_xsplit = nullptr; e->tc_xsplit_bytes = 0;
+    if (e->canon_scratch) cudaFree(e->canon_scratch);
+    e->canon_scratch = nullptr; e->canon_scratch_bytes = 0;
 }
 
 void free_dictionary(hsc_engine* e) {
@@ -865,6 +898,31 @@ int hsc_b200_decode_batch(hsc_engine* e, const int64_t* offsets_dev, const int32
     cudaStream_t st = (cudaStream_t)stream;
     return e->dtype == HSC_F32 ? decode_t<float>(e, offsets_dev, pos_dev, idx_dev, coef_dev, 0, S, T, out_dev, st)
                                : decode_t<double>(e, offsets_dev, pos_dev, idx_dev, coef_dev, 0, S, T, out_dev, st);
+}
+
+int hsc_b200_canonicalize_codes(hsc_engine* e, const int64_t* offsets_dev, const int32_t* pos_dev, const int32_t* idx_dev,
+                                const void* coef_dev, int64_t capacity, int64_t S, int64_t T, int64_t K,
+                                const int64_t* level_bounds_host, int64_t n_bounds, double min_coefficients, int64_t* out_offsets_dev,
+                                int32_t* out_pos_dev, int32_t* out_idx_dev, double* out_coef_dev, void* stream) {
+    if (!e) return HSC_E_INVALID;
+    if (!e->D_dev) return fail(e, HSC_E_STATE, "canonicalize_codes: no dictionary set (it fixes the coefficient dtype)");
+    if (!offsets_dev || !out_offsets_dev || S <= 0 || S > 65535 || T <= 0 || T >= (1ll << 31) || K <= 0 || K >= (1ll << 31) ||
+        capacity < 0 || n_bounds < 0 || n_bounds >= events::CANON_MAX_LEVELS || (n_bounds > 0 && !level_bounds_host) ||
+        (capacity > 0 && (!pos_dev || !idx_dev || !coef_dev || !out_pos_dev || !out_idx_dev || !out_coef_dev)))
+        return fail(e, HSC_E_INVALID, "canonicalize_codes: bad arguments");
+    events::LevelBounds lb{};
+    lb.n = (int)n_bounds;
+    for (int64_t j = 0; j < n_bounds; ++j) {
+        if (level_bounds_host[j] < 0 || (j > 0 && level_bounds_host[j] < level_bounds_host[j - 1]))
+            return fail(e, HSC_E_INVALID, "canonicalize_codes: level bounds must be non-negative and non-decreasing");
+        lb.b[j] = level_bounds_host[j];
+    }
+    HSC_CUDA(e, cudaSetDevice(e->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    return e->dtype == HSC_F32 ? canonicalize_t<float>(e, offsets_dev, pos_dev, idx_dev, coef_dev, capacity, S, K, lb, min_coefficients,
+                                                       out_offsets_dev, out_pos_dev, out_idx_dev, out_coef_dev, st)
+                               : canonicalize_t<double>(e, offsets_dev, pos_dev, idx_dev, coef_dev, capacity, S, K, lb, min_coefficients,
+                                                        out_offsets_dev, out_pos_dev, out_idx_dev, out_coef_dev, st);
 }
 
 int hsc_b200_copy_to_host(hsc_engine* e, const void* src_dev, void* dst_host, size_t bytes) {

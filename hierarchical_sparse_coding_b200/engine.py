@@ -847,8 +847,8 @@ class Engine(object):
         with torch.cuda.device(self.device):
             if out is None:
                 out = torch.zeros((S, T, self.F), dtype=self.torch_dtype, device=self.device)
-            assert out.shape == (S, T, self.F) and out.dtype == self.torch_dtype and out.is_contiguous()
             if len(pos) == 0:
+                assert out.shape == (S, T, self.F) and out.dtype == self.torch_dtype and out.is_contiguous()
                 return out
             # stable within each signal: the segments are already in signal order, lexsort keeps equal positions in list order
             order = np.lexsort((pos, np.repeat(np.arange(S, dtype=np.int64), np.diff(offsets))))
@@ -856,10 +856,60 @@ class Engine(object):
             p = torch.from_numpy(np.ascontiguousarray(pos[order])).to(self.device)
             i = torch.from_numpy(np.ascontiguousarray(np.asarray(idx, dtype=np.int32)[order])).to(self.device)
             c = torch.from_numpy(np.ascontiguousarray(np.asarray(coef, dtype=self.dtype)[order])).to(self.device)
+            return self.decode_batch_device(o, p, i, c, S, T, out)
+
+    @_with_stream
+    def decode_batch_device(self, offsets, pos, idx, coef, S, T, out, stream=None):
+        """decode_batch for atoms already on the device and in decode order: out [S,T,F] (device, engine dtype) += the
+        reconstruction of S signals whose atoms are entries [offsets[s], offsets[s+1]) of the device tensors pos / idx
+        (int32) / coef (engine dtype), sorted by position within each signal (the order canonicalize_codes writes).  One
+        launch, no host work on the atoms.  Asynchronous; returns out."""
+        torch = _torch()
+        S, T = int(S), int(T)
+        assert out.shape == (S, T, self.F) and out.dtype == self.torch_dtype and out.is_contiguous() and out.device == self.device
+        assert offsets.shape == (S + 1,) and offsets.dtype == torch.int64 and offsets.device == self.device
+        assert pos.dtype == torch.int32 and idx.dtype == torch.int32 and coef.dtype == self.torch_dtype
+        assert all(t.device == self.device and t.is_contiguous() for t in (pos, idx, coef))
+        if pos.numel() == 0:
+            return out
+        with torch.cuda.device(self.device):
             N.check(self.lib, self.handle, self.lib.hsc_b200_decode_batch(
-                self.handle, ctypes.c_void_p(o.data_ptr()), ctypes.c_void_p(p.data_ptr()), ctypes.c_void_p(i.data_ptr()),
-                ctypes.c_void_p(c.data_ptr()), S, T, ctypes.c_void_p(out.data_ptr()), self._stream_ptr(stream)))
+                self.handle, ctypes.c_void_p(offsets.data_ptr()), ctypes.c_void_p(pos.data_ptr()), ctypes.c_void_p(idx.data_ptr()),
+                ctypes.c_void_p(coef.data_ptr()), S, T, ctypes.c_void_p(out.data_ptr()), self._stream_ptr(stream)))
         return out
+
+    @_with_stream
+    def canonicalize_codes(self, offsets, pos, idx, coef, S, T, K, level_bounds=None, min_coefficients=1e-16, stream=None):
+        """Canonical codes of S signals from their flat, selection-ordered events on the device (the layout compact_events
+        returns: offsets int64 [S+1], pos / idx int32, coef of the engine dtype; the events of signal s are
+        [offsets[s], offsets[s+1])).  Every signal gets one entry per distinct (t, k), the float64 sum of its events in
+        selection order, without zero sums and sums below min_coefficients (None = keep all), in ascending (t, k) order.
+        With level_bounds [b_0 <= ... <= b_{L-2}], an entry with filter k goes to the first level j with k < b_j, else to the
+        last one (convertToDistributedCoefficients); without, there is one level.  Returns one dict per level: offsets int64
+        [S+1] (from 0) and pos / idx int32, coef float64 device tensors with room for every event (len(pos) entries); level
+        j's entries are the first offsets[S] of them.  Asynchronous: nothing is read back."""
+        torch = _torch()
+        S, T, K = int(S), int(T), int(K)
+        bounds = np.ascontiguousarray([] if level_bounds is None else level_bounds, dtype=np.int64)
+        assert bounds.ndim == 1
+        n_levels = len(bounds) + 1
+        assert offsets.shape == (S + 1,) and offsets.dtype == torch.int64
+        assert pos.dtype == torch.int32 and idx.dtype == torch.int32 and coef.dtype == self.torch_dtype
+        assert pos.numel() == idx.numel() == coef.numel()
+        assert all(t.device == self.device and t.is_contiguous() for t in (offsets, pos, idx, coef))
+        cap = pos.numel()
+        with torch.cuda.device(self.device):
+            off = torch.empty((n_levels, S + 1), dtype=torch.int64, device=self.device)
+            p = torch.empty((n_levels, cap), dtype=torch.int32, device=self.device)
+            i = torch.empty((n_levels, cap), dtype=torch.int32, device=self.device)
+            c = torch.empty((n_levels, cap), dtype=torch.float64, device=self.device)
+            ptr = lambda t: ctypes.c_void_p(t.data_ptr())
+            N.check(self.lib, self.handle, self.lib.hsc_b200_canonicalize_codes(
+                self.handle, ptr(offsets), ptr(pos), ptr(idx), ptr(coef), cap, S, T, K,
+                bounds.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), len(bounds),
+                -1.0 if min_coefficients is None else float(min_coefficients), ptr(off), ptr(p), ptr(i), ptr(c),
+                self._stream_ptr(stream)))
+        return [dict(offsets=off[j], pos=p[j], idx=i[j], coef=c[j]) for j in range(n_levels)]
 
 
 class EncodeSlot(object):

@@ -18,7 +18,9 @@ partition by independent signals.  The hierarchical coder has them too: one leve
 (`HierarchicalConvolutionalMatchingPursuit._forward_batch`) runs B sequences of one length through every
 level at once and `computeCoefficients` is its B = 1 call, so a sequence's codes and residual in a batch
 are bit for bit those of its own call.  `reconstructBatch` decodes B codes in one launch
-(`Engine.decode_batch`, the kernel behind `Engine.decode` too).
+(`Engine.decode_batch`, the kernel behind `Engine.decode` too).  `encodeBatchDevice` runs the same level loop but
+keeps the codes (`HierarchicalCodes`) and the residual on the GPU: the last level's events are summed, ordered and
+redistributed on the device (`Engine.canonicalize_codes`).
 """
 import collections.abc
 import copy
@@ -73,10 +75,50 @@ class _CapacityExhausted(Exception):
     pass
 
 
+class HierarchicalCodes(object):
+    """Per-level codes of B sequences of length T, as encodeBatchDevice returns them: level l has K[l] filters and the
+    tensors offsets[l] (int64 [B+1], from 0), pos[l], idx[l] (int32) and coef[l] (float64), normally on the GPU.  The
+    entries of sequence b are [offsets[l][b], offsets[l][b+1]): one per nonzero (t, k) of its code, in ascending (t, k)
+    order, which is the order the batched decoder reads."""
+
+    def __init__(self, B, T, K, offsets, pos, idx, coef):
+        self.B, self.T, self.K = int(B), int(T), [int(k) for k in K]
+        self.offsets, self.pos, self.idx, self.coef = list(offsets), list(pos), list(idx), list(coef)
+        assert len(self.offsets) == len(self.pos) == len(self.idx) == len(self.coef) == len(self.K)
+
+    def to_csc(self):
+        """The B lists of per-level float64 csc matrices [T,K_l] (canonical format), the structure encodeBatch returns."""
+        out = [[] for _ in range(self.B)]
+        for l, K in enumerate(self.K):
+            off = self.offsets[l].cpu().numpy()
+            p, i, c = self.pos[l].cpu().numpy(), self.idx[l].cpu().numpy(), self.coef[l].cpu().numpy()
+            for b in range(self.B):
+                sl = slice(off[b], off[b + 1])
+                out[b].append(scipy.sparse.csc_matrix((c[sl].astype(np.float64), (p[sl], i[sl])), shape=(self.T, K)))
+        return out
+
+
+class _DeviceChunks(list):
+    """What _encode_chunks collects on the device path: per chunk, in signal order, the canonical per-level codes of the
+    last level (Engine.canonicalize_codes, split by `bounds`) and their entry counts."""
+
+    def __init__(self, bounds):
+        list.__init__(self)
+        self.bounds = bounds
+
+
 def _dict_eps(D):
     """np.finfo(D.dtype).eps (:1057): the energy-stop threshold follows the DICTIONARY's dtype in the reference."""
     dt = np.asarray(D).dtype
     return float(np.finfo(dt).eps) if dt.kind == 'f' else float(np.finfo(np.float64).eps)
+
+
+def _np_dtype(x):
+    """NumPy dtype of an array or a torch tensor."""
+    if isinstance(x, np.ndarray):
+        return x.dtype
+    import torch
+    return torch.empty(0, dtype=x.dtype).numpy().dtype
 
 
 def _is_multilevel_dictionary(obj):
@@ -540,13 +582,14 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
         x0 = x0[:, None] if x0.ndim == 1 else x0
         return self._forward_batch(x0[None], given, multilevelDict, toleranceSnr, nbBlocks, singletonWeight)[0]
 
-    def _forward_batch(self, x, given, multilevelDict, toleranceSnr, nbBlocks, singletonWeight):
+    def _forward_batch(self, x, given, multilevelDict, toleranceSnr, nbBlocks, singletonWeight, out=None):
         """The forward phase of B independent sequences x [B,T,F] (the input of level len(given)) with the level hand-off ON
         THE DEVICE: level l's events stay in device memory, hsc_b200_mp_events_to_dense turns them into the dense float64
         code map that is level l+1's K_l-channel input (:1489), and every level's dictionary lives in its own native engine,
         so nothing is uploaded twice.  The signals run in chunks that fit the device (_chunk_size); per chunk the host reads
         every level's events once, at the end, and builds the csc matrices the reference returns.  Returns one list per
-        sequence: the given codes followed by one csc [T,K_l] per encoded level."""
+        sequence: the given codes followed by one csc [T,K_l] per encoded level.  x may also be a torch tensor, and `out` a
+        _DeviceChunks (the device path, see _forward_chunk), which is filled and returned instead."""
         if self.method == 'cmp':
             meth = 0
         elif self.method == 'locomp':
@@ -554,7 +597,8 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
         else:
             raise Exception('Unsupported sparse coding method: %s' % (self.method))
         B, T = x.shape[0], x.shape[1]
-        out = [list(given) for _ in range(B)]
+        if out is None:
+            out = [list(given) for _ in range(B)]
         if len(given) >= multilevelDict.getNbLevels() or B == 0:
             return out
         specs = []               # (D, weights, engine dtype, options, K, level) per encoded level
@@ -569,7 +613,7 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
             weights = np.ones((D.shape[0],), dtype=D.dtype)                     # :1448-1450
             weights[:nbSingletons] = singletonWeight
             # the first level encodes the input; later levels the dense code map, which is float64 (:1489)
-            dt = engine_dtype(x, D) if not specs else engine_dtype(np.zeros(0, np.float64), D)
+            dt = engine_dtype(np.zeros(0, _np_dtype(x)), D) if not specs else engine_dtype(np.zeros(0, np.float64), D)
             eng = engine_for_dictionary(D, weights, dt, self.device)
             opt = eng.make_options(None, None, targetSnr, nbBlocks, 1e-16, use_weights=True, coef_mode=self.coef_mode, method=meth,
                                    energy_eps=_dict_eps(D))
@@ -584,7 +628,8 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
 
     def _chunk_size(self, T, specs, cap_scale):
         """Signals per chunk: every level's workspace, its input and residual, the dense hand-off [S,T,K_l] float64 and the
-        event buffers (padded and compacted) of all levels fit 80 % of the free device memory; at most 65535 signals
+        event buffers (padded and compacted) of all levels, and the device path's canonical codes of the last level (one
+        set of float64 buffers per level, plus the sort scratch) fit 80 % of the free device memory; at most 65535 signals
         (hsc_b200_mp_begin)."""
         import torch
         per = 0
@@ -593,6 +638,7 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
             eng = engine_for_dictionary(D, weights, dt, self.device)
             cap = eng.default_capacity(opt, T) * cap_scale
             per += eng.workspace_bytes(1, T) + 2 * T * eng.F * eng.dtype.itemsize + T * K * 8 + 2 * cap * (8 + eng.dtype.itemsize)
+        per += cap * (16 * len(specs) + 12)
         free, _ = torch.cuda.mem_get_info(eng.device)
         free += torch.cuda.memory_reserved(eng.device) - torch.cuda.memory_allocated(eng.device)
         return int(max(1, min(65535, int(free * 0.8) // per)))
@@ -605,6 +651,9 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
         for a in range(lo, hi, n):
             b = min(hi, a + n)
             try:
+                if isinstance(out, _DeviceChunks):
+                    out.append(self._forward_chunk(x[a:b], specs, cap_scale, out.bounds))
+                    continue
                 levels = self._forward_chunk(x[a:b], specs, cap_scale)
             except _CapacityExhausted:
                 # a level wrote more events than its buffers hold (LoCOMP emits one event per refitted group atom): the
@@ -615,29 +664,41 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
                 for s in range(b - a):
                     out[a + s].append(_events_to_csc(p[off[s]:off[s + 1]], i[off[s]:off[s + 1]], c[off[s]:off[s + 1]], T, K))
 
-    def _forward_chunk(self, x, specs, cap_scale):
-        """All levels of S <= 65535 signals x [S,T,F].  Right after a level's run, on the same stream, its events are compacted
+    def _forward_chunk(self, x, specs, cap_scale, bounds=None):
+        """All levels of S <= 65535 signals x [S,T,F] (numpy, or a torch tensor, used in place when it is a contiguous device
+        tensor of the first level's engine dtype).  Right after a level's run, on the same stream, its events are compacted
         into buffers this call owns and its states copied to pinned memory, so that a later level cannot overwrite them even
         when two levels share one cached engine.  One synchronisation after the last level; then one read per level of the
-        offsets and the flat event arrays.  Returns (K, offsets, pos, idx, coef) host arrays per level."""
+        offsets and the flat event arrays.  Returns (K, offsets, pos, idx, coef) host arrays per level.
+        With `bounds` (the device path) only the last level's events are compacted; they are canonicalized on the device,
+        split into levels by `bounds`, and nothing but the states and the per-level entry counts is read back.  Returns
+        (per-level dicts of device tensors from Engine.canonicalize_codes, host array of their entry counts)."""
         import torch
         S, T = x.shape[0], x.shape[1]
         xd = None
         pending = []
         for li, (D, weights, dt, opt, K, level) in enumerate(specs):
             eng = engine_for_dictionary(D, weights, dt, self.device)
+            last = li + 1 == len(specs)
             if xd is None:
-                xd = torch.from_numpy(np.ascontiguousarray(x, dtype=dt)).to(eng.device)
+                if isinstance(x, np.ndarray):
+                    xd = torch.from_numpy(np.ascontiguousarray(x, dtype=dt)).to(eng.device)
+                else:
+                    xd = x.to(device=eng.device, dtype=eng.torch_dtype).contiguous()
             assert xd.shape[2] == eng.F, 'level %d: the dictionary has %d channels, its input %d' % (level, eng.F, xd.shape[2])
             cap = eng.default_capacity(opt, T) * cap_scale
             evp, evi, evc, _, _ = eng.encode_device(xd, opt, cap, sync_states=False)
-            flat = eng.compact_events(evp, evi, evc)
+            flat = eng.compact_events(evp, evi, evc) if bounds is None or last else None
             hstate = torch.empty((S * ctypes.sizeof(N.SignalState),), dtype=torch.uint8, pin_memory=True)
             states = (N.SignalState * S).from_address(hstate.data_ptr())
             N.check(eng.lib, eng.handle, eng.lib.hsc_b200_mp_states_async(eng.handle, states, eng._stream_ptr()))
             pending.append((K, flat, hstate, states))
-            if li + 1 < len(specs):
+            if not last:
                 xd = eng.events_to_dense(evp, evi, evc, 1e-16)
+            elif bounds is not None:
+                canon = eng.canonicalize_codes(flat['offsets'], flat['pos'], flat['idx'], flat['coef'], S, T, K, bounds, 1e-16)
+                counts = torch.empty((len(canon),), dtype=torch.int64, pin_memory=True)
+                counts.copy_(torch.stack([lv['offsets'][S] for lv in canon]), non_blocking=True)
         torch.cuda.current_stream(xd.device).synchronize()
         levels = []
         for (K, flat, hstate, states) in pending:
@@ -647,10 +708,14 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
                                           'holds groups of at most 256')
             if np.any((status == N.HSC_PAUSE_CAPACITY) | (status == N.HSC_PAUSE_PASSES) | (status == N.HSC_RUNNING)):
                 raise _CapacityExhausted()
+            if bounds is not None:
+                continue
             off = flat['offsets'].cpu().numpy()
             n = int(off[S])
             levels.append((K, off, flat['pos'][:n].cpu().numpy(), flat['idx'][:n].cpu().numpy(),
                            flat['coef'][:n].cpu().numpy()))
+        if bounds is not None:
+            return canon, counts.numpy().copy()
         return levels
 
     def convertToDistributedCoefficients(self, coefficients):
@@ -743,6 +808,67 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
         residual = self._calculateResidualBatch(x, codes, multilevelDict)
         return codes, residual
 
+    def computeCoefficientsBatchDevice(self, sequences, multilevelDict, toleranceSnr=None, nbBlocks=1, singletonWeight=0.5,
+                                       returnDistributed=True):
+        """computeCoefficientsBatch with the codes and the residual left on the GPU: sequences [B,T] or [B,T,F], a numpy
+        array or a torch tensor (a contiguous CUDA tensor on the coder's device, of the first level's engine dtype, is read
+        in place); the dtype rules are those of computeCoefficientsBatch.  Returns (HierarchicalCodes, residual), the
+        residual a float64 CUDA tensor [B,T] or [B,T,F] (the shape rule of computeCoefficientsBatch).
+        The level loop is the one of computeCoefficientsBatch; only the last level's events are kept, and per chunk they are
+        summed, ordered and redistributed on the device (Engine.canonicalize_codes).  Duplicate events are summed in
+        selection order, which the host path does not guarantee for three or more events of one (t, k), so a value may
+        differ from computeCoefficientsBatch's in the last bits; the sparsity pattern is the same."""
+        import torch
+        assert _is_multilevel_dictionary(multilevelDict)
+        if not isinstance(sequences, torch.Tensor):
+            sequences = np.asarray(sequences)
+        assert sequences.ndim == 2 or sequences.ndim == 3
+        x = sequences[:, :, None] if sequences.ndim == 2 else sequences
+        B, T = x.shape[0], x.shape[1]
+        nl = multilevelDict.getNbLevels()
+        K = [np.asarray(multilevelDict.getRawDictionary(l)).shape[0] for l in range(nl)]
+        device = engine_for_dictionary(multilevelDict.getMultiscaleDictionaries()[0], None, np.float64, self.device).device
+        if isinstance(x, np.ndarray):            # one upload, read by the first level and by the residual
+            x = torch.from_numpy(np.ascontiguousarray(x)).to(device)
+        # redistribution (:1556-1594): columns [0, K_l) of the last level's code are level l's events; bounds of 0 leave
+        # the lower levels empty
+        chunks = self._forward_batch(x, [], multilevelDict, toleranceSnr, nbBlocks, singletonWeight,
+                                     _DeviceChunks(K[:-1] if returnDistributed else [0] * (nl - 1)))
+        levels = []
+        for l in range(nl):
+            offsets, pos, idx, coef = [torch.zeros((1,), dtype=torch.int64, device=device)], [], [], []
+            base = 0
+            for canon, counts in chunks:
+                lv, n = canon[l], int(counts[l])
+                offsets.append(lv['offsets'][1:] + base)
+                pos.append(lv['pos'][:n])
+                idx.append(lv['idx'][:n])
+                coef.append(lv['coef'][:n])
+                base += n
+            cat = lambda a, dt: torch.cat(a) if a else torch.zeros((0,), dtype=dt, device=device)
+            levels.append((torch.cat(offsets), cat(pos, torch.int32), cat(idx, torch.int32), cat(coef, torch.float64)))
+        codes = HierarchicalCodes(B, T, K, *zip(*levels))
+        recon = self.reconstructBatchDevice(codes, multilevelDict)
+        return codes, x.to(device=device, dtype=torch.float64).reshape(recon.shape) - recon
+
+    def reconstructBatchDevice(self, codes, multilevelDict):
+        """The input-level reconstruction of HierarchicalCodes (:1596-1611 without the subtraction), on the device: per level,
+        one decoder launch over all sequences with that level's representations (float64 engine), accumulating into one
+        float64 buffer [B,T,F] in level order.  Returns a float64 CUDA tensor [B,T] if the base dictionary is 2-D, else
+        [B,T,F]."""
+        import torch
+        representations = multilevelDict.getMultiscaleDictionaries()
+        assert len(codes.K) == multilevelDict.getNbLevels()
+        recon = None
+        for level in range(multilevelDict.getNbLevels()):
+            eng = engine_for_dictionary(representations[level], None, np.float64, self.device)
+            if recon is None:
+                recon = torch.zeros((codes.B, codes.T, eng.F), dtype=torch.float64, device=eng.device)
+            if codes.B > 0:
+                eng.decode_batch_device(*[t.to(eng.device) for t in (codes.offsets[level], codes.pos[level], codes.idx[level],
+                                                                       codes.coef[level])], codes.B, codes.T, recon)
+        return recon[:, :, 0] if np.asarray(multilevelDict.getBaseDictionary()).ndim == 2 else recon
+
     def computeCoefficientsFromLevel(self, sequence, coefficients, multilevelDict, nbNonzeroCoefs=None,
                                      toleranceResidualScale=None, toleranceSnr=None, nbBlocks=1, minCoefficients=None,
                                      singletonWeight=0.5, stopCondition=None, returnDistributed=True):
@@ -796,6 +922,17 @@ class HierarchicalConvolutionalSparseCoder(object):
     def encodeBatch(self, X, *args, **kwargs):
         assert X.ndim == 2 or X.ndim == 3
         return self.approximator.computeCoefficientsBatch(X, self.multilevelDict, *args, **kwargs)
+
+    def encodeBatchDevice(self, X, **kwargs):
+        """encodeBatch with the codes and the residual left on the GPU: (HierarchicalCodes, float64 CUDA residual); X [B,T]
+        or [B,T,F], numpy or torch (see HierarchicalConvolutionalMatchingPursuit.computeCoefficientsBatchDevice)."""
+        assert X.ndim == 2 or X.ndim == 3
+        return self.approximator.computeCoefficientsBatchDevice(X, self.multilevelDict, **kwargs)
+
+    def reconstructBatchDevice(self, codes):
+        """The float64 reconstruction of HierarchicalCodes on the device: [B,T] (2-D base dictionary) or [B,T,F]; equal to
+        reconstructBatch(codes.to_csc())."""
+        return self.approximator.reconstructBatchDevice(codes, self.multilevelDict)
 
     def encodeFromLevel(self, sequence, coefficients, *args, **kwargs):
         assert len(coefficients) > 0

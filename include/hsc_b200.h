@@ -210,6 +210,25 @@ int hsc_b200_decode(hsc_engine* e, const int32_t* pos_dev, const int32_t* idx_de
 int hsc_b200_decode_batch(hsc_engine* e, const int64_t* offsets_dev, const int32_t* pos_dev, const int32_t* idx_dev,
                           const void* coef_dev, int64_t S, int64_t T, void* out_dev, void* stream);
 
+/* Canonical codes from the flat, selection-ordered events hsc_b200_mp_compact_events writes (offsets_dev[S+1], pos_dev,
+ * idx_dev, coef_dev in the engine's dtype; the atoms of signal s are [offsets_dev[s], offsets_dev[s+1]), fewer than 2^31 per
+ * signal): for every signal, one entry per distinct (t,k), valued at the float64 sum of its events in selection order
+ * (:992); a sum that is exactly 0 or below min_coefficients in absolute value (< 0 = keep all) is dropped (:1171-1181).
+ * This is the arithmetic of hsc_b200_mp_events_to_dense.  Within a signal the entries are in ascending (t,k) order, the
+ * list order hsc_b200_decode_batch reads.  The entries are split into n_bounds + 1 levels (redistribution, :1556-1594):
+ * an entry with filter index k goes to the first level j with k < level_bounds_host[j], else to the last level; the bounds
+ * are non-negative and non-decreasing (a bound of 0 leaves its level empty), at most 15 of them.  Level j gets
+ * out_offsets_dev[j][S+1] (from 0) and its entries at pos / idx / coef [j][capacity] of out_pos_dev / out_idx_dev /
+ * out_coef_dev (float64): the layout hsc_b200_decode_batch reads.  `capacity` is the length of the input event arrays and
+ * of every level's output arrays; offsets_dev[S] must not exceed it (events past it are not read).  Positions must lie in
+ * [0, T) and filter indices in [0, K).  Empty signals are legal.  Deterministic (no atomics on values).  HSC_E_INVALID
+ * for a NULL pointer (the event and output arrays may be NULL when capacity = 0), S outside [1, 65535], T or K outside
+ * [1, 2^31), capacity < 0 or bad bounds; HSC_E_STATE without a dictionary.  Asynchronous. */
+int hsc_b200_canonicalize_codes(hsc_engine* e, const int64_t* offsets_dev, const int32_t* pos_dev, const int32_t* idx_dev,
+                                const void* coef_dev, int64_t capacity, int64_t S, int64_t T, int64_t K,
+                                const int64_t* level_bounds_host, int64_t n_bounds, double min_coefficients, int64_t* out_offsets_dev,
+                                int32_t* out_pos_dev, int32_t* out_idx_dev, double* out_coef_dev, void* stream);
+
 /* Convenience, host buffers end to end (allocates and frees its own device memory, synchronous):
  * x_host[S][T][F] -> residual_host[S][T][F], events [S][capacity], counts_host[S], states_host[S]
  * (either may be NULL).  Returns HSC_E_NOMEM if a signal needs more than `capacity` events. */

@@ -1,17 +1,21 @@
-"""Throughput of batched hierarchical encoding (HierarchicalConvolutionalSparseCoder.encodeBatch) against a loop of encode,
-on the config-3 workload: the 3-level dictionary and test signal of tests/golden/c3_complex.npz, plus B - 1 copies of the
-signal rolled by seeded offsets.
+"""Throughput of batched hierarchical encoding (HierarchicalConvolutionalSparseCoder.encodeBatch and encodeBatchDevice)
+against a loop of encode, on the config-3 workload: the 3-level dictionary and test signal of tests/golden/c3_complex.npz,
+plus B - 1 copies of the signal rolled by seeded offsets.
 
     python tools/hier_batch_c3.py --out-dir DIR [--batches 1,16,148,592] [--repeats 3]
 
 For every scripted setting (cmp / 10 blocks, cmp / 1 block, locomp / 10 blocks) and batch size B, after one warm-up call of
-every shape, it times encodeBatch and splits it into
+every shape, it times encodeBatch and encodeBatchDevice, alternating them, and splits encodeBatch into
   forward_ms   the level loop on the device: every chunk's launches up to its one synchronise and the read of its events
                (CUDA events around HierarchicalConvolutionalMatchingPursuit._forward_chunk; host clock alongside),
                including a first attempt that filled its LoCOMP event buffers (chunk_reruns counts them),
   assembly_ms  host code assembly: the per-(signal, level) csc matrices and the per-signal distributed conversion,
   residual_ms  the batched decoder, the subtraction and the read of the residuals,
-and times a loop of encode over min(B, --loop-max) of the same signals.  Signals/s of both, and their ratio, per row.
+and encodeBatchDevice (codes and residual left on the GPU, the call ends with a device synchronise) into
+  device_forward_ms          the same level loop without the canonical-code kernels (CUDA events),
+  device_canon_residual_ms   the canonical-code kernels (CUDA events around Engine.canonicalize_codes) plus everything
+                             after the level loop: concatenation of the chunks, the decoder launches and the subtraction,
+then times a loop of encode over min(B, --loop-max) of the same signals.  Signals/s of each, and the ratios, per row.
 Prints the GPU name and power limit (read-only nvidia-smi query) and writes one JSON line to DIR/hier_batch_c3.jsonl."""
 import argparse
 import json
@@ -38,14 +42,18 @@ def gpu_info():
 
 
 class Timers(object):
-    """Wraps the phases of one approximator: forward (device level loop), residual; assembly is the rest of the call."""
+    """Wraps the phases of one approximator: forward (device level loop), residual, distributed conversion, and the
+    canonical-code kernels of the device path; the rest of a call is host assembly (encodeBatch) or the device
+    concatenation and residual (encodeBatchDevice)."""
 
-    def __init__(self, approx):
+    def __init__(self, approx, engine_cls):
         import torch
         self.torch = torch
         self.reset()
         cls = type(approx)
         fwd, res, post = cls._forward_chunk, cls._calculateResidualBatch, cls._postprocessCoefficients
+        canon = getattr(engine_cls, '_untimed_canonicalize_codes', engine_cls.canonicalize_codes)
+        engine_cls._untimed_canonicalize_codes = canon
         me = self
 
         def forward_chunk(self_, *a, **kw):
@@ -77,13 +85,26 @@ class Timers(object):
             me.post += time.perf_counter() - t0
             return out
 
+        def canonicalize(self_, *a, **kw):
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            out = canon(self_, *a, **kw)
+            e1.record()
+            me.canon_events.append((e0, e1))     # read after the chunk's synchronise
+            return out
+
         approx._forward_chunk = forward_chunk.__get__(approx)
         approx._calculateResidualBatch = residual.__get__(approx)
         approx._postprocessCoefficients = postprocess.__get__(approx)
+        engine_cls.canonicalize_codes = canonicalize
+
+    def canon_dev(self):
+        return sum(a.elapsed_time(b) for a, b in self.canon_events) / 1e3
 
     def reset(self):
         self.forward_host = self.forward_dev = self.residual = self.post = 0.0
         self.reruns = 0
+        self.canon_events = []
 
 
 def main():
@@ -110,20 +131,40 @@ def main():
     for tag, method, nb in SETTINGS:
         approx = hsc.HierarchicalConvolutionalMatchingPursuit(method=method)
         coder = hsc.HierarchicalConvolutionalSparseCoder(mld, approx)
-        tm = Timers(approx)
+        tm = Timers(approx, hsc.Engine)
         kw = dict(toleranceSnr=10.0, nbBlocks=nb, singletonWeight=0.95)
         coder.encode(X[0], **kw)                                         # warm-up: single shape
         for B in batches:
-            coder.encodeBatch(X[:B], **kw)                               # warm-up: this batch shape
-            tm.reset()
+            coder.encodeBatch(X[:B], **kw)                               # warm-up: this batch shape, both paths
+            coder.encodeBatchDevice(X[:B], **kw)
             torch.cuda.synchronize()
-            t0 = time.perf_counter()
-            for _ in range(args.repeats):
+            host = dict(t=0.0, f_dev=0.0, f_host=0.0, resid=0.0, post=0.0, reruns=0)
+            dev = dict(t=0.0, f_dev=0.0, f_host=0.0, canon=0.0, reruns=0)
+            for _ in range(args.repeats):                                # alternating: host path, then device path
+                tm.reset()
+                t0 = time.perf_counter()
                 codes, res = coder.encodeBatch(X[:B], **kw)
-            torch.cuda.synchronize()
-            t_batch = (time.perf_counter() - t0) / args.repeats
-            f_dev, f_host = tm.forward_dev / args.repeats, tm.forward_host / args.repeats
-            resid, post = tm.residual / args.repeats, tm.post / args.repeats
+                torch.cuda.synchronize()
+                host['t'] += time.perf_counter() - t0
+                host['f_dev'] += tm.forward_dev
+                host['f_host'] += tm.forward_host
+                host['resid'] += tm.residual
+                host['post'] += tm.post
+                host['reruns'] += tm.reruns
+                tm.reset()
+                t0 = time.perf_counter()
+                dcodes, dres = coder.encodeBatchDevice(X[:B], **kw)
+                torch.cuda.synchronize()
+                dev['t'] += time.perf_counter() - t0
+                dev['f_dev'] += tm.forward_dev
+                dev['f_host'] += tm.forward_host
+                dev['canon'] += tm.canon_dev()
+                dev['reruns'] += tm.reruns
+            r = float(args.repeats)
+            t_batch, f_dev, f_host, resid, post = host['t'] / r, host['f_dev'] / r, host['f_host'] / r, host['resid'] / r, host['post'] / r
+            t_dev, canon = dev['t'] / r, dev['canon'] / r
+            d_forward = dev['f_dev'] / r - canon
+            d_canon_resid = canon + (t_dev - dev['f_host'] / r)
             n_loop = min(B, args.loop_max)
             torch.cuda.synchronize()
             t0 = time.perf_counter()
@@ -133,14 +174,21 @@ def main():
             t_loop = (time.perf_counter() - t0) / n_loop
             row = dict(setting=tag, B=B, batch_s=t_batch, forward_ms=1e3 * f_dev, forward_host_ms=1e3 * f_host,
                        assembly_ms=1e3 * (t_batch - f_host - resid), distributed_ms=1e3 * post, residual_ms=1e3 * resid,
-                       batch_signals_per_s=B / t_batch, loop_signals=n_loop, loop_s_per_signal=t_loop,
-                       loop_signals_per_s=1.0 / t_loop, speedup=(B / t_batch) * t_loop,
-                       chunk_reruns=tm.reruns / args.repeats, nnz_member0=[c.nnz for c in codes[0]])
+                       batch_signals_per_s=B / t_batch, device_batch_s=t_dev, device_forward_ms=1e3 * d_forward,
+                       device_canon_ms=1e3 * canon, device_canon_residual_ms=1e3 * d_canon_resid,
+                       device_batch_signals_per_s=B / t_dev, device_vs_batch=t_batch / t_dev,
+                       loop_signals=n_loop, loop_s_per_signal=t_loop, loop_signals_per_s=1.0 / t_loop,
+                       speedup=(B / t_batch) * t_loop, device_speedup=(B / t_dev) * t_loop,
+                       chunk_reruns=host['reruns'] / r, device_chunk_reruns=dev['reruns'] / r,
+                       nnz_member0=[c.nnz for c in codes[0]],
+                       device_nnz_member0=[int(o[1] - o[0]) for o in dcodes.offsets])
             rows.append(row)
-            print('%-10s B=%4d  batch %8.1f ms (%8.1f signals/s): forward %7.1f ms device, assembly %7.1f ms (distributed %6.1f), '
-                  'residual %6.1f ms | encode loop %7.2f ms/signal (%7.1f signals/s) | x%.1f'
+            print('%-10s B=%4d  encodeBatch %8.1f ms (%8.1f signals/s): forward %7.1f ms device, assembly %7.1f ms (distributed %6.1f), '
+                  'residual %6.1f ms | encodeBatchDevice %8.1f ms (%8.1f signals/s): forward %7.1f ms device, canonicalize+residual '
+                  '%6.1f ms (kernels %5.2f ms) | encode loop %7.2f ms/signal (%7.1f signals/s)'
                   % (tag, B, 1e3 * t_batch, B / t_batch, row['forward_ms'], row['assembly_ms'], row['distributed_ms'],
-                     row['residual_ms'], 1e3 * t_loop, 1.0 / t_loop, row['speedup']), flush=True)
+                     row['residual_ms'], 1e3 * t_dev, B / t_dev, row['device_forward_ms'], row['device_canon_residual_ms'],
+                     row['device_canon_ms'], 1e3 * t_loop, 1.0 / t_loop), flush=True)
     out = dict(metric='hier_batch_c3', gpu=torch.cuda.get_device_name(0), nvidia_smi=gpu, T=int(len(x)),
                repeats=args.repeats, rows=rows)
     os.makedirs(args.out_dir, exist_ok=True)
