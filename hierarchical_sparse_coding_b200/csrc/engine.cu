@@ -1072,7 +1072,10 @@ void ksvd_launch_gram(hsc_engine* e, cudaStream_t st, const KsvdCarve& c, const 
 void ksvd_launch_finish(hsc_engine* e, cudaStream_t st, const KsvdCarve& c, const int32_t* sig, const int32_t* pos, double* coef,
                         double* D, double* C, long long k, long long q, long long T, long long L, long long F, int off,
                         bool skip_empty, bool fused_gram = false) {
+    // HSC_KSVD_SQUARINGS: the squarings every filter gets; more follow, up to ksvd::kMaxSquarings, until the power is
+    // numerically rank one (0: power iteration on C itself)
     static const int n_square = getenv("HSC_KSVD_SQUARINGS") ? atoi(getenv("HSC_KSVD_SQUARINGS")) : 6;
+    const int n_max = n_square < 1 ? 0 : (n_square > ksvd::kMaxSquarings ? n_square : ksvd::kMaxSquarings);
     const unsigned qt = (unsigned)((q + 15) / 16);
     // small windows: every squaring and the power iteration in ONE launch of a cluster spanning the grid
     // (HSC_KSVD_CHAIN=0: the separate kernels)
@@ -1090,22 +1093,33 @@ void ksvd_launch_finish(hsc_engine* e, cudaStream_t st, const KsvdCarve& c, cons
         cfg.attrs = at; cfg.numAttrs = 1;
         const long long* skip = skip_empty ? c.col_ptr : nullptr;
         const double* Wf = fused_gram ? (const double*)c.W : (const double*)nullptr;
-        const cudaError_t ce = cudaLaunchKernelEx(&cfg, ksvd::square_chain_kernel, C, (int)q, n_square, c.M0, c.M1, 100, 1e-14, 2,
+        const cudaError_t ce = cudaLaunchKernelEx(&cfg, ksvd::square_chain_kernel, C, (int)q, n_square, n_max, c.M0, c.M1, 100, 1e-14, 2,
                                                   D + k * q, c.u, skip, (int)k, Wf, (const long long*)c.col_ptr);
         if (ce == cudaSuccess) { chained = true; n_finish = 1; }
         else { (void)cudaGetLastError(); e->ksvd_chain_failed = true; }       // (cluster launch refused: the separate kernels from now on)
     }
     if (!chained) {
         if (fused_gram) { ksvd::gram_tile_kernel<<<dim3(qt, qt), 256, 0, st>>>(c.W, c.col_ptr, (int)k, (int)q, C); e->launches += 1; }
+        const double** m_final = (const double**)(c.acc + 1);      // the power the squarings stopped at (acc[0]: alpha^2)
         const double* M = C;
         double* bufs[2] = {c.M0, c.M1};
-        for (int sq = 0; sq < n_square; ++sq) {
-            ksvd::square_kernel<<<dim3(qt, qt), 256, 0, st>>>(M, (int)q, bufs[sq & 1]);
+        for (int sq = 0; sq < n_max; ++sq) {
+            ksvd::square_kernel<<<dim3(qt, qt), 256, 0, st>>>(M, (int)q, bufs[sq & 1], sq, n_square, m_final);
             M = bufs[sq & 1];
         }
-        ksvd::power_kernel<<<1, 256, 2 * q * sizeof(double), st>>>(M, C, (int)q, 100, 1e-14, 2, D + k * q, c.u,
-                                                                  skip_empty ? c.col_ptr : nullptr, (int)k);                   // new filter (:630)
-        n_finish = 1 + n_square;
+        const long long* skip = skip_empty ? c.col_ptr : nullptr;
+        const double* const* mf = n_max > 0 ? m_final : nullptr;
+        if (q <= ksvd::kPowerSmallQ) {
+            ksvd::power_small_kernel<<<1, 256, 0, st>>>(M, mf, C, (int)q, 100, 1e-14, 2, D + k * q, c.u, skip, (int)k);   // new filter (:630)
+        } else {
+            static bool smem_set = false;       // 16 * q bytes of dynamic shared memory pass the 48 KB default at q = 3072
+            if (!smem_set) {
+                cudaFuncSetAttribute(ksvd::power_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(2 * ksvd::kMaxQ * sizeof(double)));
+                smem_set = true;
+            }
+            ksvd::power_kernel<<<1, 256, 2 * q * sizeof(double), st>>>(M, mf, C, (int)q, 100, 1e-14, 2, D + k * q, c.u, skip, (int)k);
+        }
+        n_finish = 1 + n_max;
     }
     // new coefficients (:633) and the atoms back into the running reconstruction (no-op without local atoms)
     ksvd::project_scatter_kernel<<<kKsvdGrid, 256, 0, st>>>(c.W, c.u, c.col_ptr, (int)k, (int)q, coef, c.R, sig, pos, (int)T, (int)L, (int)F, off);
@@ -1122,7 +1136,7 @@ int hsc_b200_ksvd_begin(hsc_engine* e, void* D_dev_io, int64_t K, int64_t L, int
     if (!D_dev_io || !col_ptr_host || K <= 0 || L <= 0 || F <= 0 || S <= 0 || T <= 0)
         return fail(e, HSC_E_INVALID, "ksvd_begin: bad arguments");
     const long long q = L * F;
-    if (2 * q * sizeof(double) > 48 * 1024) return fail(e, HSC_E_UNSUPPORTED, "ksvd_begin: L*F > 3072");
+    if (q > ksvd::kMaxQ) return fail(e, HSC_E_UNSUPPORTED, "ksvd_begin: L*F > " + std::to_string(ksvd::kMaxQ));
     if (e->ksvd_pca) return fail(e, HSC_E_UNSUPPORTED, "ksvd_begin: the usePCA variant needs the global column means; use hsc_b200_ksvd_update");
     const long long n = col_ptr_host[K];
     long long n_max = 0;
@@ -1172,7 +1186,7 @@ int hsc_b200_ksvd_filter_gram(hsc_ksvd_sweep* w, int64_t k, int64_t* n_local) {
     HSC_CUDA(e, cudaSetDevice(e->device));
     if (n_local) *n_local = w->col_ptr[(size_t)k + 1] - w->col_ptr[(size_t)k];
     KsvdCarve c{};
-    c.R = w->R; c.W = w->W; c.C = w->C; c.M0 = w->M0; c.M1 = w->M1; c.u = w->u; c.col_ptr = w->col_ptr_dev;
+    c.R = w->R; c.W = w->W; c.C = w->C; c.M0 = w->M0; c.M1 = w->M1; c.u = w->u; c.col_ptr = w->col_ptr_dev; c.acc = w->acc;
     ksvd_launch_gram(e, w->st, c, w->sig, w->pos, w->coef, w->D, k, w->q, w->T, w->L, w->F, w->off);
     HSC_CUDA(e, cudaGetLastError());
     w->open_filter = k;
@@ -1185,7 +1199,7 @@ int hsc_b200_ksvd_filter_finish(hsc_ksvd_sweep* w, int64_t k, int skip) {
     if (k != w->open_filter) return fail(e, HSC_E_STATE, "ksvd_filter_finish: call ksvd_filter_gram for this filter first");
     HSC_CUDA(e, cudaSetDevice(e->device));
     KsvdCarve c{};
-    c.R = w->R; c.W = w->W; c.C = w->C; c.M0 = w->M0; c.M1 = w->M1; c.u = w->u; c.col_ptr = w->col_ptr_dev;
+    c.R = w->R; c.W = w->W; c.C = w->C; c.M0 = w->M0; c.M1 = w->M1; c.u = w->u; c.col_ptr = w->col_ptr_dev; c.acc = w->acc;
     if (!skip) {
         ksvd_launch_finish(e, w->st, c, w->sig, w->pos, w->coef, w->D, w->C, k, w->q, w->T, w->L, w->F, w->off, false);
     } else {
@@ -1237,7 +1251,7 @@ int hsc_b200_ksvd_update(hsc_engine* e, void* D_dev_io, int64_t K, int64_t L, in
     if (!D_dev_io || !col_ptr_host || K <= 0 || L <= 0 || F <= 0 || S <= 0 || T <= 0)
         return fail(e, HSC_E_INVALID, "ksvd_update: bad arguments");
     const long long q = L * F;
-    if (2 * q * sizeof(double) > 48 * 1024) return fail(e, HSC_E_UNSUPPORTED, "ksvd_update: L*F > 3072");
+    if (q > ksvd::kMaxQ) return fail(e, HSC_E_UNSUPPORTED, "ksvd_update: L*F > " + std::to_string(ksvd::kMaxQ));
     const long long n = col_ptr_host[K];
     long long n_max = 0;
     for (int64_t k = 0; k < K; ++k) {

@@ -14,6 +14,17 @@
 namespace hsc {
 namespace ksvd {
 
+// Largest window q = L*F the update accepts: power_kernel keeps two q-vectors in dynamic shared memory (16 * q bytes, 48 KB
+// at the limit; the launcher opts in beyond the 48 KB default), and the three q x q float64 matrices take 226 MB of scratch.
+constexpr int kMaxQ = 3072;
+// Eigen-solver budget.  Squaring stops, after the minimum count (HSC_KSVD_SQUARINGS, 6), once the trace-normalised power
+// M = C^(2^s) / tr is numerically rank one: tr((M/tr M)^2) = ||M||_F^2 / tr(M)^2 >= 3/4 bounds the ratio of its two
+// largest eigenvalues by 0.17, so that the 100 power steps converge to rounding.  This is the trace the next squaring
+// computes anyway, the same in every CTA, so the test costs nothing.  kMaxSquarings = 30 (C^(2^30)) separates relative
+// eigenvalue gaps down to ~2e-9; an exactly multiple top eigenvalue runs all of them and yields a vector of its eigenspace.
+constexpr int kMaxSquarings = 30;
+constexpr double kRankOneTrace = 0.75;
+
 // R[s][p-off+j][f] += sign * c_i * d[j][f] for the n atoms of one filter (clipped at the signal ends).
 // The per-filter kernels read the filter's slice [col_ptr[k], col_ptr[k+1]) of the code from DEVICE memory and run on fixed
 // grids, so that the launch sequence of a whole sweep does not depend on the code: it is captured once in a CUDA graph.
@@ -110,12 +121,23 @@ __global__ void __launch_bounds__(256) gram_tile_kernel(const double* __restrict
 }
 
 // out = (in / trace(in))^2: one squaring step of the power method on a PSD matrix (eigenvalue ratios are squared,
-// the trace normalisation keeps the spectrum in [0,1]).  16x16 tile per CTA.
-__global__ void __launch_bounds__(256) square_kernel(const double* __restrict__ in, int q, double* __restrict__ out) {
+// the trace normalisation keeps the spectrum in [0,1]).  16x16 tile per CTA.  Squaring number sq of a filter: the first
+// one clears *m_final; from sq = n_min on, a squaring whose input is already numerically rank one (kRankOneTrace) or zero
+// stores that input in *m_final and computes nothing, and so do the later ones (a fixed launch sequence, graph-capturable).
+__global__ void __launch_bounds__(256) square_kernel(const double* __restrict__ in, int q, double* __restrict__ out, int sq, int n_min,
+                                                     const double** m_final) {
     __shared__ double sa[16][17], sb[16][17];
     __shared__ double s_red[8];
     __shared__ double s_scale;
+    __shared__ int s_done;
     const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
+    if (tid == 0) {
+        if (sq == 0 && blockIdx.x == 0 && blockIdx.y == 0) *m_final = nullptr;
+        // (a CTA of this launch may store it meanwhile: that is the decision this CTA takes below as well)
+        s_done = sq > 0 && sq >= n_min && *(const double* volatile*)m_final != nullptr;
+    }
+    __syncthreads();
+    if (s_done) return;
     double tr = 0.0;
     for (int i = tid; i < q; i += 256) tr += in[(long long)i * q + i];
     tr = warp_sum(tr);
@@ -124,10 +146,15 @@ __global__ void __launch_bounds__(256) square_kernel(const double* __restrict__ 
     if (tid == 0) {
         double t = 0.0;
         for (int w = 0; w < 8; ++w) t += s_red[w];
-        s_scale = t > 0.0 ? 1.0 / t : 0.0;
+        s_scale = t;
     }
     __syncthreads();
-    const double sc = s_scale;
+    const double t = s_scale;
+    if (sq >= n_min && sq > 0 && (t == 0.0 || t >= kRankOneTrace)) {
+        if (tid == 0 && blockIdx.x == 0 && blockIdx.y == 0) *m_final = in;
+        return;
+    }
+    const double sc = t > 0.0 ? 1.0 / t : 0.0;
     const int a0 = blockIdx.y * 16, b0 = blockIdx.x * 16;
     double acc = 0.0;
     for (int k0 = 0; k0 < q; k0 += 16) {
@@ -280,15 +307,23 @@ __device__ __forceinline__ void power_small(const double* M, const double* C, in
     }
 }
 
-__global__ void __launch_bounds__(256) power_kernel(const double* __restrict__ M, const double* __restrict__ C, int q, int max_iter,
-                                                    double tol, int polish, double* __restrict__ d_io,
-                                                    double* __restrict__ u_out, const long long* __restrict__ skip_col_ptr, int k) {
-    // a filter without any atom keeps its row (hsc/modeling.py:598-599); skip_col_ptr == nullptr: the caller decided
+// The eigen-solver after square_kernel: M = *m_final when a squaring stored the power it stopped at (m_final may be null:
+// no squarings).  A filter without any atom keeps its row (hsc/modeling.py:598-599); skip_col_ptr == nullptr: the caller
+// decided.  q <= kPowerSmallQ: power_small_kernel, a kernel of its own so that power_kernel does not carry power_small's
+// 34 KB of static shared memory next to its 16 * q bytes of dynamic shared memory.
+__global__ void __launch_bounds__(256) power_small_kernel(const double* M, const double* const* m_final, const double* C, int q,
+                                                          int max_iter, double tol, int polish, double* d_io, double* u_out,
+                                                          const long long* __restrict__ skip_col_ptr, int k) {
     if (skip_col_ptr && skip_col_ptr[k + 1] == skip_col_ptr[k]) return;
-    if (q <= kPowerSmallQ) {
-        power_small(M, C, q, max_iter, tol, polish, d_io, u_out);
-        return;
-    }
+    if (m_final && *m_final) M = *m_final;
+    power_small(M, C, q, max_iter, tol, polish, d_io, u_out);
+}
+
+__global__ void __launch_bounds__(256) power_kernel(const double* M, const double* const* m_final, const double* __restrict__ C, int q,
+                                                    int max_iter, double tol, int polish, double* __restrict__ d_io,
+                                                    double* __restrict__ u_out, const long long* __restrict__ skip_col_ptr, int k) {
+    if (skip_col_ptr && skip_col_ptr[k + 1] == skip_col_ptr[k]) return;
+    if (m_final && *m_final) M = *m_final;
     extern __shared__ double sm[];
     double* u = sm;            // [q]
     double* z = sm + q;        // [q]
@@ -336,7 +371,8 @@ __global__ void __launch_bounds__(256) power_kernel(const double* __restrict__ M
 __device__ __forceinline__ void cluster_sync_all() {
     asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
-__global__ void __launch_bounds__(256) square_chain_kernel(double* C, int q, int n_square, double* buf0, double* buf1, int max_iter,
+// Squarings n_min .. n_max - 1 stop as in square_kernel: every CTA computes the same trace, so the exit is uniform.
+__global__ void __launch_bounds__(256) square_chain_kernel(double* C, int q, int n_min, int n_max, double* buf0, double* buf1, int max_iter,
                                                            double tol, int polish, double* d_io, double* u_out,
                                                            const long long* __restrict__ skip_col_ptr, int k,
                                                            const double* __restrict__ W, const long long* __restrict__ w_col_ptr) {
@@ -362,7 +398,7 @@ __global__ void __launch_bounds__(256) square_chain_kernel(double* C, int q, int
         cluster_sync_all();
     }
     const double* in = C;
-    for (int sq = 0; sq < n_square; ++sq) {
+    for (int sq = 0; sq < n_max; ++sq) {
         double* out = (sq & 1) ? buf1 : buf0;
         double tr = 0.0;
         for (int i = tid; i < q; i += 256) tr += __ldcg(in + (long long)i * q + i);
@@ -372,10 +408,12 @@ __global__ void __launch_bounds__(256) square_chain_kernel(double* C, int q, int
         if (tid == 0) {
             double t = 0.0;
             for (int w = 0; w < 8; ++w) t += s_red[w];
-            s_scale = t > 0.0 ? 1.0 / t : 0.0;
+            s_scale = t;
         }
         __syncthreads();
-        const double sc = s_scale;
+        const double t = s_scale;
+        if (sq >= n_min && sq > 0 && (t == 0.0 || t >= kRankOneTrace)) break;
+        const double sc = t > 0.0 ? 1.0 / t : 0.0;
         double acc = 0.0;
         for (int k0 = 0; k0 < q; k0 += 16) {
             sa[ty][tx] = (a0 + ty < q && k0 + tx < q) ? __ldcg(in + (long long)(a0 + ty) * q + k0 + tx) * sc : 0.0;

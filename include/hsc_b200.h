@@ -246,7 +246,12 @@ int hsc_b200_mp_encode_host(hsc_engine* e, const void* x_host, int64_t S, int64_
  * signal, :610-613), new filter = first left singular vector of the window matrix, new coefficients =
  * s0 * first right singular vector (:627-633).  The sign of a singular pair is arbitrary (LAPACK's in the
  * reference); here <new filter, old filter> >= 0.  D_dev_io[K][L][F] and coef_dev_io are updated in place;
- * *alpha_host = ||D_new - D_old||_F (:636).  Synchronous. */
+ * *alpha_host = ||D_new - D_old||_F (:636).  Synchronous.
+ * Window size q = L*F <= 3072, else HSC_E_UNSUPPORTED.  Accuracy of each new filter u, the dominant eigenvector of the
+ * window Gram matrix C = W^T W (c = 32, eps = 2^-52, g = 1 - lambda2/lambda1): ||C u - (u'C u) u|| <= c q eps lambda1
+ * and u'C u >= lambda1 (1 - c q eps) for every C, a multiple top eigenvalue included; ||u -+ v1|| <= c q eps / g for
+ * gaps down to about 2e-9; all-zero windows give e_0.  W^T W is formed unscaled in float64: window entries below about
+ * 1e-160 or above 1e154 underflow or overflow. */
 int hsc_b200_ksvd_update(hsc_engine* e, void* D_dev_io, int64_t K, int64_t L, int64_t F, const int64_t* col_ptr_host,
                          const int32_t* sig_dev, const int32_t* pos_dev, const int32_t* idx_dev, void* coef_dev_io, int64_t S,
                          int64_t T, double* alpha_host, void* stream);
