@@ -26,6 +26,13 @@ def engine_dtype(*arrays):
     return np.float32 if rt == np.float32 else np.float64
 
 
+def state_stats(st):
+    """The final state of one signal (N.SignalState) as the dict EncodeResult.stats returns."""
+    return dict(energy_signal=st.energy_signal, energy_residual=st.energy_residual, n_events=st.n_events, nnz=st.nnz,
+                duplicates=st.duplicates, passes=st.passes, reranked=st.reranked,
+                stop=N.STOP_NAMES.get(st.status, str(st.status)))
+
+
 class EncodeResult(object):
     """Events of S signals in selection order, plus the final states and (optionally) residuals."""
 
@@ -41,10 +48,7 @@ class EncodeResult(object):
         self.batch_index = None
 
     def stats(self, s=0):
-        st = self.states[s]
-        return dict(energy_signal=st.energy_signal, energy_residual=st.energy_residual, n_events=st.n_events, nnz=st.nnz,
-                    duplicates=st.duplicates, passes=st.passes, reranked=st.reranked,
-                    stop=N.STOP_NAMES.get(st.status, str(st.status)))
+        return state_stats(self.states[s])
 
     def total_events(self):
         if self.counts is not None:
@@ -102,6 +106,7 @@ class Engine(object):
 
     def close(self):
         self._pipe_cache = self._host_cache = self._ws_cache = self._last_workspace = None    # device + pinned staging buffers
+        self._stream_stage = None
         for h in getattr(self, '_views', []):
             self.lib.hsc_b200_destroy(h)
         self._views = []
@@ -213,14 +218,16 @@ class Engine(object):
     def workspace_bytes(self, S, T):
         return int(self.lib.hsc_b200_workspace_bytes(self.handle, S, T))
 
-    def max_signals_per_chunk(self, T, budget_bytes=None):
+    def _free_device_bytes(self):
         torch = _torch()
+        free, _ = torch.cuda.mem_get_info(self.device)
+        # blocks torch's caching allocator holds but has not handed out are reusable too
+        return free + torch.cuda.memory_reserved(self.device) - torch.cuda.memory_allocated(self.device)
+
+    def max_signals_per_chunk(self, T, budget_bytes=None, extra_per_signal=0):
         if budget_bytes is None:
-            free, _ = torch.cuda.mem_get_info(self.device)
-            # blocks torch's caching allocator holds but has not handed out are reusable too
-            free += torch.cuda.memory_reserved(self.device) - torch.cuda.memory_allocated(self.device)
-            budget_bytes = int(free * 0.8)
-        per = self.workspace_bytes(1, T) + 2 * T * self.F * self.dtype.itemsize
+            budget_bytes = int(self._free_device_bytes() * 0.8)
+        per = self.workspace_bytes(1, T) + 2 * T * self.F * self.dtype.itemsize + int(extra_per_signal)
         return max(1, int(budget_bytes // per))
 
     def default_capacity(self, options, T):
@@ -368,13 +375,13 @@ class Engine(object):
         return out
 
     # ------------------------------------------------------------------ resident pipeline (several encodes in flight)
-    def make_slots(self, n, S, T, capacity):
+    def make_slots(self, n, S, T, capacity, own_residual=True):
         """n independent encode slots on this engine's dictionary (native views: own workspace, event buffers, residual,
         pinned states), so that the correlation of one batch can run - on its own stream - while the pursuit of the
         previous one is still going, and the pursuit CTAs of the next batch move into the SMs the previous batch's tail
-        frees.  See EncodeSlot."""
+        frees.  own_residual=False: the caller passes the residual buffer to every begin().  See EncodeSlot."""
         views = self._views_for(n)
-        return [EncodeSlot(self, views[i], S, T, capacity) for i in range(n)]
+        return [EncodeSlot(self, views[i], S, T, capacity, own_residual) for i in range(n)]
 
     @_with_stream
     def compact_events(self, evp, evi, evc, out=None, stream=None):
@@ -493,6 +500,171 @@ class Engine(object):
             self._last_workspace = cache['ws']
             self._last_shape = (S, T)
         return res
+
+    # ------------------------------------------------------------------ streamed encode, codes left on the device
+    def encode_stream_device(self, x, options, capacity=None, min_coefficients=1e-16, want_residual=True):
+        """Matching pursuit of B independent signals x [B,T,F], any B, with the canonical codes and the residual left on the
+        device.  The signals run in chunks (_stream_chunk_size) through two encode slots (EncodeSlot): the correlation (K1)
+        of chunk i+1 runs on its own stream while the pursuit (K2) of chunk i is still in its tail.  Per chunk, on its slot's
+        stream: K2, the states to pinned memory, the compaction of the events and their canonical code (canonicalize_codes:
+        duplicates summed in float64 in selection order, zero sums and |sum| < min_coefficients (None: none) dropped, entries
+        in ascending (t, k) order) plus its entry count to pinned memory.  The host reads a chunk's states only after the next
+        chunk has been enqueued.  A chunk in which a signal filled its event buffers is run again at the end with 8x the
+        buffers (up to 4096x).
+
+        x: a CUDA tensor on this engine's device - read in place when it is contiguous and of the engine dtype, never
+        written -, a pinned host tensor of the engine dtype (copied to the device on a copy stream), or any other host
+        tensor or numpy array, which first goes through a pinned staging buffer: its throughput is bounded by that host copy.
+        Returns (offsets int64 [B+1], pos int32, idx int32, coef float64: device tensors, the entries of signal b being
+        [offsets[b], offsets[b+1]); the B final SignalStates; the residual [B,T,F] of the engine dtype on the device, or None
+        when not want_residual)."""
+        torch = _torch()
+        if isinstance(x, np.ndarray):
+            x = torch.from_numpy(np.ascontiguousarray(x))
+        assert x.dim() == 3 and x.shape[2] == self.F, 'signals must be [B,T,F=%d]' % self.F
+        assert not x.is_cuda or x.device == self.device, 'a CUDA input must be on the engine device %s' % self.device
+        B, T = int(x.shape[0]), int(x.shape[1])
+        cap = int(capacity) if capacity is not None else self.default_capacity(options, T)
+        with torch.cuda.device(self.device):
+            cur = torch.cuda.current_stream(self.device)
+            resid = torch.empty((B, T, self.F), dtype=self.torch_dtype, device=self.device) if want_residual else None
+            done = {}                       # first signal of a finished chunk -> (canonical code, entries, states)
+            todo = [(0, B)] if B > 0 else []
+            scale = 1
+            while todo:
+                if scale > 4096:
+                    raise N.HscError(N.HSC_E_NOMEM, 'encode_stream_device: event buffers exhausted')
+                todo = self._stream_pass(x, todo, options, cap * scale, min_coefficients, resid, done)
+                scale *= 8
+            offsets, pos, idx, coef, states = [torch.zeros((1,), dtype=torch.int64, device=self.device)], [], [], [], []
+            base = 0
+            for a in sorted(done):
+                canon, n, st = done[a]
+                offsets.append(canon['offsets'][1:] + base)
+                pos.append(canon['pos'][:n])
+                idx.append(canon['idx'][:n])
+                coef.append(canon['coef'][:n])
+                states.extend(st)
+                base += n
+            cat = lambda a, dt: torch.cat(a) if a else torch.zeros((0,), dtype=dt, device=self.device)
+            return (torch.cat(offsets), cat(pos, torch.int32), cat(idx, torch.int32), cat(coef, torch.float64), states, resid)
+
+    def _stream_chunk_size(self, T, capacity, n_signals, options):
+        """Signals per chunk of encode_stream_device: two chunks in flight - each with its workspace, an input staging and a
+        residual buffer (max_signals_per_chunk), its event buffers and their compaction, its canonical-code buffers and sort
+        scratch, and LoCOMP's refit scratch - plus the canonical codes of all n_signals kept until the end, within 80 % of the
+        free device memory (the output residual is already allocated).  At most 65535 signals (hsc_b200_mp_begin)."""
+        it = self.dtype.itemsize
+        extra = capacity * (2 * (8 + it) + 16 + 12)
+        if options.method == 1:
+            extra += (256 * 257 + 2 * 256) * 8             # kLocompScratchStride doubles per signal
+        budget = int(self._free_device_bytes() * 0.8) - n_signals * capacity * 16
+        return int(min(65535, self.max_signals_per_chunk(T, budget // 2, extra)))
+
+    def _stream_pass(self, x, ranges, options, cap, min_coefficients, resid, done):
+        """One pass of encode_stream_device over the signal ranges [a, b) with event buffers of `cap` per signal.  Finished
+        chunks go to `done`; returns the ranges of the chunks that must be run again with larger buffers."""
+        torch = _torch()
+        T, F = int(x.shape[1]), self.F
+        total = sum(b - a for a, b in ranges)
+        per = max(1, min(self._stream_chunk_size(T, cap, total, options), max(b - a for a, b in ranges)))
+        chunks = []
+        for a, b in ranges:
+            nc = -(-(b - a) // per)                        # balanced: the last chunk is not a small remainder
+            chunks += [(a + (b - a) * c // nc, a + (b - a) * (c + 1) // nc) for c in range(nc)]
+        n = max(b - a for a, b in chunks)
+        in_place = x.is_cuda and x.dtype == self.torch_dtype and x.is_contiguous()
+        direct_h2d = not x.is_cuda and x.is_pinned() and x.dtype == self.torch_dtype and x.is_contiguous()
+        slots = self.make_slots(2, n, T, cap, own_residual=resid is None)
+        xst = None if in_place else [torch.empty((n, T, F), dtype=self.torch_dtype, device=self.device) for _ in range(2)]
+        hst = None
+        if not in_place and not direct_h2d and not x.is_cuda:
+            # pinned staging of host input, kept on the engine between calls: pinning costs tens of milliseconds per GB
+            st_ = getattr(self, '_stream_stage', None)
+            if st_ is None or st_[0].shape[0] < n or tuple(st_[0].shape[1:]) != (T, F) or st_[0].dtype != self.torch_dtype:
+                self._stream_stage = None
+                self._stream_stage = [torch.empty((n, T, F), dtype=self.torch_dtype).pin_memory() for _ in range(2)]
+            hst = self._stream_stage
+        ctx = getattr(self, '_stream_ctx', None)
+        if ctx is None:
+            # K1 on the higher-priority stream: its CTAs are placed before waiting K2 CTAs as the previous chunk's tail
+            # frees SMs (the pipeline of bench.py)
+            ctx = self._stream_ctx = dict(k1=torch.cuda.Stream(device=self.device, priority=-1),
+                                          k2=[torch.cuda.Stream(device=self.device) for _ in range(2)],
+                                          copy=torch.cuda.Stream(device=self.device))
+        s_k1, s_k2, cs = ctx['k1'], ctx['k2'], ctx['copy']
+        cur = torch.cuda.current_stream(self.device)
+        count = [torch.empty((1,), dtype=torch.int64).pin_memory() for _ in range(2)]
+        compacted = [None, None]
+        slot_free = [None, None]        # per slot: the last work of its previous chunk
+        h2d = [None, None]              # per slot: the copy out of its pinned staging buffer
+        rerun = []
+        sz = ctypes.sizeof(N.SignalState)
+
+        def finish(a, b, k, canon):
+            slot_free[k].synchronize()
+            m = b - a
+            snap = (N.SignalState * m).from_buffer_copy(bytes(slots[k].hstate.numpy()[:m * sz]))
+            status = np.ctypeslib.as_array(snap)['status']
+            if np.any(status == N.HSC_STOP_GROUP):
+                raise NotImplementedError('LoCOMP: a selection has more than 255 common-support atoms; the device refit '
+                                          'holds groups of at most 256')
+            if np.any((status == N.HSC_PAUSE_CAPACITY) | (status == N.HSC_PAUSE_PASSES) | (status == N.HSC_RUNNING)):
+                rerun.append((a, b))
+                return
+            done[a] = (canon, int(count[k][0]), [snap[i] for i in range(m)])
+
+        for st_ in [s_k1, cs] + s_k2:
+            st_.wait_stream(cur)                          # the input and the residual may come from work queued on cur
+        try:
+            pending = None
+            for ci, (a, b) in enumerate(chunks):
+                k, m = ci & 1, b - a
+                sl, s2 = slots[k], s_k2[k]
+                if slot_free[k] is not None:
+                    s_k1.wait_event(slot_free[k])         # workspace, event buffers, staging: chunk ci-2 is done with them
+                if in_place:
+                    xd = x[a:b]
+                else:
+                    src = x[a:b]
+                    if hst is not None:
+                        if h2d[k] is not None:
+                            h2d[k].synchronize()          # chunk ci-2 has left the pinned staging buffer
+                        hst[k][:m].copy_(src)
+                        src = hst[k][:m]
+                    with torch.cuda.stream(cs):
+                        if slot_free[k] is not None:
+                            cs.wait_event(slot_free[k])
+                        xst[k][:m].copy_(src, non_blocking=True)
+                        h2d[k] = torch.cuda.Event()
+                        h2d[k].record(cs)
+                    s_k1.wait_event(h2d[k])
+                    xd = xst[k][:m]
+                sl.begin(xd, options, s_k1, resid=None if resid is None else resid[a:b])
+                k1_done = torch.cuda.Event()
+                k1_done.record(s_k1)
+                s2.wait_event(k1_done)
+                sl.run(s2)
+                compacted[k] = sl.compact(compacted[k], s2)
+                c = compacted[k]
+                canon = self.canonicalize_codes(c['offsets'][:m + 1], c['pos'][:m * cap], c['idx'][:m * cap], c['coef'][:m * cap],
+                                                m, T, self.K, None, min_coefficients, stream=s2, handle=sl.handle)[0]
+                with torch.cuda.stream(s2):
+                    count[k].copy_(canon['offsets'][m:], non_blocking=True)
+                slot_free[k] = torch.cuda.Event()
+                slot_free[k].record(s2)
+                if pending is not None:
+                    finish(*pending)
+                pending = (a, b, k, canon)
+            if pending is not None:
+                finish(*pending)
+        finally:
+            for st_ in [s_k1, cs] + s_k2:
+                cur.wait_stream(st_)
+            for ev in h2d:
+                if ev is not None:
+                    ev.synchronize()
+        return rerun
 
     # ------------------------------------------------------------------ K-SVD dictionary update
     def accumulate_code(self, sig, pos, idx, coef, S, T, K, min_coefficients=1e-16):
@@ -879,7 +1051,8 @@ class Engine(object):
         return out
 
     @_with_stream
-    def canonicalize_codes(self, offsets, pos, idx, coef, S, T, K, level_bounds=None, min_coefficients=1e-16, stream=None):
+    def canonicalize_codes(self, offsets, pos, idx, coef, S, T, K, level_bounds=None, min_coefficients=1e-16, stream=None,
+                           handle=None):
         """Canonical codes of S signals from their flat, selection-ordered events on the device (the layout compact_events
         returns: offsets int64 [S+1], pos / idx int32, coef of the engine dtype; the events of signal s are
         [offsets[s], offsets[s+1])).  Every signal gets one entry per distinct (t, k), the float64 sum of its events in
@@ -887,7 +1060,8 @@ class Engine(object):
         With level_bounds [b_0 <= ... <= b_{L-2}], an entry with filter k goes to the first level j with k < b_j, else to the
         last one (convertToDistributedCoefficients); without, there is one level.  Returns one dict per level: offsets int64
         [S+1] (from 0) and pos / idx int32, coef float64 device tensors with room for every event (len(pos) entries); level
-        j's entries are the first offsets[S] of them.  Asynchronous: nothing is read back."""
+        j's entries are the first offsets[S] of them.  Asynchronous: nothing is read back.  `handle`: the native handle whose
+        sort scratch the launch uses (default: this engine's; an EncodeSlot's when several chunks are in flight)."""
         torch = _torch()
         S, T, K = int(S), int(T), int(K)
         bounds = np.ascontiguousarray([] if level_bounds is None else level_bounds, dtype=np.int64)
@@ -904,8 +1078,9 @@ class Engine(object):
             i = torch.empty((n_levels, cap), dtype=torch.int32, device=self.device)
             c = torch.empty((n_levels, cap), dtype=torch.float64, device=self.device)
             ptr = lambda t: ctypes.c_void_p(t.data_ptr())
-            N.check(self.lib, self.handle, self.lib.hsc_b200_canonicalize_codes(
-                self.handle, ptr(offsets), ptr(pos), ptr(idx), ptr(coef), cap, S, T, K,
+            h = self.handle if handle is None else handle
+            N.check(self.lib, h, self.lib.hsc_b200_canonicalize_codes(
+                h, ptr(offsets), ptr(pos), ptr(idx), ptr(coef), cap, S, T, K,
                 bounds.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), len(bounds),
                 -1.0 if min_coefficients is None else float(min_coefficients), ptr(off), ptr(p), ptr(i), ptr(c),
                 self._stream_ptr(stream)))
@@ -915,17 +1090,20 @@ class Engine(object):
 class EncodeSlot(object):
     """One encode in flight: a native view of the engine's dictionary with its own workspace (correlation map, argmax
     hierarchy, states), event buffers and residual.  begin() = K1 + state reset, run() = K2, both asynchronous on the
-    stream given; states_async() copies the per-signal states to the slot's pinned buffer."""
+    stream given; states_async() copies the per-signal states to the slot's pinned buffer.  An encode may hold fewer
+    signals than the slot was made for (the last chunk of a stream): begin() takes them from xd, and run() / compact()
+    work on that many."""
 
-    def __init__(self, eng, handle, S, T, capacity):
+    def __init__(self, eng, handle, S, T, capacity, own_residual=True):
         torch = _torch()
         self.eng, self.handle = eng, handle
         self.S, self.T, self.cap = int(S), int(T), int(capacity)
+        self.n = self.S                 # signals of the encode in flight
         dev = eng.device
         with torch.cuda.device(dev):
             self.wsb = eng.workspace_bytes(S, T)
             self.ws = torch.empty((self.wsb,), dtype=torch.uint8, device=dev)
-            self.resid = torch.empty((S, T, eng.F), dtype=eng.torch_dtype, device=dev)
+            self.resid = torch.empty((S, T, eng.F), dtype=eng.torch_dtype, device=dev) if own_residual else None
             self.evp = torch.empty((S, capacity), dtype=torch.int32, device=dev)
             self.evi = torch.empty((S, capacity), dtype=torch.int32, device=dev)
             self.evc = torch.empty((S, capacity), dtype=eng.torch_dtype, device=dev)
@@ -933,11 +1111,19 @@ class EncodeSlot(object):
         self.states = (N.SignalState * S).from_address(self.hstate.data_ptr())
         self.k2_done = None
 
-    def begin(self, xd, options, stream):
+    def begin(self, xd, options, stream, resid=None):
+        """K1 + state reset of the xd.shape[0] <= S signals xd (device, engine dtype, contiguous); the residual goes to
+        `resid` (same shape; default: the slot's own buffer)."""
         e = self.eng
+        n = int(xd.shape[0])
+        assert 0 < n <= self.S and tuple(xd.shape) == (n, self.T, e.F) and xd.dtype == e.torch_dtype and xd.is_contiguous()
+        if resid is None:
+            resid = self.resid[:n]
+        assert resid.shape == xd.shape and resid.dtype == xd.dtype and resid.is_contiguous() and resid.device == xd.device
         N.check(e.lib, self.handle, e.lib.hsc_b200_mp_begin(
-            self.handle, ctypes.c_void_p(xd.data_ptr()), ctypes.c_void_p(self.resid.data_ptr()), self.S, self.T,
+            self.handle, ctypes.c_void_p(xd.data_ptr()), ctypes.c_void_p(resid.data_ptr()), n, self.T,
             ctypes.c_void_p(self.ws.data_ptr()), self.wsb, ctypes.byref(options), ctypes.c_void_p(stream.cuda_stream)))
+        self.n = n
 
     def run(self, stream):
         e = self.eng
@@ -956,10 +1142,11 @@ class EncodeSlot(object):
                        pos=torch.empty((self.S * self.cap,), dtype=torch.int32, device=dev),
                        idx=torch.empty((self.S * self.cap,), dtype=torch.int32, device=dev),
                        coef=torch.empty((self.S * self.cap,), dtype=e.torch_dtype, device=dev))
+        assert out['offsets'].numel() >= self.n + 1 and out['pos'].numel() >= self.n * self.cap
         N.check(e.lib, self.handle, e.lib.hsc_b200_mp_compact_events(
             self.handle, ctypes.c_void_p(self.evp.data_ptr()), ctypes.c_void_p(self.evi.data_ptr()), ctypes.c_void_p(self.evc.data_ptr()),
             self.cap, ctypes.c_void_p(out['offsets'].data_ptr()), ctypes.c_void_p(out['pos'].data_ptr()),
-            ctypes.c_void_p(out['idx'].data_ptr()), ctypes.c_void_p(out['coef'].data_ptr()), self.S * self.cap,
+            ctypes.c_void_p(out['idx'].data_ptr()), ctypes.c_void_p(out['coef'].data_ptr()), self.n * self.cap,
             ctypes.c_void_p(stream.cuda_stream)))
         return out
 

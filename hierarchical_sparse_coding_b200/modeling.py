@@ -31,7 +31,7 @@ import numpy as np
 import scipy.sparse
 
 from . import _native as N
-from .engine import Engine, get_engine, engine_dtype, engine_for_dictionary
+from .engine import Engine, get_engine, engine_dtype, engine_for_dictionary, state_stats
 
 logger = logging.getLogger(__name__)
 
@@ -96,6 +96,30 @@ class HierarchicalCodes(object):
                 sl = slice(off[b], off[b + 1])
                 out[b].append(scipy.sparse.csc_matrix((c[sl].astype(np.float64), (p[sl], i[sl])), shape=(self.T, K)))
         return out
+
+
+class SparseCodes(object):
+    """Single-level codes of B signals of length T over K filters, as ConvolutionalSparseCoder.encodeBatchDevice returns
+    them: offsets (int64 [B+1], from 0), pos, idx (int32) and coef (float64), normally on the GPU.  The entries of signal b
+    are [offsets[b], offsets[b+1]): one per nonzero (t, k) of its code, in ascending (t, k) order, which is the order the
+    batched decoder reads.  `states` holds the B final per-signal states (host)."""
+
+    def __init__(self, B, T, K, offsets, pos, idx, coef, states):
+        self.B, self.T, self.K = int(B), int(T), int(K)
+        self.offsets, self.pos, self.idx, self.coef = offsets, pos, idx, coef
+        self.states = list(states)
+        assert len(self.states) == self.B and int(self.offsets.numel()) == self.B + 1
+
+    def stats(self, b):
+        """The dict EncodeResult.stats returns for signal b."""
+        return state_stats(self.states[b])
+
+    def to_csc(self):
+        """The B float64 csc matrices [T,K] (canonical format) that encodeBatch returns."""
+        off = self.offsets.cpu().numpy()
+        p, i, c = self.pos.cpu().numpy(), self.idx.cpu().numpy(), self.coef.cpu().numpy()
+        return [scipy.sparse.csc_matrix((c[off[b]:off[b + 1]].astype(np.float64), (p[off[b]:off[b + 1]], i[off[b]:off[b + 1]])),
+                                        shape=(self.T, self.K)) for b in range(self.B)]
 
 
 class _DeviceChunks(list):
@@ -546,6 +570,49 @@ class ConvolutionalMatchingPursuit(SparseApproximator):
             residual = residual[:, :, 0]
         return codes, residual
 
+    def computeCoefficientsBatchDevice(self, sequences, D, nbNonzeroCoefs=None, toleranceResidualScale=None, toleranceSnr=None,
+                                       nbBlocks=1, minCoefficients=1e-16, weights=None, returnResidual=True):
+        """computeCoefficientsBatch with the codes and the residual left on the GPU, for batches of any size.  sequences
+        [B,T] or [B,T,F]: a numpy array, a host torch tensor (a pinned one of the engine dtype is copied to the device
+        without staging) or a CUDA tensor on the coder's device (read in place, never modified, when it is contiguous and of
+        the engine dtype).  Keywords and dtype rules are those of computeCoefficientsBatch.  Returns (SparseCodes, residual):
+        the residual a CUDA tensor of the engine dtype shaped like computeCoefficientsBatch's ([B,T] for 2-D sequences), or
+        None with returnResidual=False.  The signals run in chunks through two encodes in flight (Engine.encode_stream_device);
+        the codes are summed, ordered and thresholded on the device (Engine.canonicalize_codes).  Duplicate events are summed
+        in selection order, which the host path does not guarantee for three or more events of one (t, k), so such a value
+        may differ from computeCoefficientsBatch's in the last bits; sparsity pattern, states and residual are the same."""
+        import torch
+        if not isinstance(sequences, torch.Tensor):
+            sequences = np.asarray(sequences)
+        D = np.asarray(D)
+        assert sequences.ndim == 2 or sequences.ndim == 3
+        assert D.ndim == 2 or D.ndim == 3
+        x = sequences[:, :, None] if sequences.ndim == 2 else sequences
+        eng = self._engine()
+        dt = engine_dtype(np.zeros(0, _np_dtype(x)), D)
+        eng.set_dictionary(D, weights=weights, dtype=dt)
+        opt = eng.make_options(nbNonzeroCoefs, toleranceResidualScale, toleranceSnr, nbBlocks, minCoefficients,
+                               use_weights=weights is not None, coef_mode=self.coef_mode, method=self._method, energy_eps=_dict_eps(D))
+        offsets, pos, idx, coef, states, residual = eng.encode_stream_device(x, opt, min_coefficients=minCoefficients,
+                                                                             want_residual=returnResidual)
+        codes = SparseCodes(x.shape[0], x.shape[1], eng.K, offsets, pos, idx, coef, states)
+        if residual is not None and sequences.ndim == 2:
+            residual = residual[:, :, 0]
+        return codes, residual
+
+    def reconstructBatchDevice(self, codes, D):
+        """The float64 reconstruction of SparseCodes on the device, one decoder launch: [B,T] for a 2-D dictionary, else
+        [B,T,F]; equal to ConvolutionalSparseCoder.reconstructBatch(codes.to_csc()) bit for bit."""
+        import torch
+        D = np.asarray(D)
+        assert D.ndim == 2 or D.ndim == 3
+        eng = engine_for_dictionary(D, None, np.float64, self.device)
+        recon = torch.zeros((codes.B, codes.T, eng.F), dtype=torch.float64, device=eng.device)
+        if codes.B > 0:
+            eng.decode_batch_device(*[t.to(eng.device) for t in (codes.offsets, codes.pos, codes.idx, codes.coef)], codes.B, codes.T,
+                                    recon)
+        return recon[:, :, 0] if D.ndim == 2 else recon
+
 
 class LoCOMP(ConvolutionalMatchingPursuit):
     """Drop-in for hsc.modeling.LoCOMP (:1191-1425): MP plus a local least-squares refit of the selected atom and
@@ -893,6 +960,18 @@ class ConvolutionalSparseCoder(object):
     def encodeBatch(self, X, *args, **kwargs):
         assert X.ndim == 2 or X.ndim == 3
         return self.approximator.computeCoefficientsBatch(X, self.D, *args, **kwargs)
+
+    def encodeBatchDevice(self, X, *args, **kwargs):
+        """encodeBatch with the codes and the residual left on the GPU, for batches of any size: (SparseCodes, CUDA residual
+        of the engine dtype, or None with returnResidual=False); X [B,T] or [B,T,F], numpy or torch (see
+        ConvolutionalMatchingPursuit.computeCoefficientsBatchDevice)."""
+        assert X.ndim == 2 or X.ndim == 3
+        return self.approximator.computeCoefficientsBatchDevice(X, self.D, *args, **kwargs)
+
+    def reconstructBatchDevice(self, codes):
+        """The float64 reconstruction of SparseCodes on the device: [B,T] (2-D dictionary) or [B,T,F]; equal to
+        reconstructBatch(codes.to_csc())."""
+        return self.approximator.reconstructBatchDevice(codes, self.D)
 
     def reconstruct(self, coefficients):
         assert coefficients.ndim == 1 or coefficients.ndim == 2
