@@ -33,6 +33,68 @@ def state_stats(st):
                 stop=N.STOP_NAMES.get(st.status, str(st.status)))
 
 
+_STATE_DTYPE = np.dtype(N.SignalState)
+
+
+def read_states(states, n):
+    """The first n per-signal states of a ctypes SignalState array, or of the pinned uint8 tensor an asynchronous states
+    copy fills: returns (a private copy as a SignalState array, its status column int32 [n], whether any signal is paused
+    or still running - its encode has to be run again)."""
+    raw = states.numpy() if hasattr(states, 'numpy') else bytes(states)
+    snap = (N.SignalState * n).from_buffer_copy(raw[:n * _STATE_DTYPE.itemsize])
+    status = np.frombuffer(snap, _STATE_DTYPE)['status']
+    return snap, status, bool((status[:, None] == (N.HSC_PAUSE_CAPACITY, N.HSC_PAUSE_PASSES, N.HSC_RUNNING)).any())
+
+
+def check_refit_groups(status):
+    """Raises when a signal stopped because a LoCOMP selection had more common-support atoms than the device refit holds:
+    such an encode has no result to return."""
+    if np.any(np.asarray(status) == N.HSC_STOP_GROUP):
+        raise NotImplementedError('LoCOMP: a selection has more than 255 common-support atoms; the device refit holds groups '
+                                  'of at most 256')
+
+
+def escalate_capacity(run_pass, ranges, what):
+    """Runs run_pass(ranges, scale) with scale 1, 8, 64, ... 4096 (times the default event buffers) until it returns no
+    signal range to run again; signals are independent, so a range that filled its buffers is rerun on its own."""
+    scale = 1
+    while ranges:
+        if scale > 4096:
+            raise N.HscError(N.HSC_E_NOMEM, '%s: event buffers exhausted' % what)
+        ranges = run_pass(ranges, scale)
+        scale *= 8
+
+
+def _concat_codes(parts, device):
+    """(offsets int64 [B+1], pos, idx int32, coef float64) device tensors of the canonical codes `parts`, pairs (one level's
+    dict from Engine.canonicalize_codes, its entry count) in signal order: each trimmed to its count, the offsets rebased."""
+    torch = _torch()
+    offsets, pos, idx, coef = [torch.zeros((1,), dtype=torch.int64, device=device)], [], [], []
+    base = 0
+    for lv, n in parts:
+        n = int(n)
+        offsets.append(lv['offsets'][1:] + base)
+        pos.append(lv['pos'][:n])
+        idx.append(lv['idx'][:n])
+        coef.append(lv['coef'][:n])
+        base += n
+    cat = lambda a, dt: torch.cat(a) if a else torch.zeros((0,), dtype=dt, device=device)
+    return torch.cat(offsets), cat(pos, torch.int32), cat(idx, torch.int32), cat(coef, torch.float64)
+
+
+def events_to_csc(pos, idx, coef, T, K, min_coefficients=1e-16):
+    """One signal's events (selection order, duplicates allowed) -> the reference's return type: csc_matrix [T,K] float64,
+    duplicates summed (`+=`, hsc/modeling.py:992), |c| < min_coefficients dropped (:1171-1177; None: none), zeros
+    eliminated (:1180-1181)."""
+    import scipy.sparse
+    m = scipy.sparse.coo_matrix((coef.astype(np.float64), (pos.astype(np.int64), idx.astype(np.int64))), shape=(T, K)).tocsc()
+    m.sum_duplicates()
+    if min_coefficients is not None:
+        m.data[np.abs(m.data) < min_coefficients] = 0.0
+    m.eliminate_zeros()
+    return m
+
+
 class EncodeResult(object):
     """Events of S signals in selection order, plus the final states and (optionally) residuals."""
 
@@ -56,17 +118,8 @@ class EncodeResult(object):
         return int(sum(len(p) for p in self.pos))
 
     def to_csc(self, s=0, min_coefficients=1e-16):
-        """Accumulates the events of signal s into the reference's return type: csc_matrix [T,K]
-        float64, duplicates summed (`+=`, hsc/modeling.py:992), |c| < minCoefficients dropped
-        (:1171-1177), zeros eliminated (:1180-1181)."""
-        import scipy.sparse
-        m = scipy.sparse.coo_matrix((self.coef[s].astype(np.float64), (self.pos[s].astype(np.int64), self.idx[s].astype(np.int64))),
-                                    shape=(self.T, self.K)).tocsc()
-        m.sum_duplicates()
-        if min_coefficients is not None:
-            m.data[np.abs(m.data) < min_coefficients] = 0.0
-        m.eliminate_zeros()
-        return m
+        """The events of signal s as the reference's csc_matrix [T,K] float64 (events_to_csc)."""
+        return events_to_csc(self.pos[s], self.idx[s], self.coef[s], self.T, self.K, min_coefficients)
 
 
 def _with_stream(fn):
@@ -224,6 +277,42 @@ class Engine(object):
         # blocks torch's caching allocator holds but has not handed out are reusable too
         return free + torch.cuda.memory_reserved(self.device) - torch.cuda.memory_allocated(self.device)
 
+    def _event_buffers(self, S, cap):
+        """The [S,cap] event buffers mp_run fills: positions, filter indices (int32) and coefficients (engine dtype)."""
+        torch = _torch()
+        return (torch.empty((S, cap), dtype=torch.int32, device=self.device),
+                torch.empty((S, cap), dtype=torch.int32, device=self.device),
+                torch.empty((S, cap), dtype=self.torch_dtype, device=self.device))
+
+    def _compact_buffers(self, S, cap):
+        """compact_events' output for S signals of `cap` events each: offsets int64 [S+1], flat pos, idx, coef."""
+        torch = _torch()
+        return dict(offsets=torch.empty((S + 1,), dtype=torch.int64, device=self.device),
+                    pos=torch.empty((S * cap,), dtype=torch.int32, device=self.device),
+                    idx=torch.empty((S * cap,), dtype=torch.int32, device=self.device),
+                    coef=torch.empty((S * cap,), dtype=self.torch_dtype, device=self.device))
+
+    def _pinned_states(self, S):
+        """A pinned buffer for S per-signal states and its ctypes view (the target of _states_async)."""
+        torch = _torch()
+        hstate = torch.empty((S * _STATE_DTYPE.itemsize,), dtype=torch.uint8, pin_memory=True)
+        return hstate, (N.SignalState * S).from_address(hstate.data_ptr())
+
+    def _states_async(self, states, stream=None, handle=None):
+        """Enqueues the copy of the states of the encode in flight on `handle` (default: this engine's) into `states`."""
+        h = self.handle if handle is None else handle
+        N.check(self.lib, h, self.lib.hsc_b200_mp_states_async(h, states, self._stream_ptr(stream)))
+
+    def _workspace(self, S, T):
+        """The workspace of an encode of S signals of length T: kept on the engine and grown when too small."""
+        torch = _torch()
+        wsb = self.workspace_bytes(S, T)
+        ws = getattr(self, '_ws_cache', None)
+        if ws is None or ws.numel() < wsb:
+            self._ws_cache = None
+            ws = self._ws_cache = torch.empty((wsb,), dtype=torch.uint8, device=self.device)
+        return ws, wsb
+
     def max_signals_per_chunk(self, T, budget_bytes=None, extra_per_signal=0):
         if budget_bytes is None:
             budget_bytes = int(self._free_device_bytes() * 0.8)
@@ -261,9 +350,7 @@ class Engine(object):
             wsb = self.workspace_bytes(S, T)
             ws = torch.empty((wsb,), dtype=torch.uint8, device=self.device)
             resid = xd if residual_inplace else torch.empty_like(xd)
-            evp = torch.empty((S, cap), dtype=torch.int32, device=self.device)
-            evi = torch.empty((S, cap), dtype=torch.int32, device=self.device)
-            evc = torch.empty((S, cap), dtype=self.torch_dtype, device=self.device)
+            evp, evi, evc = self._event_buffers(S, cap)
             sp = self._stream_ptr(stream)
             N.check(self.lib, self.handle, self.lib.hsc_b200_mp_begin(
                 self.handle, ctypes.c_void_p(xd.data_ptr()), ctypes.c_void_p(resid.data_ptr()), S, T,
@@ -287,8 +374,7 @@ class Engine(object):
                             chunks_p[s].append(hp[s, :nb[s]].copy())
                             chunks_i[s].append(hi[s, :nb[s]].copy())
                             chunks_c[s].append(hc[s, :nb[s]].copy())
-                paused = [states[s].status in (N.HSC_PAUSE_CAPACITY, N.HSC_PAUSE_PASSES, N.HSC_RUNNING) for s in range(S)]
-                if not any(paused):
+                if not read_states(states, S)[2]:
                     break
                 if on_pass is not None:
                     self._fill(res, chunks_p, chunks_i, chunks_c, states)
@@ -306,30 +392,11 @@ class Engine(object):
         """Lean path for resident data: xd is a device tensor [S,T,F] of the engine dtype; runs K1 + one
         K2 launch and returns (ev_pos, ev_idx, ev_coef, states, residual) with the events still on the
         device ([S,capacity] each).  `states` is None when sync_states is False (fully asynchronous)."""
-        torch = _torch()
-        S, T, _ = xd.shape
-        with torch.cuda.device(self.device):
-            wsb = self.workspace_bytes(S, T)
-            ws = getattr(self, '_ws_cache', None)
-            if ws is None or ws.numel() < wsb:
-                self._ws_cache = None
-                ws = torch.empty((wsb,), dtype=torch.uint8, device=self.device)
-                self._ws_cache = ws
-            if resid is None:
-                resid = torch.empty_like(xd)
-            evp = torch.empty((S, capacity), dtype=torch.int32, device=self.device)
-            evi = torch.empty((S, capacity), dtype=torch.int32, device=self.device)
-            evc = torch.empty((S, capacity), dtype=self.torch_dtype, device=self.device)
-            sp = self._stream_ptr(stream)
-            N.check(self.lib, self.handle, self.lib.hsc_b200_mp_begin(
-                self.handle, ctypes.c_void_p(xd.data_ptr()), ctypes.c_void_p(resid.data_ptr()), S, T,
-                ctypes.c_void_p(ws.data_ptr()), wsb, ctypes.byref(options), sp))
-            states = (N.SignalState * S)() if sync_states else None
-            N.check(self.lib, self.handle, self.lib.hsc_b200_mp_run(
-                self.handle, ctypes.c_void_p(evp.data_ptr()), ctypes.c_void_p(evi.data_ptr()),
-                ctypes.c_void_p(evc.data_ptr()), capacity, states, sp))
-            self._last_workspace = ws
-            self._last_shape = (S, T)
+        if resid is None:
+            resid = _torch().empty_like(xd)
+        self.begin_only(xd, options, resid, stream=stream)
+        evp, evi, evc = self._event_buffers(xd.shape[0], capacity)
+        states = self.run_only(evp, evi, evc, capacity, sync_states, stream=stream)
         return evp, evi, evc, states, resid
 
     @_with_stream
@@ -338,12 +405,7 @@ class Engine(object):
         torch = _torch()
         S, T, _ = xd.shape
         with torch.cuda.device(self.device):
-            wsb = self.workspace_bytes(S, T)
-            ws = getattr(self, '_ws_cache', None)
-            if ws is None or ws.numel() < wsb:
-                self._ws_cache = None
-                ws = torch.empty((wsb,), dtype=torch.uint8, device=self.device)
-                self._ws_cache = ws
+            ws, wsb = self._workspace(S, T)
             N.check(self.lib, self.handle, self.lib.hsc_b200_mp_begin(
                 self.handle, ctypes.c_void_p(xd.data_ptr()), ctypes.c_void_p(resid.data_ptr()), S, T,
                 ctypes.c_void_p(ws.data_ptr()), wsb, ctypes.byref(options), self._stream_ptr(stream)))
@@ -384,20 +446,19 @@ class Engine(object):
         return [EncodeSlot(self, views[i], S, T, capacity, own_residual) for i in range(n)]
 
     @_with_stream
-    def compact_events(self, evp, evi, evc, out=None, stream=None):
+    def compact_events(self, evp, evi, evc, out=None, stream=None, handle=None):
         """Compacts the [S,capacity] event buffers of the encode in flight (after run_only / encode_device) on the device:
         returns dict(offsets=int64[S+1], pos, idx, coef flat device tensors of S*capacity entries); the atoms of signal s are
-        [offsets[s], offsets[s+1]).  `out`: a dict from an earlier call to reuse its buffers.  Asynchronous."""
+        [offsets[s], offsets[s+1]).  `out`: a dict from an earlier call to reuse its buffers (they may be larger).
+        `handle`: the native handle whose encode is in flight (default: this engine's).  Asynchronous."""
         torch = _torch()
         S, cap = evp.shape
+        h = self.handle if handle is None else handle
         with torch.cuda.device(self.device):
-            if out is None or out['pos'].numel() < S * cap or out['offsets'].numel() != S + 1:
-                out = dict(offsets=torch.empty((S + 1,), dtype=torch.int64, device=self.device),
-                           pos=torch.empty((S * cap,), dtype=torch.int32, device=self.device),
-                           idx=torch.empty((S * cap,), dtype=torch.int32, device=self.device),
-                           coef=torch.empty((S * cap,), dtype=self.torch_dtype, device=self.device))
-            N.check(self.lib, self.handle, self.lib.hsc_b200_mp_compact_events(
-                self.handle, ctypes.c_void_p(evp.data_ptr()), ctypes.c_void_p(evi.data_ptr()), ctypes.c_void_p(evc.data_ptr()), cap,
+            if out is None or out['pos'].numel() < S * cap or out['offsets'].numel() < S + 1:
+                out = self._compact_buffers(S, cap)
+            N.check(self.lib, h, self.lib.hsc_b200_mp_compact_events(
+                h, ctypes.c_void_p(evp.data_ptr()), ctypes.c_void_p(evi.data_ptr()), ctypes.c_void_p(evc.data_ptr()), cap,
                 ctypes.c_void_p(out['offsets'].data_ptr()), ctypes.c_void_p(out['pos'].data_ptr()), ctypes.c_void_p(out['idx'].data_ptr()),
                 ctypes.c_void_p(out['coef'].data_ptr()), S * cap, self._stream_ptr(stream)))
         return out
@@ -447,13 +508,11 @@ class Engine(object):
                 cache = dict(key=key, wsb=wsb, copy_stream=torch.cuda.Stream(device=self.device),
                              ws=torch.empty((wsb,), dtype=torch.uint8, device=self.device),
                              xd=torch.empty((S, T, self.F), dtype=self.torch_dtype, device=self.device),
-                             evp=torch.empty((S, cap), dtype=torch.int32, device=self.device),
-                             evi=torch.empty((S, cap), dtype=torch.int32, device=self.device),
-                             evc=torch.empty((S, cap), dtype=self.torch_dtype, device=self.device),
                              hp=torch.empty((S, cap), dtype=torch.int32).pin_memory(),
                              hi=torch.empty((S, cap), dtype=torch.int32).pin_memory(),
                              hc=torch.empty((S, cap), dtype=self.torch_dtype).pin_memory(),
                              states=(N.SignalState * S)())
+                cache['evp'], cache['evi'], cache['evc'] = self._event_buffers(S, cap)
                 self._host_cache = cache
             cur = torch.cuda.current_stream(self.device)
             cs = cache['copy_stream']
@@ -478,7 +537,7 @@ class Engine(object):
             chunks_c = [[] for _ in range(S)]
             while True:
                 N.check(self.lib, self.handle, self.lib.hsc_b200_mp_run(self.handle, pp, ip, cp_, cap, None, sp))
-                N.check(self.lib, self.handle, self.lib.hsc_b200_mp_states_async(self.handle, stt, sp))
+                self._states_async(stt, cur)
                 cache['hp'].copy_(cache['evp'], non_blocking=True)
                 cache['hi'].copy_(cache['evi'], non_blocking=True)
                 cache['hc'].copy_(cache['evc'], non_blocking=True)
@@ -490,7 +549,7 @@ class Engine(object):
                         chunks_p[s].append(hp[s, :nb].copy())
                         chunks_i[s].append(hi_[s, :nb].copy())
                         chunks_c[s].append(hc[s, :nb].copy())
-                if not any(stt[s].status in (N.HSC_PAUSE_CAPACITY, N.HSC_PAUSE_PASSES, N.HSC_RUNNING) for s in range(S)):
+                if not read_states(stt, S)[2]:
                     break
             if want_residual:
                 residual_out.copy_(cache['xd'], non_blocking=True)
@@ -529,25 +588,11 @@ class Engine(object):
             cur = torch.cuda.current_stream(self.device)
             resid = torch.empty((B, T, self.F), dtype=self.torch_dtype, device=self.device) if want_residual else None
             done = {}                       # first signal of a finished chunk -> (canonical code, entries, states)
-            todo = [(0, B)] if B > 0 else []
-            scale = 1
-            while todo:
-                if scale > 4096:
-                    raise N.HscError(N.HSC_E_NOMEM, 'encode_stream_device: event buffers exhausted')
-                todo = self._stream_pass(x, todo, options, cap * scale, min_coefficients, resid, done)
-                scale *= 8
-            offsets, pos, idx, coef, states = [torch.zeros((1,), dtype=torch.int64, device=self.device)], [], [], [], []
-            base = 0
-            for a in sorted(done):
-                canon, n, st = done[a]
-                offsets.append(canon['offsets'][1:] + base)
-                pos.append(canon['pos'][:n])
-                idx.append(canon['idx'][:n])
-                coef.append(canon['coef'][:n])
-                states.extend(st)
-                base += n
-            cat = lambda a, dt: torch.cat(a) if a else torch.zeros((0,), dtype=dt, device=self.device)
-            return (torch.cat(offsets), cat(pos, torch.int32), cat(idx, torch.int32), cat(coef, torch.float64), states, resid)
+            escalate_capacity(lambda ranges, scale: self._stream_pass(x, ranges, options, cap * scale, min_coefficients, resid, done),
+                              [(0, B)] if B > 0 else [], 'encode_stream_device')
+            chunks = [done[a] for a in sorted(done)]
+            offsets, pos, idx, coef = _concat_codes([(canon, n) for canon, n, _ in chunks], self.device)
+            return offsets, pos, idx, coef, [st for _, _, states in chunks for st in states], resid
 
     def _stream_chunk_size(self, T, capacity, n_signals, options):
         """Signals per chunk of encode_stream_device: two chunks in flight - each with its workspace, an input staging and a
@@ -599,20 +644,15 @@ class Engine(object):
         slot_free = [None, None]        # per slot: the last work of its previous chunk
         h2d = [None, None]              # per slot: the copy out of its pinned staging buffer
         rerun = []
-        sz = ctypes.sizeof(N.SignalState)
 
         def finish(a, b, k, canon):
             slot_free[k].synchronize()
-            m = b - a
-            snap = (N.SignalState * m).from_buffer_copy(bytes(slots[k].hstate.numpy()[:m * sz]))
-            status = np.ctypeslib.as_array(snap)['status']
-            if np.any(status == N.HSC_STOP_GROUP):
-                raise NotImplementedError('LoCOMP: a selection has more than 255 common-support atoms; the device refit '
-                                          'holds groups of at most 256')
-            if np.any((status == N.HSC_PAUSE_CAPACITY) | (status == N.HSC_PAUSE_PASSES) | (status == N.HSC_RUNNING)):
+            snap, status, unfinished = read_states(slots[k].hstate, b - a)
+            check_refit_groups(status)
+            if unfinished:
                 rerun.append((a, b))
                 return
-            done[a] = (canon, int(count[k][0]), [snap[i] for i in range(m)])
+            done[a] = (canon, int(count[k][0]), list(snap))
 
         for st_ in [s_k1, cs] + s_k2:
             st_.wait_stream(cur)                          # the input and the residual may come from work queued on cur
@@ -811,39 +851,31 @@ class Engine(object):
                 sl_['d2h_done'] = None
         ctx['states_copied'] = None
         pending = None          # (slot index, EncodeResult shell, residual_out)
-        sz_state = ctypes.sizeof(N.SignalState)
 
         def make_slot(S, T, cap):
             n_max = S * cap
             d = dict(xd=torch.empty((S, T, self.F), dtype=self.torch_dtype, device=self.device),
-                     evp=torch.empty((S, cap), dtype=torch.int32, device=self.device),
-                     evi=torch.empty((S, cap), dtype=torch.int32, device=self.device),
-                     evc=torch.empty((S, cap), dtype=self.torch_dtype, device=self.device),
-                     offsets=torch.empty((S + 1,), dtype=torch.int64, device=self.device),
-                     cpos=torch.empty((n_max,), dtype=torch.int32, device=self.device),
-                     cidx=torch.empty((n_max,), dtype=torch.int32, device=self.device),
-                     ccoef=torch.empty((n_max,), dtype=self.torch_dtype, device=self.device),
+                     compact=self._compact_buffers(S, cap),
                      hoff=torch.empty((S + 1,), dtype=torch.int64).pin_memory(),
                      hp=torch.empty((n_max,), dtype=torch.int32).pin_memory(),
                      hi=torch.empty((n_max,), dtype=torch.int32).pin_memory(),
                      hc=torch.empty((n_max,), dtype=self.torch_dtype).pin_memory(),
-                     hstate=torch.empty((S * sz_state,), dtype=torch.uint8).pin_memory(),
                      d2h_done=None)
-            d['states'] = (N.SignalState * S).from_address(d['hstate'].data_ptr())
+            d['evp'], d['evi'], d['evc'] = self._event_buffers(S, cap)
+            d['hstate'], d['states'] = self._pinned_states(S)
             return d
 
         def finish(p):
             k, res, residual_out = p
             sl = slots[k]
+            dev = sl['compact']
             cout = ctx['copy_codes']                  # its own stream: copy_out already holds the next batch's (waiting) work
             sl['small_done'].synchronize()            # states + offsets are on the host
             S = res.S
             # one private copy of the S states, then vectorised unpacking (a Python loop over 512 signals with three
             # array copies each costs several milliseconds per batch)
-            snap = (N.SignalState * S).from_buffer_copy(bytes(sl['hstate'].numpy()[:S * sz_state]))
-            raw = np.frombuffer(snap, dtype=np.uint8).reshape(S, sz_state)
-            status = raw[:, N.SignalState.status.offset:N.SignalState.status.offset + 4].copy().view(np.int32)[:, 0]
-            if np.any((status == N.HSC_PAUSE_CAPACITY) | (status == N.HSC_PAUSE_PASSES) | (status == N.HSC_RUNNING)):
+            snap, _, unfinished = read_states(sl['hstate'], S)
+            if unfinished:
                 sl['d2h_done'].synchronize()
                 raise N.HscError(N.HSC_E_NOMEM, 'encode_host_pipelined: event capacity exhausted before the stop rule fired')
             sl['d2h_done'].synchronize()              # residual (if wanted) and the gather hook's reads of this slot
@@ -853,14 +885,13 @@ class Engine(object):
             if on_device_events is not None:
                 # the sparse codes are still on the device, compacted: the hook gathers them over the ranks (NCCL)
                 with torch.cuda.stream(cout):
-                    res.gathered = on_device_events(res.batch_index, dict(offsets=sl['offsets'], pos=sl['cpos'], idx=sl['cidx'],
-                                                                           coef=sl['ccoef'], total=total))
+                    res.gathered = on_device_events(res.batch_index, dict(dev, total=total))
             if host_events:
                 # the codes: exactly `total` atoms cross the bus
                 with torch.cuda.stream(cout):
-                    sl['hp'][:total].copy_(sl['cpos'][:total], non_blocking=True)
-                    sl['hi'][:total].copy_(sl['cidx'][:total], non_blocking=True)
-                    sl['hc'][:total].copy_(sl['ccoef'][:total], non_blocking=True)
+                    sl['hp'][:total].copy_(dev['pos'][:total], non_blocking=True)
+                    sl['hi'][:total].copy_(dev['idx'][:total], non_blocking=True)
+                    sl['hc'][:total].copy_(dev['coef'][:total], non_blocking=True)
                     done = torch.cuda.Event()
                     done.record(cout)
                 sl['d2h_done'] = done
@@ -899,9 +930,7 @@ class Engine(object):
                 if ctx['wss'][k] is None or ctx['wss'][k].numel() < wsb:
                     ctx['wss'][k] = None
                     other = ctx['wss'][k ^ 1]
-                    free, _ = torch.cuda.mem_get_info(self.device)
-                    free += torch.cuda.memory_reserved(self.device) - torch.cuda.memory_allocated(self.device)
-                    if two_workspaces and (other is None or other.numel() < wsb or free > wsb + (4 << 30)):
+                    if two_workspaces and (other is None or other.numel() < wsb or self._free_device_bytes() > wsb + (4 << 30)):
                         ctx['wss'][k] = torch.empty((wsb,), dtype=torch.uint8, device=self.device)
                     else:
                         if other is None or other.numel() < wsb:
@@ -949,16 +978,11 @@ class Engine(object):
                     s_k1.wait_event(k2_done)                        # the next correlation overwrites this map
                 with torch.cuda.stream(cout):
                     cout.wait_event(k2_done)
-                    csp = ctypes.c_void_p(cout.cuda_stream)
-                    N.check(self.lib, hk, self.lib.hsc_b200_mp_states_async(hk, sl['states'], csp))
-                    N.check(self.lib, hk, self.lib.hsc_b200_mp_compact_events(
-                        hk, ctypes.c_void_p(sl['evp'].data_ptr()), ctypes.c_void_p(sl['evi'].data_ptr()),
-                        ctypes.c_void_p(sl['evc'].data_ptr()), cap, ctypes.c_void_p(sl['offsets'].data_ptr()),
-                        ctypes.c_void_p(sl['cpos'].data_ptr()), ctypes.c_void_p(sl['cidx'].data_ptr()),
-                        ctypes.c_void_p(sl['ccoef'].data_ptr()), S * cap, csp))
+                    self._states_async(sl['states'], cout, hk)
+                    self.compact_events(sl['evp'], sl['evi'], sl['evc'], out=sl['compact'], stream=cout, handle=hk)
                     ctx['states_copied'] = torch.cuda.Event()       # a shared workspace's states may be reset by the next batch
                     ctx['states_copied'].record(cout)
-                    sl['hoff'].copy_(sl['offsets'], non_blocking=True)
+                    sl['hoff'].copy_(sl['compact']['offsets'], non_blocking=True)
                     small = torch.cuda.Event()
                     small.record(cout)
                     sl['small_done'] = small
@@ -1104,11 +1128,8 @@ class EncodeSlot(object):
             self.wsb = eng.workspace_bytes(S, T)
             self.ws = torch.empty((self.wsb,), dtype=torch.uint8, device=dev)
             self.resid = torch.empty((S, T, eng.F), dtype=eng.torch_dtype, device=dev) if own_residual else None
-            self.evp = torch.empty((S, capacity), dtype=torch.int32, device=dev)
-            self.evi = torch.empty((S, capacity), dtype=torch.int32, device=dev)
-            self.evc = torch.empty((S, capacity), dtype=eng.torch_dtype, device=dev)
-            self.hstate = torch.empty((S * ctypes.sizeof(N.SignalState),), dtype=torch.uint8).pin_memory()
-        self.states = (N.SignalState * S).from_address(self.hstate.data_ptr())
+            self.evp, self.evi, self.evc = eng._event_buffers(S, capacity)
+            self.hstate, self.states = eng._pinned_states(S)
         self.k2_done = None
 
     def begin(self, xd, options, stream, resid=None):
@@ -1127,28 +1148,16 @@ class EncodeSlot(object):
 
     def run(self, stream):
         e = self.eng
-        sp = ctypes.c_void_p(stream.cuda_stream)
         N.check(e.lib, self.handle, e.lib.hsc_b200_mp_run(
             self.handle, ctypes.c_void_p(self.evp.data_ptr()), ctypes.c_void_p(self.evi.data_ptr()),
-            ctypes.c_void_p(self.evc.data_ptr()), self.cap, None, sp))
-        N.check(e.lib, self.handle, e.lib.hsc_b200_mp_states_async(self.handle, self.states, sp))
+            ctypes.c_void_p(self.evc.data_ptr()), self.cap, None, ctypes.c_void_p(stream.cuda_stream)))
+        e._states_async(self.states, stream, self.handle)
 
     def compact(self, out, stream):
-        e = self.eng
-        torch = _torch()
+        n, e = self.n, self.eng
         if out is None:
-            dev = e.device
-            out = dict(offsets=torch.empty((self.S + 1,), dtype=torch.int64, device=dev),
-                       pos=torch.empty((self.S * self.cap,), dtype=torch.int32, device=dev),
-                       idx=torch.empty((self.S * self.cap,), dtype=torch.int32, device=dev),
-                       coef=torch.empty((self.S * self.cap,), dtype=e.torch_dtype, device=dev))
-        assert out['offsets'].numel() >= self.n + 1 and out['pos'].numel() >= self.n * self.cap
-        N.check(e.lib, self.handle, e.lib.hsc_b200_mp_compact_events(
-            self.handle, ctypes.c_void_p(self.evp.data_ptr()), ctypes.c_void_p(self.evi.data_ptr()), ctypes.c_void_p(self.evc.data_ptr()),
-            self.cap, ctypes.c_void_p(out['offsets'].data_ptr()), ctypes.c_void_p(out['pos'].data_ptr()),
-            ctypes.c_void_p(out['idx'].data_ptr()), ctypes.c_void_p(out['coef'].data_ptr()), self.n * self.cap,
-            ctypes.c_void_p(stream.cuda_stream)))
-        return out
+            out = e._compact_buffers(self.S, self.cap)       # room for a full slot, allocated in the caller's stream context
+        return e.compact_events(self.evp[:n], self.evi[:n], self.evc[:n], out=out, stream=stream, handle=self.handle)
 
     def launches(self):
         return int(self.eng.lib.hsc_b200_launch_count(self.handle))

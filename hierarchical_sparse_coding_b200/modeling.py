@@ -24,14 +24,13 @@ redistributed on the device (`Engine.canonicalize_codes`).
 """
 import collections.abc
 import copy
-import ctypes
 import logging
 
 import numpy as np
 import scipy.sparse
 
-from . import _native as N
-from .engine import Engine, get_engine, engine_dtype, engine_for_dictionary, state_stats
+from .engine import (Engine, get_engine, engine_dtype, engine_for_dictionary, state_stats, read_states, check_refit_groups,
+                     escalate_capacity, events_to_csc, _concat_codes)
 
 logger = logging.getLogger(__name__)
 
@@ -71,8 +70,17 @@ class MultilevelDictionary(object):
                                   '(hsc.dataset.addSingletonBases); it is outside the hot path')
 
 
-class _CapacityExhausted(Exception):
-    pass
+def _codes_to_csc(offsets, pos, idx, coef, T, K):
+    """Flat canonical codes of B signals (offsets [B+1], pos, idx, coef tensors) -> B float64 csc matrices [T,K]."""
+    off = offsets.cpu().numpy()
+    p, i, c = pos.cpu().numpy(), idx.cpu().numpy(), coef.cpu().numpy()
+    return [scipy.sparse.csc_matrix((c[a:b].astype(np.float64), (p[a:b], i[a:b])), shape=(T, K)) for a, b in zip(off[:-1], off[1:])]
+
+
+def _decode_codes_device(eng, offsets, pos, idx, coef, B, T, out):
+    """out [B,T,F] (device, float64) += the reconstruction of flat device codes with eng's dictionary, one decoder launch."""
+    if B > 0:
+        eng.decode_batch_device(*[t.to(eng.device) for t in (offsets, pos, idx, coef)], B, T, out)
 
 
 class HierarchicalCodes(object):
@@ -88,14 +96,8 @@ class HierarchicalCodes(object):
 
     def to_csc(self):
         """The B lists of per-level float64 csc matrices [T,K_l] (canonical format), the structure encodeBatch returns."""
-        out = [[] for _ in range(self.B)]
-        for l, K in enumerate(self.K):
-            off = self.offsets[l].cpu().numpy()
-            p, i, c = self.pos[l].cpu().numpy(), self.idx[l].cpu().numpy(), self.coef[l].cpu().numpy()
-            for b in range(self.B):
-                sl = slice(off[b], off[b + 1])
-                out[b].append(scipy.sparse.csc_matrix((c[sl].astype(np.float64), (p[sl], i[sl])), shape=(self.T, K)))
-        return out
+        levels = [_codes_to_csc(self.offsets[l], self.pos[l], self.idx[l], self.coef[l], self.T, K) for l, K in enumerate(self.K)]
+        return [list(b) for b in zip(*levels)]
 
 
 class SparseCodes(object):
@@ -116,19 +118,7 @@ class SparseCodes(object):
 
     def to_csc(self):
         """The B float64 csc matrices [T,K] (canonical format) that encodeBatch returns."""
-        off = self.offsets.cpu().numpy()
-        p, i, c = self.pos.cpu().numpy(), self.idx.cpu().numpy(), self.coef.cpu().numpy()
-        return [scipy.sparse.csc_matrix((c[off[b]:off[b + 1]].astype(np.float64), (p[off[b]:off[b + 1]], i[off[b]:off[b + 1]])),
-                                        shape=(self.T, self.K)) for b in range(self.B)]
-
-
-class _DeviceChunks(list):
-    """What _encode_chunks collects on the device path: per chunk, in signal order, the canonical per-level codes of the
-    last level (Engine.canonicalize_codes, split by `bounds`) and their entry counts."""
-
-    def __init__(self, bounds):
-        list.__init__(self)
-        self.bounds = bounds
+        return _codes_to_csc(self.offsets, self.pos, self.idx, self.coef, self.T, self.K)
 
 
 def _dict_eps(D):
@@ -183,16 +173,6 @@ def reconstructSignal(coefficients, D, device=None):
     keep = cx.data != 0.0
     sig = eng.decode(cx.row[keep], cx.col[keep], cx.data[keep], cx.shape[0]).cpu().numpy().astype(out_dtype)
     return sig[:, 0] if squeeze else sig
-
-
-def _events_to_csc(pos, idx, coef, T, K):
-    """One signal's events of one level -> the reference's csc [T,K] float64 (hsc/modeling.py:1180-1186): duplicates summed
-    in selection order, |x| < 1e-16 dropped, zeros eliminated."""
-    m = scipy.sparse.coo_matrix((coef.astype(np.float64), (pos.astype(np.int64), idx.astype(np.int64))), shape=(T, K)).tocsc()
-    m.sum_duplicates()
-    m.data[np.abs(m.data) < 1e-16] = 0.0
-    m.eliminate_zeros()
-    return m
 
 
 def _decode_codes(eng, codes, T, out):
@@ -367,9 +347,9 @@ class ConvolutionalDictionaryLearner(object):
             if resident:
                 cap = eng.default_capacity(opt, T)
                 evp, evi, evc, st_arr, _ = eng.encode_device(xd, opt, cap, resid=resid_buf)
-                states = [st_arr[i] for i in range(S)]
-                if any(st.status in (N.HSC_PAUSE_CAPACITY, N.HSC_PAUSE_PASSES, N.HSC_RUNNING) for st in states):
-                    states = None                      # event buffers too small for this stop rule: drain through the host path
+                snap, _, unfinished = read_states(st_arr, S)
+                # event buffers too small for this stop rule: drain through the host path
+                states = None if unfinished else list(snap)
             if states is not None:
                 nb = torch.tensor([st.n_buffered for st in states], dtype=torch.int64, device=eng.device)
                 mask = torch.arange(evp.shape[1], device=eng.device)[None, :] < nb[:, None]
@@ -385,8 +365,7 @@ class ConvolutionalDictionaryLearner(object):
                 idx = np.concatenate(res.idx) if S else np.zeros(0, np.int32)
                 coef = np.concatenate(res.coef).astype(np.float64) if S else np.zeros(0)
                 n_events = int(counts.sum())
-            if any(st.status == N.HSC_STOP_GROUP for st in states):
-                raise NotImplementedError('LoCOMP: a selection has more than 255 common-support atoms')
+            check_refit_groups([st.status for st in states])
             sg, p, ix, c, col_ptr = eng.accumulate_code(sig, pos, idx, coef, S, T, D.shape[0], 1e-16)
             torch.cuda.synchronize(eng.device)
             t_encoded = time.perf_counter()
@@ -521,9 +500,7 @@ class ConvolutionalMatchingPursuit(SparseApproximator):
                 return bool(stopCondition(x0, res.residual[0].cpu().numpy(), res.to_csc(0, None).tolil()))
         res = eng.encode(np.ascontiguousarray(sequences, dtype=dt), opt, on_pass=on_pass)
         self.last_result = res
-        if any(st.status == N.HSC_STOP_GROUP for st in res.states):
-            raise NotImplementedError('LoCOMP: a selection has more than 255 common-support atoms; the device refit '
-                                      'holds groups of at most 256')
+        check_refit_groups([st.status for st in res.states])
         return res
 
     def computeCoefficients(self, sequence, D, nbNonzeroCoefs=None, toleranceResidualScale=None, toleranceSnr=None,
@@ -608,9 +585,7 @@ class ConvolutionalMatchingPursuit(SparseApproximator):
         assert D.ndim == 2 or D.ndim == 3
         eng = engine_for_dictionary(D, None, np.float64, self.device)
         recon = torch.zeros((codes.B, codes.T, eng.F), dtype=torch.float64, device=eng.device)
-        if codes.B > 0:
-            eng.decode_batch_device(*[t.to(eng.device) for t in (codes.offsets, codes.pos, codes.idx, codes.coef)], codes.B, codes.T,
-                                    recon)
+        _decode_codes_device(eng, codes.offsets, codes.pos, codes.idx, codes.coef, codes.B, codes.T, recon)
         return recon[:, :, 0] if D.ndim == 2 else recon
 
 
@@ -649,14 +624,15 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
         x0 = x0[:, None] if x0.ndim == 1 else x0
         return self._forward_batch(x0[None], given, multilevelDict, toleranceSnr, nbBlocks, singletonWeight)[0]
 
-    def _forward_batch(self, x, given, multilevelDict, toleranceSnr, nbBlocks, singletonWeight, out=None):
+    def _forward_batch(self, x, given, multilevelDict, toleranceSnr, nbBlocks, singletonWeight, bounds=None):
         """The forward phase of B independent sequences x [B,T,F] (the input of level len(given)) with the level hand-off ON
         THE DEVICE: level l's events stay in device memory, hsc_b200_mp_events_to_dense turns them into the dense float64
         code map that is level l+1's K_l-channel input (:1489), and every level's dictionary lives in its own native engine,
-        so nothing is uploaded twice.  The signals run in chunks that fit the device (_chunk_size); per chunk the host reads
+        so nothing is uploaded twice.  The signals run in chunks that fit the device (_encode_pass); per chunk the host reads
         every level's events once, at the end, and builds the csc matrices the reference returns.  Returns one list per
-        sequence: the given codes followed by one csc [T,K_l] per encoded level.  x may also be a torch tensor, and `out` a
-        _DeviceChunks (the device path, see _forward_chunk), which is filled and returned instead."""
+        sequence: the given codes followed by one csc [T,K_l] per encoded level.  x may also be a torch tensor.  With
+        `bounds` (the device path, see _forward_chunk) returns instead a dict: first signal of each chunk -> what
+        _forward_chunk returns for it."""
         if self.method == 'cmp':
             meth = 0
         elif self.method == 'locomp':
@@ -664,8 +640,7 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
         else:
             raise Exception('Unsupported sparse coding method: %s' % (self.method))
         B, T = x.shape[0], x.shape[1]
-        if out is None:
-            out = [list(given) for _ in range(B)]
+        out = [list(given) for _ in range(B)] if bounds is None else {}
         if len(given) >= multilevelDict.getNbLevels() or B == 0:
             return out
         specs = []               # (D, weights, engine dtype, options, K, level) per encoded level
@@ -685,7 +660,8 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
             opt = eng.make_options(None, None, targetSnr, nbBlocks, 1e-16, use_weights=True, coef_mode=self.coef_mode, method=meth,
                                    energy_eps=_dict_eps(D))
             specs.append((D, weights, dt, opt, D.shape[0], level))
-        self._encode_chunks(x, 0, B, specs, 1, out)
+        escalate_capacity(lambda ranges, scale: self._encode_pass(x, ranges, specs, scale, out, bounds), [(0, B)],
+                          'hierarchical encode')
         for (D, weights, dt, _, _, _) in specs:
             eng = engine_for_dictionary(D, weights, dt, self.device)
             ws = getattr(eng, '_ws_cache', None)
@@ -698,7 +674,6 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
         event buffers (padded and compacted) of all levels, and the device path's canonical codes of the last level (one
         set of float64 buffers per level, plus the sort scratch) fit 80 % of the free device memory; at most 65535 signals
         (hsc_b200_mp_begin)."""
-        import torch
         per = 0
         eng = None
         for (D, weights, dt, opt, K, _) in specs:
@@ -706,30 +681,29 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
             cap = eng.default_capacity(opt, T) * cap_scale
             per += eng.workspace_bytes(1, T) + 2 * T * eng.F * eng.dtype.itemsize + T * K * 8 + 2 * cap * (8 + eng.dtype.itemsize)
         per += cap * (16 * len(specs) + 12)
-        free, _ = torch.cuda.mem_get_info(eng.device)
-        free += torch.cuda.memory_reserved(eng.device) - torch.cuda.memory_allocated(eng.device)
-        return int(max(1, min(65535, int(free * 0.8) // per)))
+        return int(max(1, min(65535, int(eng._free_device_bytes() * 0.8) // per)))
 
-    def _encode_chunks(self, x, lo, hi, specs, cap_scale, out):
-        if cap_scale > 4096:
-            raise N.HscError(N.HSC_E_NOMEM, 'hierarchical encode: event buffers exhausted')
+    def _encode_pass(self, x, ranges, specs, cap_scale, out, bounds):
+        """One pass of the level loop over the signal ranges [a, b), in chunks of _chunk_size signals, with cap_scale times the
+        default event buffers.  Finished chunks go to `out` (see _forward_batch); returns the ranges of the chunks in which a
+        level wrote more events than its buffers hold (LoCOMP emits one event per refitted group atom): the later levels saw
+        a truncated code, so their forward phase must be repeated with larger buffers."""
         T = x.shape[1]
         n = self._chunk_size(T, specs, cap_scale)
-        for a in range(lo, hi, n):
-            b = min(hi, a + n)
-            try:
-                if isinstance(out, _DeviceChunks):
-                    out.append(self._forward_chunk(x[a:b], specs, cap_scale, out.bounds))
-                    continue
-                levels = self._forward_chunk(x[a:b], specs, cap_scale)
-            except _CapacityExhausted:
-                # a level wrote more events than its buffers hold (LoCOMP emits one event per refitted group atom): the
-                # later levels saw a truncated code, so the chunk's forward phase is repeated with larger buffers
-                self._encode_chunks(x, a, b, specs, cap_scale * 8, out)
-                continue
-            for (K, off, p, i, c) in levels:
-                for s in range(b - a):
-                    out[a + s].append(_events_to_csc(p[off[s]:off[s + 1]], i[off[s]:off[s + 1]], c[off[s]:off[s + 1]], T, K))
+        rerun = []
+        for lo, hi in ranges:
+            for a in range(lo, hi, n):
+                b = min(hi, a + n)
+                levels = self._forward_chunk(x[a:b], specs, cap_scale, bounds)
+                if levels is None:
+                    rerun.append((a, b))
+                elif bounds is not None:
+                    out[a] = levels
+                else:
+                    for (K, off, p, i, c) in levels:
+                        for s in range(b - a):
+                            out[a + s].append(events_to_csc(p[off[s]:off[s + 1]], i[off[s]:off[s + 1]], c[off[s]:off[s + 1]], T, K))
+        return rerun
 
     def _forward_chunk(self, x, specs, cap_scale, bounds=None):
         """All levels of S <= 65535 signals x [S,T,F] (numpy, or a torch tensor, used in place when it is a contiguous device
@@ -739,7 +713,8 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
         offsets and the flat event arrays.  Returns (K, offsets, pos, idx, coef) host arrays per level.
         With `bounds` (the device path) only the last level's events are compacted; they are canonicalized on the device,
         split into levels by `bounds`, and nothing but the states and the per-level entry counts is read back.  Returns
-        (per-level dicts of device tensors from Engine.canonicalize_codes, host array of their entry counts)."""
+        (per-level dicts of device tensors from Engine.canonicalize_codes, host array of their entry counts).
+        Returns None when a level's event buffers filled up before its stop rule fired."""
         import torch
         S, T = x.shape[0], x.shape[1]
         xd = None
@@ -756,10 +731,9 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
             cap = eng.default_capacity(opt, T) * cap_scale
             evp, evi, evc, _, _ = eng.encode_device(xd, opt, cap, sync_states=False)
             flat = eng.compact_events(evp, evi, evc) if bounds is None or last else None
-            hstate = torch.empty((S * ctypes.sizeof(N.SignalState),), dtype=torch.uint8, pin_memory=True)
-            states = (N.SignalState * S).from_address(hstate.data_ptr())
-            N.check(eng.lib, eng.handle, eng.lib.hsc_b200_mp_states_async(eng.handle, states, eng._stream_ptr()))
-            pending.append((K, flat, hstate, states))
+            hstate, states = eng._pinned_states(S)
+            eng._states_async(states)
+            pending.append((K, flat, hstate))
             if not last:
                 xd = eng.events_to_dense(evp, evi, evc, 1e-16)
             elif bounds is not None:
@@ -768,13 +742,11 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
                 counts.copy_(torch.stack([lv['offsets'][S] for lv in canon]), non_blocking=True)
         torch.cuda.current_stream(xd.device).synchronize()
         levels = []
-        for (K, flat, hstate, states) in pending:
-            status = np.ctypeslib.as_array(states)['status']
-            if np.any(status == N.HSC_STOP_GROUP):
-                raise NotImplementedError('LoCOMP: a selection has more than 255 common-support atoms; the device refit '
-                                          'holds groups of at most 256')
-            if np.any((status == N.HSC_PAUSE_CAPACITY) | (status == N.HSC_PAUSE_PASSES) | (status == N.HSC_RUNNING)):
-                raise _CapacityExhausted()
+        for (K, flat, hstate) in pending:
+            _, status, unfinished = read_states(hstate, S)
+            check_refit_groups(status)
+            if unfinished:
+                return None
             if bounds is not None:
                 continue
             off = flat['offsets'].cpu().numpy()
@@ -899,21 +871,10 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
             x = torch.from_numpy(np.ascontiguousarray(x)).to(device)
         # redistribution (:1556-1594): columns [0, K_l) of the last level's code are level l's events; bounds of 0 leave
         # the lower levels empty
-        chunks = self._forward_batch(x, [], multilevelDict, toleranceSnr, nbBlocks, singletonWeight,
-                                     _DeviceChunks(K[:-1] if returnDistributed else [0] * (nl - 1)))
-        levels = []
-        for l in range(nl):
-            offsets, pos, idx, coef = [torch.zeros((1,), dtype=torch.int64, device=device)], [], [], []
-            base = 0
-            for canon, counts in chunks:
-                lv, n = canon[l], int(counts[l])
-                offsets.append(lv['offsets'][1:] + base)
-                pos.append(lv['pos'][:n])
-                idx.append(lv['idx'][:n])
-                coef.append(lv['coef'][:n])
-                base += n
-            cat = lambda a, dt: torch.cat(a) if a else torch.zeros((0,), dtype=dt, device=device)
-            levels.append((torch.cat(offsets), cat(pos, torch.int32), cat(idx, torch.int32), cat(coef, torch.float64)))
+        done = self._forward_batch(x, [], multilevelDict, toleranceSnr, nbBlocks, singletonWeight,
+                                   K[:-1] if returnDistributed else [0] * (nl - 1))
+        chunks = [done[a] for a in sorted(done)]
+        levels = [_concat_codes([(canon[l], counts[l]) for canon, counts in chunks], device) for l in range(nl)]
         codes = HierarchicalCodes(B, T, K, *zip(*levels))
         recon = self.reconstructBatchDevice(codes, multilevelDict)
         return codes, x.to(device=device, dtype=torch.float64).reshape(recon.shape) - recon
@@ -931,9 +892,8 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
             eng = engine_for_dictionary(representations[level], None, np.float64, self.device)
             if recon is None:
                 recon = torch.zeros((codes.B, codes.T, eng.F), dtype=torch.float64, device=eng.device)
-            if codes.B > 0:
-                eng.decode_batch_device(*[t.to(eng.device) for t in (codes.offsets[level], codes.pos[level], codes.idx[level],
-                                                                       codes.coef[level])], codes.B, codes.T, recon)
+            _decode_codes_device(eng, codes.offsets[level], codes.pos[level], codes.idx[level], codes.coef[level], codes.B, codes.T,
+                                 recon)
         return recon[:, :, 0] if np.asarray(multilevelDict.getBaseDictionary()).ndim == 2 else recon
 
     def computeCoefficientsFromLevel(self, sequence, coefficients, multilevelDict, nbNonzeroCoefs=None,

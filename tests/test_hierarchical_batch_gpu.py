@@ -122,7 +122,7 @@ def test_chunk_boundaries_do_not_change_the_result(hsc, c3_mld, c3, monkeypatch)
     assert np.array_equal(res3, res1)
 
 
-def test_locomp_capacity_rerun(hsc, monkeypatch):
+def test_locomp_capacity_escalation(hsc, monkeypatch):
     """A member whose LoCOMP run needs more events than the default buffers hold: its chunk is rerun with 8x the buffers,
     and every member still equals its single call."""
     from oracle import hsc_oracle as O
@@ -140,8 +140,8 @@ def test_locomp_capacity_rerun(hsc, monkeypatch):
     approx = hsc.HierarchicalConvolutionalMatchingPursuit(method='locomp')
     coder = hsc.HierarchicalConvolutionalSparseCoder(mld, approx)
     scales = []
-    orig = type(approx)._encode_chunks
-    monkeypatch.setattr(type(approx), '_encode_chunks', lambda self, x, lo, hi, specs, cs, out: scales.append(cs) or orig(self, x, lo, hi, specs, cs, out))
+    orig = type(approx)._encode_pass
+    monkeypatch.setattr(type(approx), '_encode_pass', lambda self, x, r, specs, cs, *a: scales.append(cs) or orig(self, x, r, specs, cs, *a))
     kw = dict(toleranceSnr=40.0, singletonWeight=0.95)
     codes, res = coder.encodeBatch(X, **kw)
     assert max(scales) >= 8, scales

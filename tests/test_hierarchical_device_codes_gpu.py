@@ -247,7 +247,7 @@ def _locomp_rerun_input(hsc):
 
 
 @pytest.mark.gpu
-def test_device_locomp_capacity_rerun(hsc, monkeypatch):
+def test_device_locomp_capacity_escalation(hsc, monkeypatch):
     """A member that fills the LoCOMP event buffers: its chunk is rerun with 8x the buffers, and the result equals a run
     whose buffers were large enough from the start."""
     mld, X = _locomp_rerun_input(hsc)
@@ -255,9 +255,8 @@ def test_device_locomp_capacity_rerun(hsc, monkeypatch):
     coder = hsc.HierarchicalConvolutionalSparseCoder(mld, approx)
     kw = dict(toleranceSnr=40.0, singletonWeight=0.95)
     scales = []
-    orig = type(approx)._encode_chunks
-    monkeypatch.setattr(type(approx), '_encode_chunks',
-                        lambda self, x, lo, hi, specs, cs, out: scales.append(cs) or orig(self, x, lo, hi, specs, cs, out))
+    orig = type(approx)._encode_pass
+    monkeypatch.setattr(type(approx), '_encode_pass', lambda self, x, r, specs, cs, *a: scales.append(cs) or orig(self, x, r, specs, cs, *a))
     rerun = coder.encodeBatchDevice(X, **kw)
     assert max(scales) >= 8, scales
     _assert_matches_host(coder, X, kw, *rerun)

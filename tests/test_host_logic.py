@@ -22,6 +22,67 @@ def test_encode_result_to_csc_sums_duplicates_and_clips():
     assert r.total_events() == 5
 
 
+def test_capacity_escalation_scales_and_limit():
+    """The batched encode paths rerun the signal ranges that filled their event buffers with 8x the buffers, up to 4096x."""
+    from hierarchical_sparse_coding_b200 import _native as N
+    from hierarchical_sparse_coding_b200.engine import escalate_capacity
+    seen = []
+    with pytest.raises(N.HscError) as e:
+        escalate_capacity(lambda ranges, scale: seen.append((ranges, scale)) or ranges, [(0, 4)], 'test')
+    assert e.value.code == N.HSC_E_NOMEM and 'event buffers exhausted' in str(e.value)
+    assert seen == [([(0, 4)], s) for s in (1, 8, 64, 512, 4096)]
+    seen = []
+    escalate_capacity(lambda ranges, scale: seen.append((ranges, scale)) or ([(2, 3)] if scale == 1 else []),
+                      [(0, 2), (2, 5)], 'test')
+    assert seen == [([(0, 2), (2, 5)], 1), ([(2, 3)], 8)]
+    escalate_capacity(lambda ranges, scale: pytest.fail('no range to run'), [], 'test')
+
+
+def test_read_states_classifies_every_status():
+    """The per-signal state check of the encode paths, from a ctypes array and from a byte snapshot of one (the pinned
+    buffer an asynchronous states copy fills, which may hold more signals than the encode)."""
+    import torch
+    from hierarchical_sparse_coding_b200 import _native as N
+    from hierarchical_sparse_coding_b200.engine import check_refit_groups, read_states
+    unfinished = (N.HSC_PAUSE_CAPACITY, N.HSC_PAUSE_PASSES, N.HSC_RUNNING)
+    for code in N.STOP_NAMES:
+        arr = (N.SignalState * 3)()
+        for s in range(3):
+            arr[s].status, arr[s].n_events = N.HSC_STOP_SNR, 10 + s
+        arr[1].status = code
+        snapshot = torch.from_numpy(np.frombuffer(bytes(arr) * 2, np.uint8).copy())
+        for src in (arr, snapshot):
+            snap, status, paused = read_states(src, 3)
+            assert status.dtype == np.int32 and status.tolist() == [N.HSC_STOP_SNR, code, N.HSC_STOP_SNR]
+            assert paused == (code in unfinished), N.STOP_NAMES[code]
+            assert bytes(snap) == bytes(arr) and [st.n_events for st in snap] == [10, 11, 12]
+            assert read_states(src, 1)[1].tolist() == [N.HSC_STOP_SNR] and not read_states(src, 1)[2]
+        if code == N.HSC_STOP_GROUP:
+            with pytest.raises(NotImplementedError):
+                check_refit_groups(status)
+        else:
+            check_refit_groups(status)
+    arr[0].n_events = 99
+    assert snap[0].n_events == 10                                                # a private copy
+
+
+def test_concat_codes_trims_and_rebases():
+    import torch
+    from hierarchical_sparse_coding_b200.engine import _concat_codes
+
+    def level(offsets, pos):              # canonical codes with room for more entries than they hold (-1: unused room)
+        p = torch.tensor(pos, dtype=torch.int32)
+        return dict(offsets=torch.tensor(offsets, dtype=torch.int64), pos=p, idx=p + 1, coef=p.double() / 8)
+    parts = [(level([0, 2, 3], [10, 11, 12, -1, -1]), 3), (level([0, 0], [-1, -1]), 0), (level([0, 1, 2], [20, 21, -1]), np.int64(2))]
+    off, pos, idx, coef = _concat_codes(parts, 'cpu')
+    assert off.dtype == torch.int64 and pos.dtype == idx.dtype == torch.int32 and coef.dtype == torch.float64
+    assert off.tolist() == [0, 2, 3, 3, 4, 5] and pos.tolist() == [10, 11, 12, 20, 21]
+    assert idx.tolist() == [11, 12, 13, 21, 22] and coef.tolist() == [1.25, 1.375, 1.5, 2.5, 2.625]
+    off, pos, idx, coef = _concat_codes([], 'cpu')
+    assert off.tolist() == [0] and pos.numel() == idx.numel() == coef.numel() == 0
+    assert pos.dtype == idx.dtype == torch.int32 and coef.dtype == torch.float64
+
+
 def test_convert_to_distributed_matches_oracle():
     import hierarchical_sparse_coding_b200.modeling as M
     rs = np.random.RandomState(0)

@@ -61,10 +61,9 @@ class Timers(object):
             t0 = time.perf_counter()
             e0.record()
             try:
-                return fwd(self_, *a, **kw)
-            except Exception:
-                me.reruns += 1                   # a chunk that filled its LoCOMP event buffers: counted, then rerun
-                raise
+                out = fwd(self_, *a, **kw)
+                me.reruns += out is None         # a chunk that filled its LoCOMP event buffers: counted, then rerun
+                return out
             finally:
                 e1.record()
                 e1.synchronize()
