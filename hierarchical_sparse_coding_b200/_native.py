@@ -32,6 +32,7 @@ EXPORTED_SYMBOLS = [
     'hsc_b200_mp_states_async', 'hsc_b200_mp_begin_part', 'hsc_b200_ksvd_update', 'hsc_b200_ksvd_set_pca', 'hsc_b200_kmeans_assign',
     'hsc_b200_ksvd_begin', 'hsc_b200_ksvd_filter_gram', 'hsc_b200_ksvd_filter_finish', 'hsc_b200_ksvd_end',
     'hsc_b200_mp_compact_events', 'hsc_b200_mp_events_to_dense', 'hsc_b200_decode_batch', 'hsc_b200_canonicalize_codes',
+    'hsc_b200_mp_begin_lengths',
 ]
 
 
@@ -111,6 +112,8 @@ def load_library():
     lib.hsc_b200_mp_begin.argtypes = [vp, vp, vp, i64, i64, vp, sz, ctypes.POINTER(MpOptions), vp]
     lib.hsc_b200_mp_begin_part.restype = ctypes.c_int
     lib.hsc_b200_mp_begin_part.argtypes = [vp, vp, vp, i64, i64, vp, sz, ctypes.POINTER(MpOptions), i64, i64, vp]
+    lib.hsc_b200_mp_begin_lengths.restype = ctypes.c_int
+    lib.hsc_b200_mp_begin_lengths.argtypes = [vp, vp, vp, i64, i64, ctypes.POINTER(i64), vp, sz, ctypes.POINTER(MpOptions), vp]
     lib.hsc_b200_mp_run.restype = ctypes.c_int
     lib.hsc_b200_mp_run.argtypes = [vp, vp, vp, vp, i64, ctypes.POINTER(SignalState), vp]
     lib.hsc_b200_mp_states.restype = ctypes.c_int

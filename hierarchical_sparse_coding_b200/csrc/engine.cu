@@ -6,6 +6,7 @@
 #include <string.h>
 #include <math.h>
 
+#include <algorithm>
 #include <string>
 #include <vector>
 
@@ -105,6 +106,11 @@ struct hsc_engine {
     unsigned char* ws = nullptr;
     void* resid = nullptr;
     hsc_mp_options opt{};
+    // per-signal lengths of the encode in flight (hsc_b200_mp_begin_lengths): a device copy owned by this handle, read by
+    // every hsc_b200_mp_run of that encode; has_len = false for uniform encodes
+    int* len_dev = nullptr;
+    long long len_cap = 0;
+    bool has_len = false;
 };
 
 namespace {
@@ -303,6 +309,7 @@ int run_t(hsc_engine* e, int32_t* evp, int32_t* evi, void* evc, long long cap, c
     MpArgs<real> a;
     const Layout& l = e->lay;
     a.T = (int)e->T; a.K = (int)e->K; a.L = (int)e->L; a.F = (int)e->F; a.off = centre_offset((int)e->L);
+    a.len = e->has_len ? e->len_dev : nullptr;
     a.G1 = l.G1; a.n2 = l.n2; a.G2 = l.G2; a.n3 = l.n3;
     a.D = (const real*)e->D_dev; a.G = (const real*)e->G_dev;
     a.w = (e->opt.use_weights && e->w_dev) ? (const real*)e->w_dev : nullptr;
@@ -452,13 +459,19 @@ int run_t(hsc_engine* e, int32_t* evp, int32_t* evi, void* evc, long long cap, c
                    (2 * e->L - 1 + l.G1 - 1) / l.G1 + 1 <= kDirtyMax && (long long)l.G1 * e->K < (1ll << 32);
             if (fast) {
                 const size_t smem = dyn_smem + (size_t)l.n2 * sizeof(unsigned long long) + slot3_bytes;
-                HSC_CUDA(e, cudaFuncSetAttribute(locomp_fast_kernel<float, 256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                locomp_fast_kernel<float, 256><<<(unsigned)e->S, 256, smem, st>>>(a);
+                if (a.len) {
+                    HSC_CUDA(e, cudaFuncSetAttribute(locomp_fast_kernel<float, 256, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+                    locomp_fast_kernel<float, 256, true><<<(unsigned)e->S, 256, smem, st>>>(a);
+                } else {
+                    HSC_CUDA(e, cudaFuncSetAttribute(locomp_fast_kernel<float, 256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+                    locomp_fast_kernel<float, 256><<<(unsigned)e->S, 256, smem, st>>>(a);
+                }
             }
         }
         if (!fast) {
             a.tma_rows = a.tma_stages = a.tma_bytes = 0;
-            locomp_kernel<real, 128><<<(unsigned)e->S, 128, 0, st>>>(a);      // 4 CTAs of 128 threads x 128 registers per SM
+            if (a.len) locomp_kernel<real, 128, true><<<(unsigned)e->S, 128, 0, st>>>(a);
+            else locomp_kernel<real, 128><<<(unsigned)e->S, 128, 0, st>>>(a);      // 4 CTAs of 128 threads x 128 registers per SM
         }
         e->launches++;
         HSC_CUDA(e, cudaGetLastError());
@@ -477,13 +490,17 @@ int run_t(hsc_engine* e, int32_t* evp, int32_t* evi, void* evc, long long cap, c
         static const int smem_kb = getenv("HSC_K2_SMEM_KB") ? atoi(getenv("HSC_K2_SMEM_KB")) : 0;
         if (smem_kb > 0 && dyn_smem > 0 && dyn_smem < (size_t)smem_kb * 1024) dyn_smem = (size_t)smem_kb * 1024;
     }
-#define HSC_LAUNCH_K2(NT_, MINB_, VIF_, TMA_, SMH_, RPS_)                                                                        \
+#define HSC_LAUNCH_K2_K(KERNEL_, NT_, MINB_, VIF_, TMA_, SMH_, RPS_)                                                             \
     do {                                                                                                                          \
         if (dyn_smem > 0)                                                                                                         \
-            HSC_CUDA(e, cudaFuncSetAttribute(pursuit_kernel<real, NT_, MINB_, VIF_, TMA_, SMH_, RPS_>,                            \
+            HSC_CUDA(e, cudaFuncSetAttribute(KERNEL_<real, NT_, MINB_, VIF_, TMA_, SMH_, RPS_>,                                   \
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn_smem));                        \
-        pursuit_kernel<real, NT_, MINB_, VIF_, TMA_, SMH_, RPS_><<<(unsigned)e->S, NT_, dyn_smem, st>>>(a);                       \
+        KERNEL_<real, NT_, MINB_, VIF_, TMA_, SMH_, RPS_><<<(unsigned)e->S, NT_, dyn_smem, st>>>(a);                              \
     } while (0)
+#define HSC_LAUNCH_K2(NT_, MINB_, VIF_, TMA_, SMH_, RPS_) HSC_LAUNCH_K2_K(pursuit_kernel, NT_, MINB_, VIF_, TMA_, SMH_, RPS_)
+#define HSC_LAUNCH_K2_R(NT_, MINB_, VIF_, TMA_, SMH_, RPS_) HSC_LAUNCH_K2_K(pursuit_kernel_ragged, NT_, MINB_, VIF_, TMA_, SMH_, RPS_)
+    // ragged batches (per-signal lengths) are instantiated for the default launch shape only
+    if (a.len && (variant == 0 || variant == 6)) return fail(e, HSC_E_UNSUPPORTED, "mp_run: per-signal lengths need the default K2 launch shape (HSC_PURSUIT_VARIANT=4)");
     switch (variant) {
         case 0:            // register path, 2 CTAs per SM
             HSC_LAUNCH_K2(256, 2, 4, false, false, 1);
@@ -496,6 +513,13 @@ int run_t(hsc_engine* e, int32_t* evp, int32_t* evi, void* evc, long long cap, c
             else HSC_LAUNCH_K2(128, 4, 2, false, false, 1);
             break;
         default:           // 8 warps per signal, 64 registers per thread
+            if (a.len) {
+                if (tiny_row && smh) HSC_LAUNCH_K2_R(256, 4, 2, false, true, 1);
+                else if (dyn_smem > 0 && smh) HSC_LAUNCH_K2_R(256, 4, 2, true, true, 1);
+                else if (dyn_smem > 0) HSC_LAUNCH_K2_R(256, 4, 2, true, false, 1);
+                else HSC_LAUNCH_K2_R(256, 4, 2, false, false, 1);
+                break;
+            }
             if (tiny_row && smh) HSC_LAUNCH_K2(256, 4, 2, false, true, 1);
             else if (dyn_smem > 0 && smh) HSC_LAUNCH_K2(256, 4, 2, true, true, 1);
             else if (dyn_smem > 0) HSC_LAUNCH_K2(256, 4, 2, true, false, 1);
@@ -503,6 +527,8 @@ int run_t(hsc_engine* e, int32_t* evp, int32_t* evi, void* evc, long long cap, c
             break;
     }
 #undef HSC_LAUNCH_K2
+#undef HSC_LAUNCH_K2_R
+#undef HSC_LAUNCH_K2_K
     e->launches++;
     HSC_CUDA(e, cudaGetLastError());
 #ifdef HSC_PROFILE_PHASES
@@ -613,6 +639,8 @@ void free_scratch(hsc_engine* e) {
     e->tc_xsplit = nullptr; e->tc_xsplit_bytes = 0;
     if (e->canon_scratch) cudaFree(e->canon_scratch);
     e->canon_scratch = nullptr; e->canon_scratch_bytes = 0;
+    if (e->len_dev) cudaFree(e->len_dev);
+    e->len_dev = nullptr; e->len_cap = 0; e->has_len = false;
 }
 
 void free_dictionary(hsc_engine* e) {
@@ -719,8 +747,13 @@ size_t hsc_b200_workspace_bytes(const hsc_engine* e, int64_t S, int64_t T) {
     return make_layout(S, T, e->K, e->L, e->dtype == HSC_F32 ? 4 : 8, e->F).total;
 }
 
-int hsc_b200_mp_begin_part(hsc_engine* e, const void* x_dev, void* residual_dev, int64_t S, int64_t T, void* workspace_dev,
-                           size_t workspace_bytes, const hsc_mp_options* opt, int64_t s_lo, int64_t s_count, void* stream) {
+}  // extern "C"
+
+namespace {
+
+// hsc_b200_mp_begin_part, and hsc_b200_mp_begin_lengths when lengths_host is set (then s_lo = 0, s_count = S).
+int mp_begin_impl(hsc_engine* e, const void* x_dev, void* residual_dev, int64_t S, int64_t T, const int64_t* lengths_host,
+                  void* workspace_dev, size_t workspace_bytes, const hsc_mp_options* opt, int64_t s_lo, int64_t s_count, void* stream) {
     if (!e) return HSC_E_INVALID;
     if (!e->D_dev) return fail(e, HSC_E_STATE, "mp_begin: no dictionary set");
     if (!x_dev || !residual_dev || !workspace_dev || !opt || S <= 0 || T <= 0 || S > 65535 || s_lo < 0 || s_count <= 0 ||
@@ -734,13 +767,30 @@ int hsc_b200_mp_begin_part(hsc_engine* e, const void* x_dev, void* residual_dev,
     if (opt->method != 0 && opt->method != 1) return fail(e, HSC_E_INVALID, "mp_begin: method must be 0 (MP) or 1 (LoCOMP)");
     if (opt->nb_blocks != 1) {
         if (opt->nb_blocks == 0 || opt->nb_blocks < -1) return fail(e, HSC_E_INVALID, "mp_begin: nbBlocks must be 1, > 1 or -1 ('auto')");
-        long long bs = opt->nb_blocks < 0 ? 4 * e->L : T / opt->nb_blocks;
-        if (bs & 1) bs += 1;
-        if (bs < 2) return fail(e, HSC_E_INVALID, "mp_begin: nbBlocks larger than T/2");
-        if ((T + bs - 1) / bs + 1 > l.ncand_max) return fail(e, HSC_E_UNSUPPORTED, "mp_begin: too many selection blocks for the candidate lists");
+        // (per signal: the block size follows each signal's own length)
+        for (int64_t s = 0; s < (lengths_host ? S : 1); ++s) {
+            const long long Ts = lengths_host ? lengths_host[s] : T;
+            long long bs = opt->nb_blocks < 0 ? 4 * e->L : Ts / opt->nb_blocks;
+            if (bs & 1) bs += 1;
+            if (bs < 2) return fail(e, HSC_E_INVALID, "mp_begin: nbBlocks larger than T/2");
+            if ((Ts + bs - 1) / bs + 1 > l.ncand_max) return fail(e, HSC_E_UNSUPPORTED, "mp_begin: too many selection blocks for the candidate lists");
+        }
     }
     cudaStream_t st = (cudaStream_t)stream;
     { int rcg = ensure_gram(e); if (rcg != HSC_OK) return rcg; }
+    if (lengths_host) {            // the handle's copy of the lengths, read by this encode's hsc_b200_mp_run calls
+        if (e->len_cap < S) {
+            if (e->len_dev) cudaFree(e->len_dev);
+            e->len_dev = nullptr; e->len_cap = 0;
+            HSC_CUDA(e, cudaMalloc((void**)&e->len_dev, (size_t)S * sizeof(int)));
+            e->len_cap = S;
+        }
+        std::vector<int> len32((size_t)S);
+        for (int64_t s = 0; s < S; ++s) len32[(size_t)s] = (int)lengths_host[s];
+        // (pageable source: staged before the call returns, the vector may go)
+        HSC_CUDA(e, cudaMemcpyAsync(e->len_dev, len32.data(), (size_t)S * sizeof(int), cudaMemcpyHostToDevice, st));
+    }
+    e->has_len = lengths_host != nullptr;
     e->S = S; e->T = T; e->lay = l; e->ws = (unsigned char*)workspace_dev; e->resid = residual_dev; e->opt = *opt;
     // everything below touches only signals [s_lo, s_lo + s_count) of the S-signal arrays
     const size_t sig_x = (size_t)T * e->F * rsz, sig_map = (size_t)T * e->K * rsz;
@@ -752,6 +802,15 @@ int hsc_b200_mp_begin_part(hsc_engine* e, const void* x_dev, void* residual_dev,
     const int64_t Sc = s_count;
     if ((const void*)xp != (const void*)rp)
         HSC_CUDA(e, cudaMemcpyAsync(rp, xp, (size_t)Sc * sig_x, cudaMemcpyDeviceToDevice, st));
+    if (e->has_len) {
+        // the padding of every signal <- 0 in the residual, which K1 then reads instead of x (zero_signal_tails_kernel)
+        const unsigned tail_gx = (unsigned)std::min<long long>((T * e->F + 255) / 256, 32);
+        if (e->dtype == HSC_F32) zero_signal_tails_kernel<float><<<dim3(tail_gx, (unsigned)Sc), 256, 0, st>>>((float*)rp, e->len_dev, (int)T, (int)e->F);
+        else zero_signal_tails_kernel<double><<<dim3(tail_gx, (unsigned)Sc), 256, 0, st>>>((double*)rp, e->len_dev, (int)T, (int)e->F);
+        e->launches++;
+        HSC_CUDA(e, cudaGetLastError());
+        xp = rp;
+    }
     // Level-1 keys: fused into the tensor-core K1 epilogue when every 32-column chunk of the product lies in
     // one time row and the scores are unweighted; otherwise a grid-wide pass over the map builds them.
     static const bool force_simt = getenv("HSC_K1") && !strcmp(getenv("HSC_K1"), "simt");
@@ -783,11 +842,36 @@ int hsc_b200_mp_begin_part(hsc_engine* e, const void* x_dev, void* residual_dev,
         e->launches++;
         HSC_CUDA(e, cudaGetLastError());
     }
+    if (e->has_len) {
+        const unsigned gx = (unsigned)std::min<long long>((T + 255) / 256, 32);
+        if (e->dtype == HSC_F32) clear_tail_keys_kernel<float><<<dim3(gx, (unsigned)Sc), 256, 0, st>>>((float*)v1p, i1p, e->len_dev, (int)T);
+        else clear_tail_keys_kernel<double><<<dim3(gx, (unsigned)Sc), 256, 0, st>>>((double*)v1p, i1p, e->len_dev, (int)T);
+        e->launches++;
+        HSC_CUDA(e, cudaGetLastError());
+    }
     HSC_CUDA(e, cudaMemsetAsync(e->ws + l.off_bitmap + (size_t)s_lo * l.bitmap_words * sizeof(unsigned), 0,
                                 (size_t)Sc * l.bitmap_words * sizeof(unsigned), st));
     HSC_CUDA(e, cudaMemsetAsync(e->ws + l.off_state + (size_t)s_lo * sizeof(hsc_signal_state), 0, (size_t)Sc * sizeof(hsc_signal_state), st));
     e->active = true;
     return HSC_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int hsc_b200_mp_begin_part(hsc_engine* e, const void* x_dev, void* residual_dev, int64_t S, int64_t T, void* workspace_dev,
+                           size_t workspace_bytes, const hsc_mp_options* opt, int64_t s_lo, int64_t s_count, void* stream) {
+    return mp_begin_impl(e, x_dev, residual_dev, S, T, nullptr, workspace_dev, workspace_bytes, opt, s_lo, s_count, stream);
+}
+
+int hsc_b200_mp_begin_lengths(hsc_engine* e, const void* x_dev, void* residual_dev, int64_t S, int64_t T, const int64_t* lengths_host,
+                              void* workspace_dev, size_t workspace_bytes, const hsc_mp_options* opt, void* stream) {
+    if (!e) return HSC_E_INVALID;
+    if (!lengths_host || S <= 0 || S > 65535) return fail(e, HSC_E_INVALID, "mp_begin_lengths: bad arguments");
+    for (int64_t s = 0; s < S; ++s)
+        if (lengths_host[s] < 1 || lengths_host[s] > T) return fail(e, HSC_E_INVALID, "mp_begin_lengths: every length must lie in [1, T]");
+    return mp_begin_impl(e, x_dev, residual_dev, S, T, lengths_host, workspace_dev, workspace_bytes, opt, 0, S, stream);
 }
 
 int hsc_b200_mp_begin(hsc_engine* e, const void* x_dev, void* residual_dev, int64_t S, int64_t T, void* workspace_dev,

@@ -25,10 +25,10 @@ constexpr int kLocompOverlayBytes = kLocompSmemGroup * (kLocompSmemGroup + 1) * 
 constexpr int HSC_STOP_STALL_ = 9;        // |delta E| < eps (:1377-1381)
 constexpr int HSC_STOP_GROUP_ = 10;       // common-support group larger than kLocompMaxGroup
 
-// <atom (ti,ki), atom (tj,kj)> with both atoms clipped to [0,T).
-template <typename real>
+// <atom (ti,ki), atom (tj,kj)> with both atoms clipped to [0,T) (T: the signal's length).
+template <typename real, bool RAGGED>
 __device__ double atom_inner(const MpArgs<real>& a, int ti, int ki, int tj, int kj) {
-    const int L = a.L, F = a.F, T = a.T, off = a.off;
+    const int L = a.L, F = a.F, T = signal_length<RAGGED>(a), off = a.off;
     const int d = tj - ti;
     if (d >= L || d <= -L) return 0.0;
     const int si = ti - off, sj = tj - off;
@@ -50,9 +50,9 @@ __device__ double atom_inner(const MpArgs<real>& a, int ti, int ki, int tj, int 
 //            residual with reflect padding (hsc/modeling.py:1046).
 // All incremental updates of a group must precede all absolute ones: a re-correlated row already reflects
 // every residual change of the group, so a later increment on it would count an atom twice.
-template <typename real, int NT>
+template <typename real, int NT, bool RAGGED>
 __device__ void locomp_window(const MpArgs<real>& a, real* map_s, const real* res_s, int t, int k, real coef, int phase) {
-    const int T = a.T, K = a.K, L = a.L, F = a.F, off = a.off, W = 2 * L - 1, LF = L * F;
+    const int T = signal_length<RAGGED>(a), K = a.K, L = a.L, F = a.F, off = a.off, W = 2 * L - 1, LF = L * F;
     const int tid = threadIdx.x;
     const int row_lo = max(t - (L - 1), 0), row_hi = min(t + (L - 1), T - 1);
     const long long first = (long long)t - off - (L - 1);
@@ -83,18 +83,18 @@ __device__ void locomp_window(const MpArgs<real>& a, real* map_s, const real* re
     __syncthreads();
 }
 
-template <typename real, int NT>
+template <typename real, int NT, bool RAGGED = false>       // RAGGED: per-signal lengths (see pursuit_kernel)
 __global__ void __launch_bounds__(NT, 512 / NT) locomp_kernel(MpArgs<real> a) {       // 512 threads per SM: 128 registers each
     const int s = blockIdx.x;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     constexpr int NW = NT / 32;
     constexpr int NG = kLocompMaxGroup;
-    const int T = a.T, K = a.K, L = a.L, F = a.F, off = a.off, LF = L * F;
+    const int T = RAGGED ? a.len[s] : a.T, K = a.K, L = a.L, F = a.F, off = a.off, LF = L * F;     // (a.T: the row stride)
 
-    real* map_s = a.map + (long long)s * T * K;
-    real* res_s = a.resid + (long long)s * T * F;
-    real* v1 = a.val1 + (long long)s * T;
-    int* i1 = a.idx1 + (long long)s * T;
+    real* map_s = a.map + (long long)s * a.T * K;
+    real* res_s = a.resid + (long long)s * a.T * F;
+    real* v1 = a.val1 + (long long)s * a.T;
+    int* i1 = a.idx1 + (long long)s * a.T;
     real* v2 = a.val2 + (long long)s * a.n2;
     int* i2 = a.idx2 + (long long)s * a.n2;
     real* v3 = a.val3 + (long long)s * a.n3;
@@ -170,7 +170,7 @@ __global__ void __launch_bounds__(NT, 512 / NT) locomp_kernel(MpArgs<real> a) { 
             break;
         }
         if (block_mode && new_pass) {
-            const int n = build_pass_list<real, NT>(a, map_s, res_s, v1, i1, ct, ck, cc, st.offset_flag, st.energy_signal);
+            const int n = build_pass_list<real, NT, RAGGED>(a, map_s, res_s, v1, i1, ct, ck, cc, st.offset_flag, st.energy_signal);
             if (tid == 0) {
                 st.pass_count = n;
                 st.pass_cursor = 0;
@@ -295,7 +295,7 @@ __global__ void __launch_bounds__(NT, 512 / NT) locomp_kernel(MpArgs<real> a) { 
             for (int e = tid; e < n * n; e += NT) {
                 const int i = e / n, j = e - i * n;
                 if (j >= i) {
-                    const double v = atom_inner(a, g_t[i], g_k[i], g_t[j], g_k[j]);
+                    const double v = atom_inner<real, RAGGED>(a, g_t[i], g_k[i], g_t[j], g_k[j]);
                     g_A(i, j) = v;
                     g_A(j, i) = v;
                 }
@@ -413,13 +413,13 @@ __global__ void __launch_bounds__(NT, 512 / NT) locomp_kernel(MpArgs<real> a) { 
                     else gram_update_vec<real, 4, NT, 4, false>(K, L, a.w, map_s, Gk, v1, i1, ti, (real)g_x[i], gv);
                     __syncthreads();
                 } else {
-                    locomp_window<real, NT>(a, map_s, res_s, ti, g_k[i], (real)g_x[i], 0);
+                    locomp_window<real, NT, RAGGED>(a, map_s, res_s, ti, g_k[i], (real)g_x[i], 0);
                 }
             }
             for (int i = 0; i < ng; ++i) {
                 const int ti = g_t[i];
                 const bool edge_i = (ti - (L - 1) < off) || (ti + (L - 1) > T - L + off);
-                if (edge_i) locomp_window<real, NT>(a, map_s, res_s, ti, g_k[i], (real)g_x[i], 1);
+                if (edge_i) locomp_window<real, NT, RAGGED>(a, map_s, res_s, ti, g_k[i], (real)g_x[i], 1);
             }
             for (int i = 0; i < ng; ++i) {
                 const int ti = g_t[i];
@@ -496,22 +496,24 @@ __global__ void __launch_bounds__(NT, 512 / NT) locomp_kernel(MpArgs<real> a) { 
 //  * the refit scratch (normal matrix, right-hand side, rank-sort keys) overlaid on the stage rings, which are idle while a
 //    group is fitted; the fitted group (t, k, delta) goes to a small per-signal list in global memory for the apply phase.
 // Groups that contain an edge atom keep the two-phase element-wise windows (all increments before all re-correlations).
-template <typename real, int NT>
+template <typename real, int NT, bool RAGGED = false>       // RAGGED: per-signal lengths (see pursuit_kernel)
 __global__ void __launch_bounds__(NT, 4) locomp_fast_kernel(MpArgs<real> a) {
     const int s = blockIdx.x;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     constexpr int NW = NT / 32;
     constexpr int NG = kLocompMaxGroup;
-    const int T = a.T, K = a.K, L = a.L, F = a.F, off = a.off, LF = L * F, W = 2 * L - 1;
+    const int Tst = a.T, K = a.K, L = a.L, F = a.F, off = a.off, LF = L * F, W = 2 * L - 1;     // Tst: the row stride
 
+    // per-signal base pointers and a ragged signal's length T (which bounds everything below; the arrays keep the row stride
+    // Tst) live in shared memory, loaded at the use sites (CtaLength)
     struct Ctx { real* map_s; real* res_s; real* v1; int* i1; unsigned* bits; int* evp; int* evi; real* evc; int* ct; int* ck; real* cc;
                  double* gl_x; int* gl_t; int* gl_k; };
     __shared__ Ctx cx;
     if (tid == 0) {
-        cx.map_s = a.map + (long long)s * T * K;
-        cx.res_s = a.resid + (long long)s * T * F;
-        cx.v1 = a.val1 + (long long)s * T;
-        cx.i1 = a.idx1 + (long long)s * T;
+        cx.map_s = a.map + (long long)s * Tst * K;
+        cx.res_s = a.resid + (long long)s * Tst * F;
+        cx.v1 = a.val1 + (long long)s * Tst;
+        cx.i1 = a.idx1 + (long long)s * Tst;
         cx.bits = a.bitmap + (long long)s * a.bitmap_words;
         cx.evp = a.ev_pos + (long long)s * a.cap;
         cx.evi = a.ev_idx + (long long)s * a.cap;
@@ -522,7 +524,9 @@ __global__ void __launch_bounds__(NT, 4) locomp_fast_kernel(MpArgs<real> a) {
         cx.gl_x = a.locomp_scratch + (long long)s * kLocompScratchStride + (long long)NG * (NG + 1);
         cx.gl_t = reinterpret_cast<int*>(cx.gl_x + NG);
         cx.gl_k = cx.gl_t + NG;
+        if constexpr (RAGGED) CtaLength<true>::set(a.len[s]);
     }
+#define T (CtaLength<RAGGED>::get(Tst))
 #define map_s (cx.map_s)
 #define res_s (cx.res_s)
 #define v1 (cx.v1)
@@ -623,7 +627,7 @@ __global__ void __launch_bounds__(NT, 4) locomp_fast_kernel(MpArgs<real> a) {
             break;
         }
         if (block_mode && new_pass) {
-            const int n = build_pass_list<real, NT>(a, map_s, res_s, v1, i1, cx.ct, cx.ck, cx.cc, st.offset_flag, st.energy_signal);
+            const int n = build_pass_list<real, NT, RAGGED>(a, map_s, res_s, v1, i1, cx.ct, cx.ck, cx.cc, st.offset_flag, st.energy_signal);
             if (tid == 0) {
                 st.pass_count = n;
                 st.pass_cursor = 0;
@@ -742,7 +746,7 @@ __global__ void __launch_bounds__(NT, 4) locomp_fast_kernel(MpArgs<real> a) {
             for (int e = tid; e < n * n; e += NT) {
                 const int i = e / n, j = e - i * n;
                 if (j >= i) {
-                    const double v = atom_inner(a, g_t[i], g_k[i], g_t[j], g_k[j]);
+                    const double v = atom_inner<real, RAGGED>(a, g_t[i], g_k[i], g_t[j], g_k[j]);
                     g_A(i, j) = v;
                     g_A(j, i) = v;
                 }
@@ -855,7 +859,7 @@ __global__ void __launch_bounds__(NT, 4) locomp_fast_kernel(MpArgs<real> a) {
             const real ci = GL_X(i);
             const bool edge_i = (ti - (L - 1) < off) || (ti + (L - 1) > T - L + off);
             if (edge_i) {
-                locomp_window<real, NT>(a, map_s, res_s, ti, ki, ci, 0);         // increments on the rows that are not re-correlated
+                locomp_window<real, NT, RAGGED>(a, map_s, res_s, ti, ki, ci, 0);         // increments on the rows that are not re-correlated
                 fence_proxy_async_all();            // generic map writes -> later bulk loads of these rows
                 __syncthreads();
                 continue;
@@ -893,7 +897,7 @@ __global__ void __launch_bounds__(NT, 4) locomp_fast_kernel(MpArgs<real> a) {
         if (any_edge) {
             for (int i = 0; i < ng; ++i) {
                 const int ti = GL_T(i);
-                if ((ti - (L - 1) < off) || (ti + (L - 1) > T - L + off)) locomp_window<real, NT>(a, map_s, res_s, ti, GL_K(i), GL_X(i), 1);
+                if ((ti - (L - 1) < off) || (ti + (L - 1) > T - L + off)) locomp_window<real, NT, RAGGED>(a, map_s, res_s, ti, GL_K(i), GL_X(i), 1);
             }
             fence_proxy_async_all();
             __syncthreads();
@@ -975,6 +979,7 @@ __global__ void __launch_bounds__(NT, 4) locomp_fast_kernel(MpArgs<real> a) {
 #undef GL_T
 #undef GL_K
 #undef GL_X
+#undef T
 #undef map_s
 #undef res_s
 #undef v1

@@ -26,7 +26,7 @@ namespace hsc {
 
 template <typename real>
 struct MpArgs {
-    int T, K, L, F, off;
+    int T, K, L, F, off;  // T: row stride of every [S][T][...] array, and the length of every signal unless `len` is set
     int G1, n2, G2, n3;
     const real* D;        // [K][L][F]
     const real* G;        // [K][2L-1][K]
@@ -65,7 +65,15 @@ struct MpArgs {
     int early_issue;          // 1: the first window chunks of an interior atom are issued right after the pick (bulk-copy path)
     float rerank_tol;         // float maps: candidates within rerank_tol * (best score + largest initial score) of the best
                               // approximate score are re-scored from the residual before the pick (0 = off)
+    const int* len;           // [S] per-signal lengths in [1, T] (hsc_b200_mp_begin_lengths), or nullptr: all signals have T samples
 };
+
+// Length of the signal of this CTA (one CTA per signal).  Every BOUND of the pursuit - edge and overhang tests, window
+// and residual clipping, group and block ranges, the energy and residual-scale scans - uses it; a.T stays the stride.
+// Samples and map rows at or past it are never read: a ragged batch encodes each signal as if it were alone.
+// RAGGED is a compile-time choice of every kernel and helper that bounds with it: a uniform launch compiles to a.T alone.
+template <bool RAGGED, typename real>
+__device__ __forceinline__ int signal_length(const MpArgs<real>& a) { return RAGGED ? __ldg(a.len + blockIdx.x) : a.T; }
 
 // Packed keys of the shared-memory argmax hierarchy (float scores, pursuit_kernel<..., SMH = true>): the score's
 // bit pattern (non-negative floats order like unsigned integers) above ~(row_in_group*K + filter), so that an
@@ -229,6 +237,43 @@ __global__ void __launch_bounds__(256) rowkey_kernel(const real* __restrict__ ma
                 i1[row] = bi[r];
             }
         }
+    }
+}
+
+// The signal length of a CTA inside a kernel: a ragged launch keeps it in a shared-memory slot that is re-read at every
+// use (never a live register of the persistent loops); a uniform launch uses its own value.  Only the ragged
+// specialization declares the slot - a shared variable in the uniform kernels changes their register allocation.
+template <bool RAGGED> struct CtaLength {
+    static __device__ __forceinline__ void set(int) {}
+    static __device__ __forceinline__ int get(int uniform) { return uniform; }
+};
+template <> struct CtaLength<true> {
+    static __device__ __forceinline__ volatile int* slot() { __shared__ int len; return &len; }
+    static __device__ __forceinline__ void set(int v) { *slot() = v; }
+    static __device__ __forceinline__ int get(int) { return *slot(); }
+};
+
+// Ragged batches (hsc_b200_mp_begin_lengths).  Before K1: samples [len[s], T) of signal s's residual <- 0, so that K1, which
+// then reads the residual, sees each signal followed by the 'same' zero padding of a signal of len[s] samples
+// (hsc/modeling.py:161-164): map rows below len[s], the per-signal scale of the tensor-core path and the signal energy are
+// those of the signal alone, whatever the padding held.  Grid: (x, S).
+template <typename real>
+__global__ void __launch_bounds__(256) zero_signal_tails_kernel(real* __restrict__ x, const int* __restrict__ len, int T, int F) {
+    const long long s = blockIdx.y;
+    const long long n = (long long)T * F;
+    real* xs = x + s * n;
+    for (long long i = (long long)len[s] * F + blockIdx.x * 256ll + threadIdx.x; i < n; i += (long long)gridDim.x * 256)
+        xs[i] = (real)0;
+}
+
+// ... and after K1: the level-1 keys of rows [len[s], T) <- "no candidate", so that no selection can reach them.
+template <typename real>
+__global__ void __launch_bounds__(256) clear_tail_keys_kernel(real* __restrict__ val1, int* __restrict__ idx1, const int* __restrict__ len,
+                                                              int T) {
+    const long long s = blockIdx.y;
+    for (long long r = len[s] + blockIdx.x * 256ll + threadIdx.x; r < T; r += (long long)gridDim.x * 256) {
+        val1[s * T + r] = (real)0;
+        idx1[s * T + r] = 0;
     }
 }
 
@@ -715,11 +760,11 @@ __device__ __forceinline__ void mark_overhang_rows(hsc_signal_state& st, int lo,
 // Score of map entry (r, k) from the residual by one warp: <r[r-off : r-off+L], D[k]> in float64, clipped (= zero
 // padded) at the signal ends.  Returns the signed value; only meaningful for rows that are NOT reflect-rewritten.
 template <typename real>
-__device__ __forceinline__ double residual_dot_warp(const MpArgs<real>& a, const real* res_s, int r, int k) {
+__device__ __forceinline__ double residual_dot_warp(const MpArgs<real>& a, const real* res_s, int r, int k, int T) {
     const int lane = threadIdx.x & 31;
     const int sstart = r - a.off;
     const int jlo = sstart < 0 ? -sstart : 0;
-    const int jhi = (sstart + a.L > a.T) ? (a.T - sstart) : a.L;
+    const int jhi = (sstart + a.L > T) ? (T - sstart) : a.L;
     const real* rr = res_s + (long long)sstart * a.F;
     const real* dd = a.D + (long long)k * a.L * a.F;
     double acc = 0.0;
@@ -732,8 +777,9 @@ template <typename real>
 __device__ __forceinline__ double exact_score_warp(const MpArgs<real>& a, const hsc_signal_state& st, const real* map_s, const real* res_s,
                                                    int r, int k) {
     double sc;
-    const bool overhang = (r < a.off) || (r > a.T - a.L + a.off);
-    if (!overhang || !overhang_row_written(st, r, a.off, a.T, a.L)) sc = fabs(residual_dot_warp<real>(a, res_s, r, k));
+    const int T = a.T;
+    const bool overhang = (r < a.off) || (r > T - a.L + a.off);
+    if (!overhang || !overhang_row_written(st, r, a.off, T, a.L)) sc = fabs(residual_dot_warp<real>(a, res_s, r, k, T));
     else sc = fabs((double)__ldcg(map_s + (long long)r * a.K + k));
     return a.w ? sc * fabs((double)a.w[k]) : sc;
 }
@@ -744,33 +790,34 @@ __device__ __forceinline__ double exact_score_warp(const MpArgs<real>& a, const 
 // `lvl2(g)` gives the approximate best score of 128-row group g.
 constexpr int kRerankMax = 32;          // candidates per stage; beyond that the surplus is dropped (the window holds a handful)
 
-template <typename real, typename Lvl2>
+template <bool RAGGED, typename real, typename Lvl2>
 __device__ __forceinline__ void rerank_candidates(const MpArgs<real>& a, const hsc_signal_state& st, const real* map_s, const real* res_s,
                                                   const real* v1, Lvl2 lvl2, uint32_t slot3_saddr, int g1s, real thr, int& t_out, int& k_out) {
     __shared__ int cand_g[kRerankMax], cand_r[kRerankMax], cand_k[kRerankMax];
     const int lane = threadIdx.x & 31;
-    const int T = a.T, K = a.K, L = a.L, F = a.F, LF = a.L * a.F;
+    const int T = signal_length<RAGGED>(a), K = a.K, L = a.L, F = a.F, LF = a.L * a.F;
+    const int n2 = RAGGED ? (T + (1 << g1s) - 1) >> g1s : a.n2;    // the signal's groups (a.n2: those of the stride)
     // stage 1: groups - through the block scores where the hierarchy has them (a block below thr holds no candidate group)
     int ng = 0;
     if (slot3_saddr) {
-        const int n3 = (a.n2 + 31) >> 5;
+        const int n3 = (n2 + 31) >> 5;
         for (int b0 = 0; b0 < n3; b0 += 32) {
             const int b = b0 + lane;
             unsigned mb = __ballot_sync(0xffffffffu, b < n3 && (real)__uint_as_float(lds_u32(slot3_saddr + 4u * (unsigned)b)) >= thr);
             while (mb) {                                           // (warp-uniform) candidate blocks, ascending
                 const int g = ((b0 + __ffs(mb) - 1) << 5) + lane;
                 mb &= mb - 1;
-                const bool h = g < a.n2 && lvl2(g) >= thr;
+                const bool h = g < n2 && lvl2(g) >= thr;
                 const unsigned m = __ballot_sync(0xffffffffu, h);
                 if (h) { const int slot = ng + __popc(m & ((1u << lane) - 1u)); if (slot < kRerankMax) cand_g[slot] = g; }
                 ng += __popc(m);
             }
         }
     } else
-    for (int g0 = 0; g0 < a.n2; g0 += 128) {                       // four independent key loads per lane and step
+    for (int g0 = 0; g0 < n2; g0 += 128) {                         // four independent key loads per lane and step
         bool h[4];
 #pragma unroll
-        for (int u = 0; u < 4; ++u) { const int g = g0 + u * 32 + lane; h[u] = g < a.n2 && lvl2(g) >= thr; }
+        for (int u = 0; u < 4; ++u) { const int g = g0 + u * 32 + lane; h[u] = g < n2 && lvl2(g) >= thr; }
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
             const unsigned m = __ballot_sync(0xffffffffu, h[u]);
@@ -872,11 +919,11 @@ __device__ __forceinline__ void rerank_candidates(const MpArgs<real>& a, const h
 
 // Fast test by one warp, after the approximate pick (t, k): is any OTHER entry of the atom's own row or of the other rows
 // of its 128-row group within tol?  (Other groups are tested by the caller on the group keys.)
-template <typename real>
+template <typename real, bool RAGGED>
 __device__ __forceinline__ bool near_tie_in_group(const MpArgs<real>& a, const real* map_s, const real* v1, int g1s, int t, int k, real thr) {
     const int lane = threadIdx.x & 31;
     bool amb = false;
-    const int r0 = (t >> g1s) << g1s, r1 = min(r0 + (1 << g1s), a.T);
+    const int r0 = (t >> g1s) << g1s, r1 = min(r0 + (1 << g1s), signal_length<RAGGED>(a));
     const real* mrow = map_s + (long long)t * a.K;
     // every load of the test is issued before the first compare: the level-1 keys of the group's rows and the first 256
     // entries of the atom's map row fly together (one dependent round trip under load instead of two)
@@ -906,7 +953,7 @@ __device__ __forceinline__ bool near_tie_in_group(const MpArgs<real>& a, const r
 // entry score within the re-rank window of it - the other 128-row groups on their keys (SMH: `second`, a by-product of
 // warp 0's scan of the group keys), the other rows of the atom's group on their level-1 keys, the other filters of its row
 // on the map?  Returns the score threshold of the candidate set, or a negative value when the pick is unambiguous.
-template <typename real, bool SMH>
+template <typename real, bool SMH, bool RAGGED>
 __device__ __noinline__ real near_tie_watch(const MpArgs<real>& a, hsc_signal_state& st, const real* map_s, const real* res_s,
                                             const real* v1, const int* i1, const real* v2g, const real* v3g, const int* i3g, int g1s,
                                             int t, int k, real vbest, real second, uint32_t slot2_saddr, int next_g) {
@@ -932,11 +979,12 @@ __device__ __noinline__ real near_tie_watch(const MpArgs<real>& a, hsc_signal_st
         amb = second >= thr;
     } else {
         const int gsel = t >> g1s;
+        const int n2 = RAGGED ? (signal_length<RAGGED>(a) + (1 << g1s) - 1) >> g1s : a.n2;
         amb = false;
-        for (int e = lane; e < a.n2; e += 32) amb |= (e != gsel) && (v2g[e] >= thr);
+        for (int e = lane; e < n2; e += 32) amb |= (e != gsel) && (v2g[e] >= thr);
         amb = __any_sync(0xffffffffu, amb);
     }
-    if (!amb) amb = near_tie_in_group<real>(a, map_s, v1, g1s, t, k, thr);
+    if (!amb) amb = near_tie_in_group<real, RAGGED>(a, map_s, v1, g1s, t, k, thr);
     if constexpr (SMH) {
         // The best entry of the OTHER groups is, most of the time, the next pick (an update only changes the 2L-1 rows
         // around its atom): pull what its selection will read - the residual under its support, its map row, the level-1
@@ -967,14 +1015,14 @@ __device__ __noinline__ real near_tie_watch(const MpArgs<real>& a, hsc_signal_st
             if (lane == 0) {
                 const int s0 = max(t2 - a.off, 0);
                 p = res_s + (long long)s0 * a.F;
-                bytes = (unsigned)(min(t2 - a.off + a.L, a.T) - s0) * a.F * sizeof(real);
+                bytes = (unsigned)(min(t2 - a.off + a.L, signal_length<RAGGED>(a)) - s0) * a.F * sizeof(real);
             } else if (lane == 1) {
                 p = map_s + (long long)t2 * a.K;
                 bytes = (unsigned)a.K * sizeof(real);
             } else {
                 const int r0 = next_g << g1s;
                 p = v1 + r0;
-                bytes = (unsigned)(min(r0 + (1 << g1s), a.T) - r0) * sizeof(real);
+                bytes = (unsigned)(min(r0 + (1 << g1s), signal_length<RAGGED>(a)) - r0) * sizeof(real);
             }
             if ((((unsigned long long)p) & 15ull) == 0 && (bytes & 15u) == 0 && bytes > 0)
                 asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" :: "l"(p), "r"(bytes) : "memory");
@@ -985,20 +1033,21 @@ __device__ __noinline__ real near_tie_watch(const MpArgs<real>& a, hsc_signal_st
 
 // ... and its resolution, by warp 0, in the rare case the test fires: every entry with an approximate score >= thr is
 // re-scored from the residual and (t, k) becomes the best of them; returns its coefficient.
-template <typename real, bool SMH>
+template <typename real, bool SMH, bool RAGGED>
 __device__ __noinline__ real near_tie_resolve(const MpArgs<real>& a, hsc_signal_state& st, const real* map_s, const real* res_s,
                                               const real* v1, uint32_t slot2_saddr, const real* v2g, int g1s, real thr,
                                               int& t, int& k) {
     if constexpr (SMH) {
         auto lvl2 = [&](int g) { return (real)__uint_as_float(lds_u32(slot2_saddr + 8u * (unsigned)g + 4u)); };
-        rerank_candidates<real>(a, st, map_s, res_s, v1, lvl2, slot2_saddr + 8u * (unsigned)a.n2, g1s, thr, t, k);   // (slot3 follows slot2)
+        rerank_candidates<RAGGED, real>(a, st, map_s, res_s, v1, lvl2, slot2_saddr + 8u * (unsigned)a.n2, g1s, thr, t, k);   // (slot3 follows slot2)
     } else {
         auto lvl2 = [&](int g) { return v2g[g]; };
-        rerank_candidates<real>(a, st, map_s, res_s, v1, lvl2, 0u, g1s, thr, t, k);
+        rerank_candidates<RAGGED, real>(a, st, map_s, res_s, v1, lvl2, 0u, g1s, thr, t, k);
     }
-    const bool row_overhangs = (t < a.off) || (t > a.T - a.L + a.off);
-    const bool from_residual = a.coef_mode == 1 && (!row_overhangs || !overhang_row_written(st, t, a.off, a.T, a.L));
-    return from_residual ? (real)residual_dot_warp<real>(a, res_s, t, k) : __ldcg(map_s + (long long)t * a.K + k);
+    const int T = signal_length<RAGGED>(a);
+    const bool row_overhangs = (t < a.off) || (t > T - a.L + a.off);
+    const bool from_residual = a.coef_mode == 1 && (!row_overhangs || !overhang_row_written(st, t, a.off, T, a.L));
+    return from_residual ? (real)residual_dot_warp<real>(a, res_s, t, k, T) : __ldcg(map_s + (long long)t * a.K + k);
 }
 
 // Block-wise selection of one pass (_selectBestAtoms with nbBlocks > 1 or 'auto', hsc/modeling.py:908-963,
@@ -1006,10 +1055,10 @@ __device__ __noinline__ real near_tie_resolve(const MpArgs<real>& a, hsc_signal_
 // by half a block on 'offset' passes), range / null / interference filters, sort by |c| descending.  The
 // coefficient of every atom is captured HERE, before any atom of the pass is applied (:946, :1101-1120).
 // Returns the number of atoms, left in selection order in list 1 (cand_*[ncand_max ...]).
-template <typename real, int NT>
+template <typename real, int NT, bool RAGGED>
 __device__ __noinline__ int build_pass_list(const MpArgs<real>& a, const real* map_s, const real* res_s, const real* v1,
                                             const int* i1, int* ct, int* ck, real* cc, int offset_flag, double energy_signal) {
-    const int T = a.T, K = a.K, L = a.L, F = a.F, off = a.off, LF = L * F;
+    const int T = signal_length<RAGGED>(a), K = a.K, L = a.L, F = a.F, off = a.off, LF = L * F;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = NT >> 5;
     __shared__ int s_count;
     int bs = a.nb_blocks < 0 ? 4 * L : (int)floor((double)T / (double)a.nb_blocks);
@@ -1026,11 +1075,12 @@ __device__ __noinline__ int build_pass_list(const MpArgs<real>& a, const real* m
         int bt = INT_MAX;
         for (int r = r0 + lane; r < r1; r += 32) take_first_max(bv, bt, v1[r], r);
         group_argmax(bv, bt, 32);
-        if (r0 < r1 && bt == INT_MAX) bt = r0;            // all-zero block: first row (coefficient 0)
-        int k = 0;
+        const bool all_zero = bt == INT_MAX;              // every row's key is 0: np.argmax gives the block's first entry,
+        if (r0 < r1 && all_zero) bt = r0;                 // (first row, filter 0), of coefficient 0 - an all-zero row's key
+        int k = 0;                                        // index is INT_MAX, not a filter
         real c = (real)0;
         if (r0 < r1) {
-            k = i1[bt];
+            k = all_zero ? 0 : i1[bt];
             c = __ldcg(map_s + (long long)bt * K + k);
             const bool edge = (bt - (L - 1) < off) || (bt + (L - 1) > T - L + off);
             if (a.coef_mode == 1 && !edge) {
@@ -1179,12 +1229,15 @@ __device__ __forceinline__ void refold_block(const unsigned long long* slot2, un
 constexpr int kSlotMax = 1024;
 constexpr int kDirtyMax = 8;
 
-template <typename real, int NT, int MINB, int VIF, bool TMA, bool SMH, int RPS = 1>
-__global__ void __launch_bounds__(NT, MINB) pursuit_kernel(MpArgs<real> a) {
+// The body of K2 (pursuit_kernel / pursuit_kernel_ragged).  RAGGED: the signals have their own lengths (a.len,
+// hsc_b200_mp_begin_lengths); a separate kernel, so that the uniform launches bound everything by the parameter a.T
+// exactly as before and pay nothing for it.
+template <typename real, int NT, int VIF, bool TMA, bool SMH, int RPS, bool RAGGED>
+__device__ __forceinline__ void pursuit_body(MpArgs<real> a) {
     const int s = blockIdx.x;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     constexpr int NW = NT / 32;
-    const int T = a.T, K = a.K, L = a.L, F = a.F, off = a.off;
+    const int Tst = a.T, K = a.K, L = a.L, F = a.F, off = a.off;       // Tst: the row stride (and a uniform batch's length)
     const int W = 2 * L - 1;
     const int LF = L * F;
 #ifdef HSC_PROFILE_PHASES
@@ -1193,7 +1246,8 @@ __global__ void __launch_bounds__(NT, MINB) pursuit_kernel(MpArgs<real> a) {
 #endif
 
     // per-signal base pointers live in shared memory (loaded at the use sites) to keep the persistent
-    // loop's register footprint small
+    // loop's register footprint small; so does a ragged signal's length T, which bounds everything below (the arrays
+    // keep the row stride a.T)
     struct Ctx {
         real* map_s; real* res_s; real* v1; int* i1; real* v2; int* i2; real* v3; int* i3;
         unsigned* bits; int* evp; int* evi; real* evc;
@@ -1201,10 +1255,10 @@ __global__ void __launch_bounds__(NT, MINB) pursuit_kernel(MpArgs<real> a) {
     };
     __shared__ Ctx cx;
     if (threadIdx.x == 0) {
-        cx.map_s = a.map + (long long)s * T * K;
-        cx.res_s = a.resid + (long long)s * T * F;
-        cx.v1 = a.val1 + (long long)s * T;
-        cx.i1 = a.idx1 + (long long)s * T;
+        cx.map_s = a.map + (long long)s * Tst * K;
+        cx.res_s = a.resid + (long long)s * Tst * F;
+        cx.v1 = a.val1 + (long long)s * Tst;
+        cx.i1 = a.idx1 + (long long)s * Tst;
         cx.v2 = a.val2 + (long long)s * a.n2;
         cx.i2 = a.idx2 + (long long)s * a.n2;
         cx.v3 = a.val3 + (long long)s * a.n3;
@@ -1216,7 +1270,9 @@ __global__ void __launch_bounds__(NT, MINB) pursuit_kernel(MpArgs<real> a) {
         cx.ct = a.cand_t ? a.cand_t + (long long)s * 2 * a.ncand_max : nullptr;
         cx.ck = a.cand_k ? a.cand_k + (long long)s * 2 * a.ncand_max : nullptr;
         cx.cc = a.cand_c ? a.cand_c + (long long)s * 2 * a.ncand_max : nullptr;
+        if constexpr (RAGGED) CtaLength<true>::set(a.len[s]);
     }
+#define T (CtaLength<RAGGED>::get(Tst))
 #define map_s (cx.map_s)
 #define res_s (cx.res_s)
 #define v1 (cx.v1)
@@ -1362,7 +1418,7 @@ __global__ void __launch_bounds__(NT, MINB) pursuit_kernel(MpArgs<real> a) {
         }
         if (block_mode && new_pass) {
             // ---------------------------------------------------------------- block-wise selection of a pass
-            const int n = build_pass_list<real, NT>(a, map_s, res_s, v1, i1, cx.ct, cx.ck, cx.cc, st.offset_flag, st.energy_signal);
+            const int n = build_pass_list<real, NT, RAGGED>(a, map_s, res_s, v1, i1, cx.ct, cx.ck, cx.cc, st.offset_flag, st.energy_signal);
             if (tid == 0) {
                 st.pass_count = n;
                 st.pass_cursor = 0;
@@ -1426,7 +1482,7 @@ __global__ void __launch_bounds__(NT, MINB) pursuit_kernel(MpArgs<real> a) {
             // float map: the zero-padded product in float64 instead of K1's tensor-core value)
             const bool row_overhangs = (t < off) || (t > T - L + off);
             const bool from_residual = a.coef_mode == 1 && (!row_overhangs || (sizeof(real) == 4 && !overhang_row_written(st, t, off, T, L)));
-            real coef = from_residual ? (real)residual_dot_warp<real>(a, res_s, t, k) : __ldcg(map_s + (long long)t * K + k);
+            real coef = from_residual ? (real)residual_dot_warp<real>(a, res_s, t, k, T) : __ldcg(map_s + (long long)t * K + k);
             if (lane == 0) {
                 sel.t = t;
                 sel.k = k;
@@ -1451,11 +1507,11 @@ __global__ void __launch_bounds__(NT, MINB) pursuit_kernel(MpArgs<real> a) {
             if constexpr (SMH) {
                 asm volatile("bar.sync 1, 64;" ::: "memory");           // warp 0's pick is in `watch`
                 if (watch.t >= 0)
-                    thr = near_tie_watch<real, true>(a, st, map_s, res_s, v1, i1, v2, v3, i3, g1s, watch.t, watch.k,
+                    thr = near_tie_watch<real, true, RAGGED>(a, st, map_s, res_s, v1, i1, v2, v3, i3, g1s, watch.t, watch.k,
                                                      (real)__uint_as_float(watch.vbest), (real)__uint_as_float(watch.second),
                                                      smem_addr_u32(slot2), watch.g2);
             } else {
-                thr = near_tie_watch<real, false>(a, st, map_s, res_s, v1, i1, v2, v3, i3, g1s, 0, 0, (real)0, (real)-1, 0u, -1);
+                thr = near_tie_watch<real, false, RAGGED>(a, st, map_s, res_s, v1, i1, v2, v3, i3, g1s, 0, 0, (real)0, (real)-1, 0u, -1);
             }
             if (lane == 0) sel.thr = thr;
         }
@@ -1464,7 +1520,7 @@ __global__ void __launch_bounds__(NT, MINB) pursuit_kernel(MpArgs<real> a) {
             // near-tie (a fraction of a percent of the atoms): warp 0 re-scores the candidate set from the residual
             if (warp == 0) {
                 int t = sel.t, k = sel.k;
-                const real coef = near_tie_resolve<real, SMH>(a, st, map_s, res_s, v1, smem_addr_u32(slot2), v2, g1s, sel.thr, t, k);
+                const real coef = near_tie_resolve<real, SMH, RAGGED>(a, st, map_s, res_s, v1, smem_addr_u32(slot2), v2, g1s, sel.thr, t, k);
                 __syncwarp();
                 if (lane == 0) {
                     sel.t = t;
@@ -1763,6 +1819,7 @@ __global__ void __launch_bounds__(NT, MINB) pursuit_kernel(MpArgs<real> a) {
 #endif
     if (tid == 0) a.state[s] = st;
 #undef HSC_STAMP
+#undef T
 #undef map_s
 #undef res_s
 #undef v1
@@ -1776,5 +1833,11 @@ __global__ void __launch_bounds__(NT, MINB) pursuit_kernel(MpArgs<real> a) {
 #undef evi
 #undef evc
 }
+
+template <typename real, int NT, int MINB, int VIF, bool TMA, bool SMH, int RPS = 1>
+__global__ void __launch_bounds__(NT, MINB) pursuit_kernel(MpArgs<real> a) { pursuit_body<real, NT, VIF, TMA, SMH, RPS, false>(a); }
+
+template <typename real, int NT, int MINB, int VIF, bool TMA, bool SMH, int RPS = 1>
+__global__ void __launch_bounds__(NT, MINB) pursuit_kernel_ragged(MpArgs<real> a) { pursuit_body<real, NT, VIF, TMA, SMH, RPS, true>(a); }
 
 }  // namespace hsc

@@ -561,7 +561,7 @@ class Engine(object):
         return res
 
     # ------------------------------------------------------------------ streamed encode, codes left on the device
-    def encode_stream_device(self, x, options, capacity=None, min_coefficients=1e-16, want_residual=True):
+    def encode_stream_device(self, x, options, capacity=None, min_coefficients=1e-16, want_residual=True, lengths=None):
         """Matching pursuit of B independent signals x [B,T,F], any B, with the canonical codes and the residual left on the
         device.  The signals run in chunks (_stream_chunk_size) through two encode slots (EncodeSlot): the correlation (K1)
         of chunk i+1 runs on its own stream while the pursuit (K2) of chunk i is still in its tail.  Per chunk, on its slot's
@@ -576,7 +576,11 @@ class Engine(object):
         tensor or numpy array, which first goes through a pinned staging buffer: its throughput is bounded by that host copy.
         Returns (offsets int64 [B+1], pos int32, idx int32, coef float64: device tensors, the entries of signal b being
         [offsets[b], offsets[b+1]); the B final SignalStates; the residual [B,T,F] of the engine dtype on the device, or None
-        when not want_residual)."""
+        when not want_residual).
+
+        lengths: None (every signal has T samples) or an int64 numpy array [B] of values in [1, T] (checked by the caller):
+        signal b is x[b, :lengths[b]] and is encoded as if it were alone (hsc_b200_mp_begin_lengths); its residual past
+        its length is 0."""
         torch = _torch()
         if isinstance(x, np.ndarray):
             x = torch.from_numpy(np.ascontiguousarray(x))
@@ -588,7 +592,8 @@ class Engine(object):
             cur = torch.cuda.current_stream(self.device)
             resid = torch.empty((B, T, self.F), dtype=self.torch_dtype, device=self.device) if want_residual else None
             done = {}                       # first signal of a finished chunk -> (canonical code, entries, states)
-            escalate_capacity(lambda ranges, scale: self._stream_pass(x, ranges, options, cap * scale, min_coefficients, resid, done),
+            escalate_capacity(lambda ranges, scale: self._stream_pass(x, ranges, options, cap * scale, min_coefficients, resid, done,
+                                                                      lengths),
                               [(0, B)] if B > 0 else [], 'encode_stream_device')
             chunks = [done[a] for a in sorted(done)]
             offsets, pos, idx, coef = _concat_codes([(canon, n) for canon, n, _ in chunks], self.device)
@@ -606,7 +611,7 @@ class Engine(object):
         budget = int(self._free_device_bytes() * 0.8) - n_signals * capacity * 16
         return int(min(65535, self.max_signals_per_chunk(T, budget // 2, extra)))
 
-    def _stream_pass(self, x, ranges, options, cap, min_coefficients, resid, done):
+    def _stream_pass(self, x, ranges, options, cap, min_coefficients, resid, done, lengths=None):
         """One pass of encode_stream_device over the signal ranges [a, b) with event buffers of `cap` per signal.  Finished
         chunks go to `done`; returns the ranges of the chunks that must be run again with larger buffers."""
         torch = _torch()
@@ -680,7 +685,8 @@ class Engine(object):
                         h2d[k].record(cs)
                     s_k1.wait_event(h2d[k])
                     xd = xst[k][:m]
-                sl.begin(xd, options, s_k1, resid=None if resid is None else resid[a:b])
+                sl.begin(xd, options, s_k1, resid=None if resid is None else resid[a:b],
+                         lengths=None if lengths is None else lengths[a:b])
                 k1_done = torch.cuda.Event()
                 k1_done.record(s_k1)
                 s2.wait_event(k1_done)
@@ -1132,18 +1138,27 @@ class EncodeSlot(object):
             self.hstate, self.states = eng._pinned_states(S)
         self.k2_done = None
 
-    def begin(self, xd, options, stream, resid=None):
+    def begin(self, xd, options, stream, resid=None, lengths=None):
         """K1 + state reset of the xd.shape[0] <= S signals xd (device, engine dtype, contiguous); the residual goes to
-        `resid` (same shape; default: the slot's own buffer)."""
+        `resid` (same shape; default: the slot's own buffer).  lengths: None, or one length in [1, T] per signal (int64
+        numpy array): signal s is xd[s, :lengths[s]] (hsc_b200_mp_begin_lengths)."""
         e = self.eng
         n = int(xd.shape[0])
         assert 0 < n <= self.S and tuple(xd.shape) == (n, self.T, e.F) and xd.dtype == e.torch_dtype and xd.is_contiguous()
         if resid is None:
             resid = self.resid[:n]
         assert resid.shape == xd.shape and resid.dtype == xd.dtype and resid.is_contiguous() and resid.device == xd.device
-        N.check(e.lib, self.handle, e.lib.hsc_b200_mp_begin(
-            self.handle, ctypes.c_void_p(xd.data_ptr()), ctypes.c_void_p(resid.data_ptr()), n, self.T,
-            ctypes.c_void_p(self.ws.data_ptr()), self.wsb, ctypes.byref(options), ctypes.c_void_p(stream.cuda_stream)))
+        if lengths is None:
+            N.check(e.lib, self.handle, e.lib.hsc_b200_mp_begin(
+                self.handle, ctypes.c_void_p(xd.data_ptr()), ctypes.c_void_p(resid.data_ptr()), n, self.T,
+                ctypes.c_void_p(self.ws.data_ptr()), self.wsb, ctypes.byref(options), ctypes.c_void_p(stream.cuda_stream)))
+        else:
+            ln = np.ascontiguousarray(lengths, dtype=np.int64)
+            assert ln.shape == (n,)
+            N.check(e.lib, self.handle, e.lib.hsc_b200_mp_begin_lengths(
+                self.handle, ctypes.c_void_p(xd.data_ptr()), ctypes.c_void_p(resid.data_ptr()), n, self.T,
+                ln.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), ctypes.c_void_p(self.ws.data_ptr()), self.wsb,
+                ctypes.byref(options), ctypes.c_void_p(stream.cuda_stream)))
         self.n = n
 
     def run(self, stream):

@@ -70,11 +70,32 @@ class MultilevelDictionary(object):
                                   '(hsc.dataset.addSingletonBases); it is outside the hot path')
 
 
-def _codes_to_csc(offsets, pos, idx, coef, T, K):
-    """Flat canonical codes of B signals (offsets [B+1], pos, idx, coef tensors) -> B float64 csc matrices [T,K]."""
+def _codes_to_csc(offsets, pos, idx, coef, T, K, lengths=None):
+    """Flat canonical codes of B signals (offsets [B+1], pos, idx, coef tensors) -> B float64 csc matrices [T,K], or
+    [lengths[b],K] for signal b when lengths is given."""
     off = offsets.cpu().numpy()
     p, i, c = pos.cpu().numpy(), idx.cpu().numpy(), coef.cpu().numpy()
-    return [scipy.sparse.csc_matrix((c[a:b].astype(np.float64), (p[a:b], i[a:b])), shape=(T, K)) for a, b in zip(off[:-1], off[1:])]
+    rows = [T] * (len(off) - 1) if lengths is None else [int(n) for n in lengths]
+    return [scipy.sparse.csc_matrix((c[a:b].astype(np.float64), (p[a:b], i[a:b])), shape=(n, K))
+            for a, b, n in zip(off[:-1], off[1:], rows)]
+
+
+def _check_lengths(lengths, B, T):
+    """Per-signal lengths of a ragged batch [B,T,...] (list, numpy array or host tensor of B integers in [1, T]) as an int64
+    numpy array; raises ValueError otherwise, before any device work."""
+    if hasattr(lengths, 'is_cuda'):
+        if lengths.is_cuda:
+            raise ValueError('lengths must be on the host (a list, a numpy array or a CPU tensor)')
+        lengths = lengths.numpy()
+    a = np.asarray(lengths)
+    if a.ndim != 1 or a.shape[0] != B:
+        raise ValueError('lengths must hold one length per signal: %d expected, got shape %s' % (B, a.shape))
+    if a.dtype.kind not in 'iu':
+        raise ValueError('lengths must be integers, got dtype %s' % a.dtype)
+    a = a.astype(np.int64)
+    if B > 0 and (a.min() < 1 or a.max() > T):
+        raise ValueError('every length must lie in [1, %d] (the padded length)' % T)
+    return a
 
 
 def _decode_codes_device(eng, offsets, pos, idx, coef, B, T, out):
@@ -104,12 +125,15 @@ class SparseCodes(object):
     """Single-level codes of B signals of length T over K filters, as ConvolutionalSparseCoder.encodeBatchDevice returns
     them: offsets (int64 [B+1], from 0), pos, idx (int32) and coef (float64), normally on the GPU.  The entries of signal b
     are [offsets[b], offsets[b+1]): one per nonzero (t, k) of its code, in ascending (t, k) order, which is the order the
-    batched decoder reads.  `states` holds the B final per-signal states (host)."""
+    batched decoder reads.  `states` holds the B final per-signal states (host).  `lengths` is None for a batch of one
+    length, or the int64 host array [B] of the signal lengths of a ragged batch (encodeBatchDevice(..., lengths=)); T is
+    then the padded length, and every position of signal b lies below lengths[b]."""
 
-    def __init__(self, B, T, K, offsets, pos, idx, coef, states):
+    def __init__(self, B, T, K, offsets, pos, idx, coef, states, lengths=None):
         self.B, self.T, self.K = int(B), int(T), int(K)
         self.offsets, self.pos, self.idx, self.coef = offsets, pos, idx, coef
         self.states = list(states)
+        self.lengths = None if lengths is None else _check_lengths(lengths, self.B, self.T)
         assert len(self.states) == self.B and int(self.offsets.numel()) == self.B + 1
 
     def stats(self, b):
@@ -117,8 +141,9 @@ class SparseCodes(object):
         return state_stats(self.states[b])
 
     def to_csc(self):
-        """The B float64 csc matrices [T,K] (canonical format) that encodeBatch returns."""
-        return _codes_to_csc(self.offsets, self.pos, self.idx, self.coef, self.T, self.K)
+        """The B float64 csc matrices [T,K] (canonical format) that encodeBatch returns; [lengths[b],K] for signal b of a
+        ragged batch."""
+        return _codes_to_csc(self.offsets, self.pos, self.idx, self.coef, self.T, self.K, self.lengths)
 
 
 def _dict_eps(D):
@@ -548,7 +573,7 @@ class ConvolutionalMatchingPursuit(SparseApproximator):
         return codes, residual
 
     def computeCoefficientsBatchDevice(self, sequences, D, nbNonzeroCoefs=None, toleranceResidualScale=None, toleranceSnr=None,
-                                       nbBlocks=1, minCoefficients=1e-16, weights=None, returnResidual=True):
+                                       nbBlocks=1, minCoefficients=1e-16, weights=None, returnResidual=True, lengths=None):
         """computeCoefficientsBatch with the codes and the residual left on the GPU, for batches of any size.  sequences
         [B,T] or [B,T,F]: a numpy array, a host torch tensor (a pinned one of the engine dtype is copied to the device
         without staging) or a CUDA tensor on the coder's device (read in place, never modified, when it is contiguous and of
@@ -557,13 +582,23 @@ class ConvolutionalMatchingPursuit(SparseApproximator):
         None with returnResidual=False.  The signals run in chunks through two encodes in flight (Engine.encode_stream_device);
         the codes are summed, ordered and thresholded on the device (Engine.canonicalize_codes).  Duplicate events are summed
         in selection order, which the host path does not guarantee for three or more events of one (t, k), so such a value
-        may differ from computeCoefficientsBatch's in the last bits; sparsity pattern, states and residual are the same."""
+        may differ from computeCoefficientsBatch's in the last bits; sparsity pattern, states and residual are the same.
+
+        lengths: None, or B integers in [1, T] (list, numpy array or host tensor) for a ragged batch: signal b is
+        sequences[b, :lengths[b]], and the padding past it is never read (it may hold anything, NaN included; a CUDA input
+        stays unmodified).  Each signal's codes, states and residual[b, :lengths[b]] are, bit for bit, those of encoding
+        sequences[b:b+1, :lengths[b]] alone with the same keywords, as long as both encodes take the same kernel paths - they
+        do for T <= 131072 with T*K < 2^31 (the tensor-core correlation path is chosen on T*K, and the shared-memory argmax
+        hierarchy, with its near-tie re-ranking, on T).  residual[b, lengths[b]:] is 0; codes.lengths holds the lengths.
+        Bad lengths raise ValueError before any device work."""
         import torch
         if not isinstance(sequences, torch.Tensor):
             sequences = np.asarray(sequences)
         D = np.asarray(D)
         assert sequences.ndim == 2 or sequences.ndim == 3
         assert D.ndim == 2 or D.ndim == 3
+        if lengths is not None:
+            lengths = _check_lengths(lengths, int(sequences.shape[0]), int(sequences.shape[1]))
         x = sequences[:, :, None] if sequences.ndim == 2 else sequences
         eng = self._engine()
         dt = engine_dtype(np.zeros(0, _np_dtype(x)), D)
@@ -571,21 +606,26 @@ class ConvolutionalMatchingPursuit(SparseApproximator):
         opt = eng.make_options(nbNonzeroCoefs, toleranceResidualScale, toleranceSnr, nbBlocks, minCoefficients,
                                use_weights=weights is not None, coef_mode=self.coef_mode, method=self._method, energy_eps=_dict_eps(D))
         offsets, pos, idx, coef, states, residual = eng.encode_stream_device(x, opt, min_coefficients=minCoefficients,
-                                                                             want_residual=returnResidual)
-        codes = SparseCodes(x.shape[0], x.shape[1], eng.K, offsets, pos, idx, coef, states)
+                                                                             want_residual=returnResidual, lengths=lengths)
+        codes = SparseCodes(x.shape[0], x.shape[1], eng.K, offsets, pos, idx, coef, states, lengths=lengths)
         if residual is not None and sequences.ndim == 2:
             residual = residual[:, :, 0]
         return codes, residual
 
     def reconstructBatchDevice(self, codes, D):
         """The float64 reconstruction of SparseCodes on the device, one decoder launch: [B,T] for a 2-D dictionary, else
-        [B,T,F]; equal to ConvolutionalSparseCoder.reconstructBatch(codes.to_csc()) bit for bit."""
+        [B,T,F]; equal to ConvolutionalSparseCoder.reconstructBatch(codes.to_csc()) bit for bit.  For a ragged batch row b
+        is signal b's reconstruction on [0, lengths[b]) and 0 past it: decoding at the padded length and zeroing the tail is
+        exact, because clipping an atom at lengths[b] only drops samples at or past it."""
         import torch
         D = np.asarray(D)
         assert D.ndim == 2 or D.ndim == 3
         eng = engine_for_dictionary(D, None, np.float64, self.device)
         recon = torch.zeros((codes.B, codes.T, eng.F), dtype=torch.float64, device=eng.device)
         _decode_codes_device(eng, codes.offsets, codes.pos, codes.idx, codes.coef, codes.B, codes.T, recon)
+        if codes.lengths is not None and codes.B > 0:
+            keep = torch.arange(codes.T, device=eng.device)[None, :] < torch.from_numpy(codes.lengths).to(eng.device)[:, None]
+            recon.masked_fill_(~keep[:, :, None], 0.0)
         return recon[:, :, 0] if D.ndim == 2 else recon
 
 

@@ -162,6 +162,17 @@ int hsc_b200_mp_begin_part(hsc_engine* e, const void* x_dev, void* residual_dev,
                            void* workspace_dev, size_t workspace_bytes, const hsc_mp_options* opt,
                            int64_t s_lo, int64_t s_count, void* stream);
 
+/* hsc_b200_mp_begin for a ragged batch: signal s is x_dev[s][0 .. lengths_host[s]) and is encoded as if it
+ * were alone - samples at or past its length are never read (they may hold anything, NaN included), and
+ * its residual there becomes exactly 0.  T is the row stride of every [S][T][...] array (x, residual,
+ * workspace: hsc_b200_workspace_bytes(S, T)).  Every length must lie in [1, T], and nb_blocks must
+ * leave blocks of at least 2 samples in every signal; otherwise HSC_E_INVALID.  The engine keeps a
+ * device copy of the lengths per handle (views have their own), which the following hsc_b200_mp_run
+ * calls read like the workspace; hsc_b200_mp_begin / _begin_part forget it (uniform encodes). */
+int hsc_b200_mp_begin_lengths(hsc_engine* e, const void* x_dev, void* residual_dev, int64_t S, int64_t T,
+                              const int64_t* lengths_host, void* workspace_dev, size_t workspace_bytes,
+                              const hsc_mp_options* opt, void* stream);
+
 /* Runs the select/update loop of every unfinished signal until it stops or has written `capacity`
  * events into its slice of the output buffers: ev_pos_dev/ev_idx_dev/ev_coef_dev are
  * [S][capacity] (int32 centre position, int32 filter, `dtype` coefficient), in selection order.
