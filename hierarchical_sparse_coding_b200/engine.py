@@ -156,10 +156,15 @@ class Engine(object):
         self.K = self.L = self.F = None
         self._D_host = None
         self._w_host = None
+        self._dict_version = 0
+        self._views, self._views_version = [], None
+        self._slots = {}                # (S, T, capacity, dictionary version) -> the slot of encode / encode_host
+        self._pipe_slots = {}           # the same key -> the two slots of encode_host_pipelined
+        self._stream_set = None
 
     def close(self):
-        self._pipe_cache = self._host_cache = self._ws_cache = self._last_workspace = None    # device + pinned staging buffers
-        self._stream_stage = None
+        self._slots, self._pipe_slots = {}, {}                          # device + pinned buffers
+        self._ws_cache = self._stream_stage = self._stream_set = None
         for h in getattr(self, '_views', []):
             self.lib.hsc_b200_destroy(h)
         self._views = []
@@ -202,7 +207,7 @@ class Engine(object):
                 wh.ctypes.data_as(ctypes.c_void_p) if wh is not None else None))
         self.dtype = dt
         self.K, self.L, self.F = Dh.shape
-        self._dict_version = getattr(self, '_dict_version', 0) + 1
+        self._dict_version += 1
         self._D_host, self._w_host = Dh.copy(), (None if wh is None else wh.copy())
         return self
 
@@ -303,6 +308,25 @@ class Engine(object):
         h = self.handle if handle is None else handle
         N.check(self.lib, h, self.lib.hsc_b200_mp_states_async(h, states, self._stream_ptr(stream)))
 
+    def _streams(self):
+        """The engine's streams, made on first use: K1 at a higher priority (its CTAs go before waiting K2 CTAs as the tail of
+        the previous encode frees SMs), two K2 streams, copy in, copy out, and one for the codes (copy_out already holds the
+        next batch's waiting work)."""
+        if self._stream_set is None:
+            torch = _torch()
+            new = lambda priority=0: torch.cuda.Stream(device=self.device, priority=priority)
+            self._stream_set = dict(k1=new(-1), k2=[new(), new()], copy_in=new(), copy_out=new(), codes=new())
+        return self._stream_set
+
+    def _slot(self, S, T, cap, staging=False):
+        """The slot encode() and encode_host() run on, on the engine's own handle: kept until a call of another shape or
+        dictionary, and remade with a staging buffer for the first encode_host() that needs one."""
+        key = (S, T, cap, self._dict_version)
+        if key not in self._slots or (staging and self._slots[key].xd is None):
+            self._slots = {}                # the previous slot's buffers go before the new ones are allocated
+            self._slots[key] = EncodeSlot(self, self.handle, S, T, cap, own_residual=False, staging=staging, readback=True)
+        return self._slots[key]
+
     def _workspace(self, S, T):
         """The workspace of an encode of S signals of length T: kept on the engine and grown when too small."""
         torch = _torch()
@@ -347,43 +371,16 @@ class Engine(object):
             if S == 0:
                 return res
             cap = int(capacity) if capacity is not None else self.default_capacity(options, T)
-            wsb = self.workspace_bytes(S, T)
-            ws = torch.empty((wsb,), dtype=torch.uint8, device=self.device)
+            sl = self._slot(S, T, cap)
             resid = xd if residual_inplace else torch.empty_like(xd)
-            evp, evi, evc = self._event_buffers(S, cap)
-            sp = self._stream_ptr(stream)
-            N.check(self.lib, self.handle, self.lib.hsc_b200_mp_begin(
-                self.handle, ctypes.c_void_p(xd.data_ptr()), ctypes.c_void_p(resid.data_ptr()), S, T,
-                ctypes.c_void_p(ws.data_ptr()), wsb, ctypes.byref(options), sp))
-            states = (N.SignalState * S)()
-            chunks_p = [[] for _ in range(S)]
-            chunks_i = [[] for _ in range(S)]
-            chunks_c = [[] for _ in range(S)]
-            while True:
-                N.check(self.lib, self.handle, self.lib.hsc_b200_mp_run(
-                    self.handle, ctypes.c_void_p(evp.data_ptr()), ctypes.c_void_p(evi.data_ptr()),
-                    ctypes.c_void_p(evc.data_ptr()), cap, states, sp))
-                nb = np.array([states[s].n_buffered for s in range(S)], dtype=np.int64)
-                m = int(nb.max())
-                if m > 0:
-                    hp = evp[:, :m].cpu().numpy()
-                    hi = evi[:, :m].cpu().numpy()
-                    hc = evc[:, :m].cpu().numpy()
-                    for s in range(S):
-                        if nb[s] > 0:
-                            chunks_p[s].append(hp[s, :nb[s]].copy())
-                            chunks_i[s].append(hi[s, :nb[s]].copy())
-                            chunks_c[s].append(hc[s, :nb[s]].copy())
-                if not read_states(states, S)[2]:
-                    break
-                if on_pass is not None:
-                    self._fill(res, chunks_p, chunks_i, chunks_c, states)
-                    res.residual = resid
-                    if on_pass(res, states):
-                        break
-            self._fill(res, chunks_p, chunks_i, chunks_c, states)
+            cur = torch.cuda.current_stream(self.device)
+            sl.begin(xd, options, cur, resid=resid)
+
+            def stop(pos, idx, coef, states):
+                res.pos, res.idx, res.coef, res.states, res.residual = pos, idx, coef, states, resid
+                return on_pass(res, states)
+            res.pos, res.idx, res.coef, res.states = sl.drain(None if on_pass is None else stop)
             res.residual = resid if return_residual else None
-            self._last_workspace = ws   # keeps the map alive for map_snapshot()
             self._last_shape = (S, T)
         return res
 
@@ -409,7 +406,6 @@ class Engine(object):
             N.check(self.lib, self.handle, self.lib.hsc_b200_mp_begin(
                 self.handle, ctypes.c_void_p(xd.data_ptr()), ctypes.c_void_p(resid.data_ptr()), S, T,
                 ctypes.c_void_p(ws.data_ptr()), wsb, ctypes.byref(options), self._stream_ptr(stream)))
-            self._last_workspace = ws
             self._last_shape = (S, T)
 
     @_with_stream
@@ -437,13 +433,12 @@ class Engine(object):
         return out
 
     # ------------------------------------------------------------------ resident pipeline (several encodes in flight)
-    def make_slots(self, n, S, T, capacity, own_residual=True):
+    def make_slots(self, n, S, T, capacity, own_residual=True, staging=False):
         """n independent encode slots on this engine's dictionary (native views: own workspace, event buffers, residual,
         pinned states), so that the correlation of one batch can run - on its own stream - while the pursuit of the
         previous one is still going, and the pursuit CTAs of the next batch move into the SMs the previous batch's tail
         frees.  own_residual=False: the caller passes the residual buffer to every begin().  See EncodeSlot."""
-        views = self._views_for(n)
-        return [EncodeSlot(self, views[i], S, T, capacity, own_residual) for i in range(n)]
+        return [EncodeSlot(self, h, S, T, capacity, own_residual, staging=staging) for h in self._views_for(n)]
 
     @_with_stream
     def compact_events(self, evp, evi, evc, out=None, stream=None, handle=None):
@@ -465,26 +460,22 @@ class Engine(object):
 
     # ------------------------------------------------------------------ host pipeline (public batched path)
     def _views_for(self, n):
-        """n extra native handles sharing this engine's device dictionary, one per in-flight chunk."""
-        ver = getattr(self, '_dict_version', 0)
-        if getattr(self, '_views_version', None) != ver or len(getattr(self, '_views', [])) < n:
-            for h in getattr(self, '_views', []):
+        """n extra native handles sharing this engine's device dictionary, kept (for the slots holding them) until it changes."""
+        if self._views_version != self._dict_version:
+            for h in self._views:
                 self.lib.hsc_b200_destroy(h)
-            self._views = []
-            for _ in range(n):
-                h = ctypes.c_void_p()
-                N.check(self.lib, self.handle, self.lib.hsc_b200_create_view(self.handle, ctypes.byref(h)))
-                self._views.append(h)
-            self._views_version = ver
-            self._chunk_cache = {}
+            self._views, self._views_version = [], self._dict_version
+        while len(self._views) < n:
+            h = ctypes.c_void_p()
+            N.check(self.lib, self.handle, self.lib.hsc_b200_create_view(self.handle, ctypes.byref(h)))
+            self._views.append(h)
         return self._views[:n]
 
     def encode_host(self, x_host, options, capacity=None, n_chunks=4, residual_out=None, want_residual=True):
         """Matching pursuit of S independent signals that live in HOST memory (ideally a pinned torch tensor
-        [S,T,F] of the engine dtype).  The host-to-device copy is cut into `n_chunks` chunks on a copy stream;
-        the correlation (K1) of a chunk starts as soon as its copy has landed (hsc_b200_mp_begin_part), so the
-        PCIe transfer hides under K1.  The select/update loop (K2) then runs once over the whole batch - it
-        needs every signal resident to fill the GPU - and codes + residuals are copied back.
+        [S,T,F] of the engine dtype).  The host-to-device copy, in `n_chunks` chunks, hides under the correlation
+        (EncodeSlot.begin_from_host); the select/update loop (K2) then runs over the whole batch - it needs every
+        signal resident to fill the GPU - and codes + residuals are copied back.
         Residuals land in `residual_out` (host tensor like x; allocated, pinned if x is, when None and wanted).
         Returns EncodeResult (events as numpy arrays, residual = the host tensor)."""
         torch = _torch()
@@ -496,67 +487,19 @@ class Engine(object):
         if S == 0:
             return res
         cap = int(capacity) if capacity is not None else self.default_capacity(options, T)
-        n_chunks = max(1, min(int(n_chunks), S))
         if want_residual and residual_out is None:
             residual_out = torch.empty_like(x_host).pin_memory() if x_host.is_pinned() else torch.empty_like(x_host)
         with torch.cuda.device(self.device):
-            key = (S, T, cap, self.F, str(self.dtype))
-            cache = getattr(self, '_host_cache', None)
-            if cache is None or cache['key'] != key:
-                self._host_cache = None
-                wsb = self.workspace_bytes(S, T)
-                cache = dict(key=key, wsb=wsb, copy_stream=torch.cuda.Stream(device=self.device),
-                             ws=torch.empty((wsb,), dtype=torch.uint8, device=self.device),
-                             xd=torch.empty((S, T, self.F), dtype=self.torch_dtype, device=self.device),
-                             hp=torch.empty((S, cap), dtype=torch.int32).pin_memory(),
-                             hi=torch.empty((S, cap), dtype=torch.int32).pin_memory(),
-                             hc=torch.empty((S, cap), dtype=self.torch_dtype).pin_memory(),
-                             states=(N.SignalState * S)())
-                cache['evp'], cache['evi'], cache['evc'] = self._event_buffers(S, cap)
-                self._host_cache = cache
+            sl = self._slot(S, T, cap, staging=True)
             cur = torch.cuda.current_stream(self.device)
-            cs = cache['copy_stream']
+            cs = self._streams()['copy_in']
             cs.wait_stream(cur)                       # the staging buffer may still be read by earlier work
-            sp = ctypes.c_void_p(cur.cuda_stream)
-            xp = ctypes.c_void_p(cache['xd'].data_ptr())
-            wsp = ctypes.c_void_p(cache['ws'].data_ptr())
-            for c in range(n_chunks):
-                lo, hi = S * c // n_chunks, S * (c + 1) // n_chunks
-                with torch.cuda.stream(cs):
-                    cache['xd'][lo:hi].copy_(x_host[lo:hi], non_blocking=True)
-                    ev = torch.cuda.Event()
-                    ev.record(cs)
-                cur.wait_event(ev)
-                N.check(self.lib, self.handle, self.lib.hsc_b200_mp_begin_part(
-                    self.handle, xp, xp, S, T, wsp, cache['wsb'], ctypes.byref(options), lo, hi - lo, sp))
-            stt = cache['states']
-            pp, ip, cp_ = (ctypes.c_void_p(cache['evp'].data_ptr()), ctypes.c_void_p(cache['evi'].data_ptr()),
-                           ctypes.c_void_p(cache['evc'].data_ptr()))
-            chunks_p = [[] for _ in range(S)]
-            chunks_i = [[] for _ in range(S)]
-            chunks_c = [[] for _ in range(S)]
-            while True:
-                N.check(self.lib, self.handle, self.lib.hsc_b200_mp_run(self.handle, pp, ip, cp_, cap, None, sp))
-                self._states_async(stt, cur)
-                cache['hp'].copy_(cache['evp'], non_blocking=True)
-                cache['hi'].copy_(cache['evi'], non_blocking=True)
-                cache['hc'].copy_(cache['evc'], non_blocking=True)
-                cur.synchronize()
-                hp, hi_, hc = cache['hp'].numpy(), cache['hi'].numpy(), cache['hc'].numpy()
-                for s in range(S):
-                    nb = stt[s].n_buffered
-                    if nb > 0:
-                        chunks_p[s].append(hp[s, :nb].copy())
-                        chunks_i[s].append(hi_[s, :nb].copy())
-                        chunks_c[s].append(hc[s, :nb].copy())
-                if not read_states(stt, S)[2]:
-                    break
+            sl.begin_from_host(x_host, options, cs, cur, n_chunks)
+            res.pos, res.idx, res.coef, res.states = sl.drain()
             if want_residual:
-                residual_out.copy_(cache['xd'], non_blocking=True)
+                residual_out.copy_(sl.xd, non_blocking=True)
                 cur.synchronize()
-            self._fill(res, chunks_p, chunks_i, chunks_c, stt)
             res.residual = residual_out if want_residual else None
-            self._last_workspace = cache['ws']
             self._last_shape = (S, T)
         return res
 
@@ -625,8 +568,7 @@ class Engine(object):
         n = max(b - a for a, b in chunks)
         in_place = x.is_cuda and x.dtype == self.torch_dtype and x.is_contiguous()
         direct_h2d = not x.is_cuda and x.is_pinned() and x.dtype == self.torch_dtype and x.is_contiguous()
-        slots = self.make_slots(2, n, T, cap, own_residual=resid is None)
-        xst = None if in_place else [torch.empty((n, T, F), dtype=self.torch_dtype, device=self.device) for _ in range(2)]
+        slots = self.make_slots(2, n, T, cap, own_residual=resid is None, staging=not in_place)
         hst = None
         if not in_place and not direct_h2d and not x.is_cuda:
             # pinned staging of host input, kept on the engine between calls: pinning costs tens of milliseconds per GB
@@ -635,29 +577,21 @@ class Engine(object):
                 self._stream_stage = None
                 self._stream_stage = [torch.empty((n, T, F), dtype=self.torch_dtype).pin_memory() for _ in range(2)]
             hst = self._stream_stage
-        ctx = getattr(self, '_stream_ctx', None)
-        if ctx is None:
-            # K1 on the higher-priority stream: its CTAs are placed before waiting K2 CTAs as the previous chunk's tail
-            # frees SMs (the pipeline of bench.py)
-            ctx = self._stream_ctx = dict(k1=torch.cuda.Stream(device=self.device, priority=-1),
-                                          k2=[torch.cuda.Stream(device=self.device) for _ in range(2)],
-                                          copy=torch.cuda.Stream(device=self.device))
-        s_k1, s_k2, cs = ctx['k1'], ctx['k2'], ctx['copy']
+        streams = self._streams()
+        s_k1, s_k2, cs = streams['k1'], streams['k2'], streams['copy_in']
         cur = torch.cuda.current_stream(self.device)
         count = [torch.empty((1,), dtype=torch.int64).pin_memory() for _ in range(2)]
-        compacted = [None, None]
-        slot_free = [None, None]        # per slot: the last work of its previous chunk
         h2d = [None, None]              # per slot: the copy out of its pinned staging buffer
         rerun = []
 
-        def finish(a, b, k, canon):
-            slot_free[k].synchronize()
-            snap, status, unfinished = read_states(slots[k].hstate, b - a)
+        def finish(a, b, sl, n_entries, canon):
+            sl.done.synchronize()
+            snap, status, unfinished = read_states(sl.hstate, b - a)
             check_refit_groups(status)
             if unfinished:
                 rerun.append((a, b))
                 return
-            done[a] = (canon, int(count[k][0]), list(snap))
+            done[a] = (canon, int(n_entries[0]), list(snap))
 
         for st_ in [s_k1, cs] + s_k2:
             st_.wait_stream(cur)                          # the input and the residual may come from work queued on cur
@@ -666,8 +600,8 @@ class Engine(object):
             for ci, (a, b) in enumerate(chunks):
                 k, m = ci & 1, b - a
                 sl, s2 = slots[k], s_k2[k]
-                if slot_free[k] is not None:
-                    s_k1.wait_event(slot_free[k])         # workspace, event buffers, staging: chunk ci-2 is done with them
+                if sl.done is not None:
+                    s_k1.wait_event(sl.done)              # workspace, event buffers, staging: chunk ci-2 is done with them
                 if in_place:
                     xd = x[a:b]
                 else:
@@ -677,31 +611,30 @@ class Engine(object):
                             h2d[k].synchronize()          # chunk ci-2 has left the pinned staging buffer
                         hst[k][:m].copy_(src)
                         src = hst[k][:m]
+                    xd = sl.xd[:m]
                     with torch.cuda.stream(cs):
-                        if slot_free[k] is not None:
-                            cs.wait_event(slot_free[k])
-                        xst[k][:m].copy_(src, non_blocking=True)
+                        if sl.done is not None:
+                            cs.wait_event(sl.done)
+                        xd.copy_(src, non_blocking=True)
                         h2d[k] = torch.cuda.Event()
                         h2d[k].record(cs)
                     s_k1.wait_event(h2d[k])
-                    xd = xst[k][:m]
                 sl.begin(xd, options, s_k1, resid=None if resid is None else resid[a:b],
                          lengths=None if lengths is None else lengths[a:b])
                 k1_done = torch.cuda.Event()
                 k1_done.record(s_k1)
                 s2.wait_event(k1_done)
                 sl.run(s2)
-                compacted[k] = sl.compact(compacted[k], s2)
-                c = compacted[k]
+                c = sl.compacted = sl.compact(sl.compacted, s2)
                 canon = self.canonicalize_codes(c['offsets'][:m + 1], c['pos'][:m * cap], c['idx'][:m * cap], c['coef'][:m * cap],
                                                 m, T, self.K, None, min_coefficients, stream=s2, handle=sl.handle)[0]
                 with torch.cuda.stream(s2):
                     count[k].copy_(canon['offsets'][m:], non_blocking=True)
-                slot_free[k] = torch.cuda.Event()
-                slot_free[k].record(s2)
+                sl.done = torch.cuda.Event()
+                sl.done.record(s2)
                 if pending is not None:
                     finish(*pending)
-                pending = (a, b, k, canon)
+                pending = (a, b, sl, count[k], canon)
             if pending is not None:
                 finish(*pending)
         finally:
@@ -799,7 +732,7 @@ class Engine(object):
             n = r.S
             out.pos[lo:lo + n], out.idx[lo:lo + n], out.coef[lo:lo + n] = r.pos, r.idx, r.coef
             out.states.extend(r.states)
-            self._last_workspace = None
+        self._slots = {}                    # the chunks fill the free device memory: their buffers are not kept
         return out
 
     # ------------------------------------------------------------------ convolutional k-means assignment step
@@ -824,13 +757,14 @@ class Engine(object):
         return pos, idx, sums, counts
 
     def encode_host_pipelined(self, batches, options, capacity=None, n_chunks=8, want_residual=False, residual_outs=None,
-                              host_events=True, on_device_events=None, two_workspaces=True):
+                              host_events=True, on_device_events=None):
         """Generator over EncodeResult, one per batch of `batches` (an iterable of host tensors [S,T,F] of the engine
         dtype, ideally pinned, all the same shape).  Per batch: chunked host-to-device copy hidden under the correlation
         (hsc_b200_mp_begin_part), the select/update loop, compaction of the event buffers on the device
-        (hsc_b200_mp_compact_events) and the device-to-host read of the codes - exactly 12-16 bytes per atom.  Two sets of
-        staging buffers let the copies out of batch i (their own stream) overlap the copy in and the correlation of batch
-        i+1 (PCIe is full duplex), and the host-side unpacking of batch i overlaps the GPU work of batch i+1.
+        (hsc_b200_mp_compact_events) and the device-to-host read of the codes - exactly 12-16 bytes per atom.  Two encode
+        slots (_pipeline_slots), kept on the engine between calls, let the copies out of batch i (their own stream) overlap
+        the copy in and the correlation of batch i+1 (PCIe is full duplex), and the host-side unpacking of batch i overlaps
+        the GPU work of batch i+1.
 
         want_residual: also copy the residual [S,T,F] back (as large as the input; off by default - the codes are the
           result, the residual is x - decode(codes)).  `residual_outs`: one host tensor per batch to receive it.
@@ -840,185 +774,117 @@ class Engine(object):
           dict(offsets=int64[S+1], pos=int32[..], idx=int32[..], coef=[..], total=n) - the compacted codes still on the
           device (valid until the hook's stream work is done): the hook for the NCCL gather of the sparse codes
           (distributed.gather_device_events); its return value becomes result.gathered.
-        two_workspaces: keep one workspace per staging slot when device memory allows (2 x the correlation maps), so that
-          the correlation of batch i+1 overlaps the tail of batch i's pursuit.
         A batch whose event buffers overflow (`capacity`) raises: use encode_host for open-ended stop rules."""
         torch = _torch()
-        it = iter(batches)
-        # staging buffers (device + pinned host) and streams are kept on the engine between calls: pinned allocations
-        # cost tens of milliseconds
-        cache = getattr(self, '_pipe_cache', None)
-        if cache is None:
-            cache = self._pipe_cache = dict(slots=[None, None], ctx=dict(copy_in=None, copy_out=None))
-        slots, ctx = cache['slots'], cache['ctx']
-        for sl_ in slots:                     # an abandoned earlier call may have left copies in flight
-            if sl_ is not None and sl_['d2h_done'] is not None:
-                sl_['d2h_done'].synchronize()
-                sl_['d2h_done'] = None
-        ctx['states_copied'] = None
-        pending = None          # (slot index, EncodeResult shell, residual_out)
-
-        def make_slot(S, T, cap):
-            n_max = S * cap
-            d = dict(xd=torch.empty((S, T, self.F), dtype=self.torch_dtype, device=self.device),
-                     compact=self._compact_buffers(S, cap),
-                     hoff=torch.empty((S + 1,), dtype=torch.int64).pin_memory(),
-                     hp=torch.empty((n_max,), dtype=torch.int32).pin_memory(),
-                     hi=torch.empty((n_max,), dtype=torch.int32).pin_memory(),
-                     hc=torch.empty((n_max,), dtype=self.torch_dtype).pin_memory(),
-                     d2h_done=None)
-            d['evp'], d['evi'], d['evc'] = self._event_buffers(S, cap)
-            d['hstate'], d['states'] = self._pinned_states(S)
-            return d
+        streams = self._streams()
+        cin, cout, ccodes, s_k1, s_k2 = streams['copy_in'], streams['copy_out'], streams['codes'], streams['k1'], streams['k2']
+        for slots in self._pipe_slots.values():       # an abandoned earlier call may have left copies in flight
+            for sl in slots:
+                if sl.done is not None:
+                    sl.done.synchronize()
+        pending = None          # (slot, EncodeResult shell, residual_out)
 
         def finish(p):
-            k, res, residual_out = p
-            sl = slots[k]
-            dev = sl['compact']
-            cout = ctx['copy_codes']                  # its own stream: copy_out already holds the next batch's (waiting) work
-            sl['small_done'].synchronize()            # states + offsets are on the host
-            S = res.S
+            sl, res, residual_out = p
+            sl.k2_done.synchronize()                  # states + offsets are on the host
             # one private copy of the S states, then vectorised unpacking (a Python loop over 512 signals with three
             # array copies each costs several milliseconds per batch)
-            snap, _, unfinished = read_states(sl['hstate'], S)
+            snap, _, unfinished = read_states(sl.hstate, res.S)
+            sl.done.synchronize()                     # the residual, if wanted
             if unfinished:
-                sl['d2h_done'].synchronize()
                 raise N.HscError(N.HSC_E_NOMEM, 'encode_host_pipelined: event capacity exhausted before the stop rule fired')
-            sl['d2h_done'].synchronize()              # residual (if wanted) and the gather hook's reads of this slot
-            off = sl['hoff'].numpy().copy()
+            host, dev = sl.host, sl.compacted
+            off = host['offsets'].numpy().copy()
             total = int(off[-1])
             res.counts = np.diff(off)
-            if on_device_events is not None:
-                # the sparse codes are still on the device, compacted: the hook gathers them over the ranks (NCCL)
-                with torch.cuda.stream(cout):
+            with torch.cuda.stream(ccodes):
+                if on_device_events is not None:
+                    # the sparse codes are still on the device, compacted: the hook gathers them over the ranks (NCCL)
                     res.gathered = on_device_events(res.batch_index, dict(dev, total=total))
+                if host_events:
+                    # the codes: exactly `total` atoms cross the bus
+                    for f in ('pos', 'idx', 'coef'):
+                        host[f][:total].copy_(dev[f][:total], non_blocking=True)
+                    sl.done = torch.cuda.Event()
+                    sl.done.record(ccodes)
             if host_events:
-                # the codes: exactly `total` atoms cross the bus
-                with torch.cuda.stream(cout):
-                    sl['hp'][:total].copy_(dev['pos'][:total], non_blocking=True)
-                    sl['hi'][:total].copy_(dev['idx'][:total], non_blocking=True)
-                    sl['hc'][:total].copy_(dev['coef'][:total], non_blocking=True)
-                    done = torch.cuda.Event()
-                    done.record(cout)
-                sl['d2h_done'] = done
-                done.synchronize()
-                cuts = off[1:-1]
-                res.pos = np.split(sl['hp'].numpy()[:total].copy(), cuts)
-                res.idx = np.split(sl['hi'].numpy()[:total].copy(), cuts)
-                res.coef = np.split(sl['hc'].numpy()[:total].copy(), cuts)
-            res.states = [snap[i] for i in range(S)]
+                sl.done.synchronize()
+                res.pos, res.idx, res.coef = (np.split(host[f].numpy()[:total].copy(), off[1:-1]) for f in ('pos', 'idx', 'coef'))
+            res.states = list(snap)
             res.residual = residual_out
             return res
 
         with torch.cuda.device(self.device):
             cur = torch.cuda.current_stream(self.device)
-            for bi, x_host in enumerate(it):
-                if isinstance(x_host, np.ndarray):
-                    x_host = torch.from_numpy(np.ascontiguousarray(x_host, dtype=self.dtype))
-                assert x_host.dim() == 3 and x_host.shape[2] == self.F and x_host.dtype == self.torch_dtype
-                S, T, _ = x_host.shape
-                cap = int(capacity) if capacity is not None else self.default_capacity(options, T)
-                k = bi & 1
-                if slots[k] is None or slots[k]['xd'].shape != (S, T, self.F) or slots[k]['evp'].shape[1] != cap:
-                    slots[k] = make_slot(S, T, cap)
-                wsb = self.workspace_bytes(S, T)
-                if ctx.get('copy_in') is None:
-                    ctx['copy_in'] = torch.cuda.Stream(device=self.device)
-                    ctx['copy_out'] = torch.cuda.Stream(device=self.device)
-                    ctx['copy_codes'] = torch.cuda.Stream(device=self.device)
-                    ctx['k1'] = torch.cuda.Stream(device=self.device, priority=-1)
-                    ctx['k2'] = [torch.cuda.Stream(device=self.device), torch.cuda.Stream(device=self.device)]
-                    ctx['wss'] = [None, None]
-                # Two workspaces (one per staging slot) when they fit: the correlation of batch i+1 - on its own stream,
-                # under the chunks of its copy in - then starts while the pursuit of batch i is still in its tail, and the
-                # pursuit of batch i+1 moves into the SMs that tail frees.  One shared workspace otherwise: the correlation
-                # of batch i+1 waits for the pursuit of batch i.
-                if ctx['wss'][k] is None or ctx['wss'][k].numel() < wsb:
-                    ctx['wss'][k] = None
-                    other = ctx['wss'][k ^ 1]
-                    if two_workspaces and (other is None or other.numel() < wsb or self._free_device_bytes() > wsb + (4 << 30)):
-                        ctx['wss'][k] = torch.empty((wsb,), dtype=torch.uint8, device=self.device)
-                    else:
-                        if other is None or other.numel() < wsb:
-                            ctx['wss'][k ^ 1] = other = torch.empty((wsb,), dtype=torch.uint8, device=self.device)
-                        ctx['wss'][k] = other                       # shared
-                shared_ws = ctx['wss'][0] is ctx['wss'][1]
-                handles = [self.handle, self.handle] if shared_ws else self._views_for(2)
-                sl, ws, cin, cout = slots[k], ctx['wss'][k], ctx['copy_in'], ctx['copy_out']
-                s_k1, s_k2, hk = ctx['k1'], ctx['k2'][k], handles[k]
-                if bi == 0:
-                    for st_ in (cin, s_k1, ctx['k2'][0], ctx['k2'][1]):
-                        st_.wait_stream(cur)                        # work queued by the caller before this call
-                residual_out = None
-                if want_residual:
-                    residual_out = residual_outs[bi] if residual_outs is not None else (
-                        torch.empty_like(x_host).pin_memory() if x_host.is_pinned() else torch.empty_like(x_host))
-                # this slot's staging buffers (and its workspace) are free once the copies of batch bi-2 have left them;
-                # a shared workspace also waits for the pursuit and the compaction of batch bi-1
-                if sl['d2h_done'] is not None:
-                    cin.wait_event(sl['d2h_done'])
-                    s_k1.wait_event(sl['d2h_done'])
-                if shared_ws and ctx.get('states_copied') is not None:
-                    s_k1.wait_event(ctx['states_copied'])
-                xp, wsp = ctypes.c_void_p(sl['xd'].data_ptr()), ctypes.c_void_p(ws.data_ptr())
-                k1p = ctypes.c_void_p(s_k1.cuda_stream)
-                nch = max(1, min(int(n_chunks), S))
-                for c in range(nch):
-                    lo, hi = S * c // nch, S * (c + 1) // nch
-                    with torch.cuda.stream(cin):
-                        sl['xd'][lo:hi].copy_(x_host[lo:hi], non_blocking=True)
-                        ev = torch.cuda.Event()
-                        ev.record(cin)
-                    s_k1.wait_event(ev)
-                    N.check(self.lib, hk, self.lib.hsc_b200_mp_begin_part(
-                        hk, xp, xp, S, T, wsp, wsb, ctypes.byref(options), lo, hi - lo, k1p))
-                k1_done = torch.cuda.Event()
-                k1_done.record(s_k1)
-                s_k2.wait_event(k1_done)
-                N.check(self.lib, hk, self.lib.hsc_b200_mp_run(
-                    hk, ctypes.c_void_p(sl['evp'].data_ptr()), ctypes.c_void_p(sl['evi'].data_ptr()),
-                    ctypes.c_void_p(sl['evc'].data_ptr()), cap, None, ctypes.c_void_p(s_k2.cuda_stream)))
-                k2_done = torch.cuda.Event()
-                k2_done.record(s_k2)
-                if shared_ws:
-                    s_k1.wait_event(k2_done)                        # the next correlation overwrites this map
-                with torch.cuda.stream(cout):
-                    cout.wait_event(k2_done)
-                    self._states_async(sl['states'], cout, hk)
-                    self.compact_events(sl['evp'], sl['evi'], sl['evc'], out=sl['compact'], stream=cout, handle=hk)
-                    ctx['states_copied'] = torch.cuda.Event()       # a shared workspace's states may be reset by the next batch
-                    ctx['states_copied'].record(cout)
-                    sl['hoff'].copy_(sl['compact']['offsets'], non_blocking=True)
-                    small = torch.cuda.Event()
-                    small.record(cout)
-                    sl['small_done'] = small
+            try:
+                for bi, x_host in enumerate(batches):
+                    if isinstance(x_host, np.ndarray):
+                        x_host = torch.from_numpy(np.ascontiguousarray(x_host, dtype=self.dtype))
+                    assert x_host.dim() == 3 and x_host.shape[2] == self.F and x_host.dtype == self.torch_dtype
+                    S, T, _ = x_host.shape
+                    cap = int(capacity) if capacity is not None else self.default_capacity(options, T)
+                    key = (S, T, cap, self._dict_version)
+                    if key not in self._pipe_slots:
+                        self._pipe_slots = {}           # the previous slots' buffers go before the new ones are allocated
+                        self._pipe_slots[key] = self._pipeline_slots(S, T, cap)
+                    slots = self._pipe_slots[key]
+                    sl, other, s2 = slots[bi & 1], slots[~bi & 1], s_k2[bi & 1]
+                    if bi == 0:
+                        for st_ in [cin, s_k1] + s_k2:
+                            st_.wait_stream(cur)                    # work queued by the caller before this call
+                    residual_out = None
                     if want_residual:
-                        residual_out.copy_(sl['xd'], non_blocking=True)
-                    done = torch.cuda.Event()
-                    done.record(cout)
-                sl['d2h_done'] = done
-                self._last_workspace, self._last_shape = ws, (S, T)
-                shell = EncodeResult(S, T, self.K)
-                shell.batch_index = bi
+                        residual_out = residual_outs[bi] if residual_outs is not None else (
+                            torch.empty_like(x_host).pin_memory() if x_host.is_pinned() else torch.empty_like(x_host))
+                    # this slot's buffers (and its workspace) are free once the copies of batch bi-2 have left them; a shared
+                    # workspace also waits for the pursuit of batch bi-1 and everything that reads its states
+                    if sl.done is not None:
+                        cin.wait_event(sl.done)
+                        s_k1.wait_event(sl.done)
+                    if sl.ws is other.ws and other.k2_done is not None:
+                        s_k1.wait_event(other.k2_done)
+                    sl.begin_from_host(x_host, options, cin, s_k1, n_chunks)
+                    k1_done = torch.cuda.Event()
+                    k1_done.record(s_k1)
+                    s2.wait_event(k1_done)
+                    sl.run(s2)
+                    sl.compacted = sl.compact(sl.compacted, s2)
+                    with torch.cuda.stream(s2):
+                        sl.host['offsets'].copy_(sl.compacted['offsets'], non_blocking=True)
+                    sl.k2_done = torch.cuda.Event()
+                    sl.k2_done.record(s2)
+                    with torch.cuda.stream(cout):
+                        cout.wait_event(sl.k2_done)
+                        if want_residual:
+                            residual_out.copy_(sl.xd, non_blocking=True)
+                        sl.done = torch.cuda.Event()
+                        sl.done.record(cout)
+                    self._last_shape = (S, T)
+                    shell = EncodeResult(S, T, self.K)
+                    shell.batch_index = bi
+                    if pending is not None:
+                        yield finish(pending)
+                    pending = (sl, shell, residual_out)
                 if pending is not None:
                     yield finish(pending)
-                pending = (k, shell, residual_out)
-            if pending is not None:
-                yield finish(pending)
-            for st_ in (ctx['copy_out'], ctx['copy_codes']):
-                cur.wait_stream(st_)
+            finally:
+                for st_ in (cout, ccodes):
+                    cur.wait_stream(st_)
 
-    def _fill(self, res, cp, ci, cc, states):
-        for s in range(res.S):
-            res.pos[s] = np.concatenate(cp[s]) if cp[s] else np.zeros(0, np.int32)
-            res.idx[s] = np.concatenate(ci[s]) if ci[s] else np.zeros(0, np.int32)
-            res.coef[s] = np.concatenate(cc[s]) if cc[s] else np.zeros(0, self.dtype)
-        res.states = [N.SignalState.from_buffer_copy(bytes(states[s])) for s in range(res.S)]
-
-    def map_snapshot(self):
-        """Copy of the correlation map of the last encode [S,T,K] (tests / diagnostics)."""
-        S, T = self._last_shape
-        return self._to_host(self.lib.hsc_b200_mp_map_dev(self.handle), (S, T, self.K))
+    def _pipeline_slots(self, S, T, cap):
+        """The two slots of encode_host_pipelined.  If, once all their other buffers exist, a second workspace fits with 4 GB
+        to spare, each gets its own on a native view: the correlation of batch i+1 then starts while the pursuit of batch i
+        is still in its tail.  Otherwise both share one on the engine's own handle."""
+        torch = _torch()
+        ws = torch.empty((self.workspace_bytes(S, T),), dtype=torch.uint8, device=self.device)
+        slots = [EncodeSlot(self, self.handle, S, T, cap, own_residual=False, workspace=ws, staging=True, readback=True)
+                 for _ in range(2)]
+        for sl in slots:
+            sl.compacted = self._compact_buffers(S, cap)
+        if self._free_device_bytes() > ws.numel() + (4 << 30):
+            slots[1].ws = torch.empty_like(ws)
+            slots[0].handle, slots[1].handle = self._views_for(2)
+        return slots
 
     # ------------------------------------------------------------------ decoder
     @_with_stream
@@ -1118,25 +984,34 @@ class Engine(object):
 
 
 class EncodeSlot(object):
-    """One encode in flight: a native view of the engine's dictionary with its own workspace (correlation map, argmax
-    hierarchy, states), event buffers and residual.  begin() = K1 + state reset, run() = K2, both asynchronous on the
-    stream given; states_async() copies the per-signal states to the slot's pinned buffer.  An encode may hold fewer
-    signals than the slot was made for (the last chunk of a stream): begin() takes them from xd, and run() / compact()
-    work on that many."""
+    """One encode in flight: a native handle on the engine's dictionary (its own or a view) with a workspace, event
+    buffers, pinned states and optionally a residual, a device input-staging buffer `xd` [S,T,F] and pinned read-back
+    buffers `host`.  begin() / begin_from_host() = K1 + state reset, run() = K2 + a copy of the states to the pinned
+    buffer, both asynchronous on the stream given; drain() runs K2 to the end and reads the events back.  An encode may
+    hold fewer signals than the slot was made for: begin() takes them from xd, and run() / compact() work on that many.
+    `workspace`: a buffer of at least workspace_bytes(S, T) to use instead of a new one."""
 
-    def __init__(self, eng, handle, S, T, capacity, own_residual=True):
+    def __init__(self, eng, handle, S, T, capacity, own_residual=True, workspace=None, staging=False, readback=False):
         torch = _torch()
         self.eng, self.handle = eng, handle
         self.S, self.T, self.cap = int(S), int(T), int(capacity)
         self.n = self.S                 # signals of the encode in flight
-        dev = eng.device
+        dev, n = eng.device, self.S * self.cap
         with torch.cuda.device(dev):
             self.wsb = eng.workspace_bytes(S, T)
-            self.ws = torch.empty((self.wsb,), dtype=torch.uint8, device=dev)
+            assert workspace is None or workspace.numel() >= self.wsb
+            self.ws = torch.empty((self.wsb,), dtype=torch.uint8, device=dev) if workspace is None else workspace
             self.resid = torch.empty((S, T, eng.F), dtype=eng.torch_dtype, device=dev) if own_residual else None
+            self.xd = torch.empty((S, T, eng.F), dtype=eng.torch_dtype, device=dev) if staging else None
             self.evp, self.evi, self.evc = eng._event_buffers(S, capacity)
             self.hstate, self.states = eng._pinned_states(S)
-        self.k2_done = None
+        pin = lambda shape, dt: torch.empty(shape, dtype=dt, pin_memory=True)
+        # read-back buffers: offsets int64 [S+1]; flat pos, idx (int32) and coef (engine dtype) of S * capacity entries
+        self.host = dict(offsets=pin((S + 1,), torch.int64), pos=pin((n,), torch.int32), idx=pin((n,), torch.int32),
+                         coef=pin((n,), eng.torch_dtype)) if readback else None
+        self.compacted = None           # compact()'s output, kept by callers that reuse it
+        self.k2_done = None             # the last K2 of this slot, recorded by its user
+        self.done = None                # the last work that reads this slot's buffers, recorded by its user
 
     def begin(self, xd, options, stream, resid=None, lengths=None):
         """K1 + state reset of the xd.shape[0] <= S signals xd (device, engine dtype, contiguous); the residual goes to
@@ -1161,12 +1036,55 @@ class EncodeSlot(object):
                 ctypes.byref(options), ctypes.c_void_p(stream.cuda_stream)))
         self.n = n
 
+    def begin_from_host(self, x_host, options, copy_stream, stream, n_chunks):
+        """K1 + state reset of S host signals x_host [S,T,F] (engine dtype, ideally pinned) with the residual in place in xd:
+        the copy runs in n_chunks chunks on copy_stream, and the correlation of a chunk starts on `stream` once its copy
+        has landed (hsc_b200_mp_begin_part), so that the transfer hides under K1."""
+        torch, e, S, xd = _torch(), self.eng, self.S, self.xd
+        assert tuple(x_host.shape) == (S, self.T, e.F)
+        xp, wsp, sp = ctypes.c_void_p(xd.data_ptr()), ctypes.c_void_p(self.ws.data_ptr()), ctypes.c_void_p(stream.cuda_stream)
+        n_chunks = max(1, min(int(n_chunks), S))
+        for c in range(n_chunks):
+            lo, hi = S * c // n_chunks, S * (c + 1) // n_chunks
+            with torch.cuda.stream(copy_stream):
+                xd[lo:hi].copy_(x_host[lo:hi], non_blocking=True)
+                ev = torch.cuda.Event()
+                ev.record(copy_stream)
+            stream.wait_event(ev)
+            N.check(e.lib, self.handle, e.lib.hsc_b200_mp_begin_part(
+                self.handle, xp, xp, S, self.T, wsp, self.wsb, ctypes.byref(options), lo, hi - lo, sp))
+        self.n = S
+
     def run(self, stream):
         e = self.eng
         N.check(e.lib, self.handle, e.lib.hsc_b200_mp_run(
             self.handle, ctypes.c_void_p(self.evp.data_ptr()), ctypes.c_void_p(self.evi.data_ptr()),
             ctypes.c_void_p(self.evc.data_ptr()), self.cap, None, ctypes.c_void_p(stream.cuda_stream)))
         e._states_async(self.states, stream, self.handle)
+
+    def drain(self, on_pass=None):
+        """Runs K2 on the current stream until no signal is paused or running.  After each launch: one wait for the states,
+        then the first max(n_buffered) columns of the event buffers through `host` and one more wait.  on_pass(pos, idx,
+        coef, states), if given, is called after every launch that leaves a signal unfinished, with the events so far;
+        returning True stops.  Returns (pos, idx, coef, states): per signal, its events in selection order and its state."""
+        n, stream = self.n, _torch().cuda.current_stream(self.eng.device)
+        out = [[np.zeros(0, dt)] * n for dt in (np.int32, np.int32, self.eng.dtype)]
+        while True:
+            self.run(stream)
+            stream.synchronize()
+            states, _, unfinished = read_states(self.hstate, n)
+            nb = np.frombuffer(states, _STATE_DTYPE)['n_buffered']
+            m = int(nb.max())
+            if m > 0:
+                cols = [self.host[f][:n * m].view(n, m).copy_(ev[:n, :m], non_blocking=True)
+                        for f, ev in (('pos', self.evp), ('idx', self.evi), ('coef', self.evc))]
+                stream.synchronize()
+                for o, a in zip(out, cols):
+                    a = a.numpy()
+                    for s in np.flatnonzero(nb):
+                        o[s] = np.concatenate((o[s], a[s, :nb[s]]))
+            if not unfinished or (on_pass is not None and on_pass(*[list(o) for o in out], list(states))):
+                return out + [list(states)]
 
     def compact(self, out, stream):
         n, e = self.n, self.eng

@@ -706,7 +706,7 @@ class HierarchicalConvolutionalMatchingPursuit(SparseApproximator):
             eng = engine_for_dictionary(D, weights, dt, self.device)
             ws = getattr(eng, '_ws_cache', None)
             if ws is not None and ws.numel() > (256 << 20):      # the per-level engines outlive the call: do not pin large maps
-                eng._ws_cache = eng._last_workspace = None
+                eng._ws_cache = None
         return out
 
     def _chunk_size(self, T, specs, cap_scale):
